@@ -2,7 +2,7 @@
 """Benchmark of the EVQE circuit-evaluation hot path (BASELINE.json: "EVQE circuit evals/sec at 20q; gate-apply
 HBM GB/s vs peak; at 1/2/4/8 GPU").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--layers L]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--layers L] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1], SURVEY.md section 8d "C2"): a population of 32 random EVQE individuals
 (reference generation rules, seed 0 on EVERY rank) on 20 qubits with L parameterised layers, evaluated against a
@@ -16,6 +16,8 @@ circuit incl. the write-only first sweep), ``cpu_baseline`` (C/OpenMP oracle por
 ``c4_26q_sampler`` (BASELINE configs 3 and 4 through the evaluators, with the error against the C oracle), ``e2e_threaded``
 (the reference's calling pattern: 32 threads x single-circuit calls), ``optimizer_calls`` (one circuit, one or two parameter points
 per call, last layer parameterised: microseconds per call).
+``--dump-outputs DIR`` writes what the timed paths returned in their last step as float64 ``DIR/<name>.npy`` (rank 0): the inputs
+are seeded, so two builds run with the same arguments can be compared output for output.
 Multi-GPU (torchrun, one process per GPU): the headline is WEAK scaling -- every rank evaluates the same population of 32, no
 data-path collective.  Extras at N > 1: ``strong`` (ONE population of 32 split over the N ranks + an all-gather of the 32
 doubles per step), ``api_all_devices`` (ONE process driving all N GPUs through ``B200EstimatorV2(devices="all")``, the
@@ -227,8 +229,10 @@ def run_reference(args):
         cpu_evaluate(prepared, table, N_QUBITS)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        cpu_evaluate(prepared, table, N_QUBITS)
+        last = cpu_evaluate(prepared, table, N_QUBITS)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"values": last})
     value = sample * args.steps / dt
     desc = (f"{sample} of the {POPULATION} individuals per step on rank 0, C/OpenMP oracle port, omp_get_max_threads() = {threads} per evaluation "
             f"({host_threads()} host cores available to the process), diagonal table prebuilt")
@@ -251,6 +255,13 @@ def run_reference(args):
         "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }
     print(json.dumps(line))
+
+
+def dump_outputs(directory, arrays):
+    """One float64 ``<name>.npy`` per entry of ``arrays`` (written after the timed region)."""
+    os.makedirs(directory, exist_ok=True)
+    for name, arr in arrays.items():
+        np.save(os.path.join(directory, f"{name}.npy"), np.asarray(arr, dtype=np.float64))
 
 
 def workload_config(args, n_gpus):
@@ -337,6 +348,7 @@ def run_b200(args):
         torch.cuda.synchronize()
     gpu_launches = engine.launch_count - launches0
     barrier()
+    last_values = batch.read()  # the last timed step's results (read after the events: not part of the timed region)
     ms_total = max_over_ranks(ev0.elapsed_time(ev1))
     ms_per_step = ms_total / args.steps
     value = world * POPULATION * args.steps / (ms_total * 1e-3)
@@ -359,6 +371,9 @@ def run_b200(args):
     e2e_s = max_over_ranks(time.perf_counter() - t0)
     e2e_value = world * POPULATION * args.steps / e2e_s
     assert np.allclose(out, values, rtol=0, atol=1e-12)
+    if args.dump_outputs and rank == 0:
+        # "values": device-resident batch (the headline), "e2e_values": B200OperatorCircuitEvaluator.evaluate_circuits
+        dump_outputs(args.dump_outputs, {"values": last_values, "e2e_values": out})
 
     # ---- roofline of the dominant kernel (sweep_kernel<double>), live CUDA events ----
     peak, peak_kind = measured_peak_gbs()
@@ -952,14 +967,23 @@ def sharded_probe(dist, rank, world, local_rank):
     return out
 
 
+def positive_int(text):
+    value = int(text)
+    if value < 1:
+        raise argparse.ArgumentTypeError(f"must be at least 1, got {value}")
+    return value
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=positive_int, default=200,
+                    help="timed steps of the headline and e2e loops (the e2e_threaded and complex64 legs clamp it to 10..100, api_all_devices to >= 10)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", choices=["b200", "reference"], default="b200")
     ap.add_argument("--layers", type=int, default=6)
     ap.add_argument("--skip-extras", action="store_true", help="headline line only: no gate-apply / C3 / C4 / threaded / CPU legs (N = 1), no strong / all-devices / sharded legs (N > 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results as float64 DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)
