@@ -173,6 +173,18 @@ int qb_sample(qb_context* ctx, int batch, const int64_t* plan_ids,
 int qb_statevector(qb_context* ctx, int64_t plan_id, const double* params, int n_params,
                    double* out_re_im /* 2 * 2^n doubles */);
 
+/* qb_evaluate_cvar  <->  OperatorSamplerCircuitEvaluator / BitstringCircuitEvaluator with CVaR(alpha) on the exact
+ * distribution instead of shots: out[i] = expectation.lower_tail_expectation_arrays(|psi_i|^2, E, alpha) over all 2^n basis
+ * states, E(k) = sum_t c_t (-1)^{popcount(k & z_t)} -- the lower alpha tail of |psi_i|^2 in stable ascending (E(k), k) order,
+ * greedy fill stopped once the mass is numpy.isclose to alpha, divided by alpha.  With alpha isclose to 1 the fill runs in basis
+ * order (no sort), as in that function.  The Hamiltonian must be diagonal (QB_ERR_INVALID otherwise, and for alpha outside
+ * (0, 1], and when a plan's width or dtype differs from the first plan's or the Hamiltonian's).  Its data is built on first use
+ * and kept until the Hamiltonian is destroyed: E in basis order (8 B per amplitude), and for alpha < 1 the sorted order and E
+ * sorted (12 B more); QB_ERR_MEMORY when it does not fit the workspace.  Deterministic: bit-identical across runs and
+ * independent of the other entries of the batch. */
+int qb_evaluate_cvar(qb_context* ctx, int batch, const int64_t* plan_ids, const double* params,
+                     const int64_t* param_offsets, int64_t ham_id, double alpha, double* out_values);
+
 /* One evaluate_circuits() list split over several GPUs of one process (the device sets of queasars_b200/primitives.py: the
  * reference wraps ONE primitive in a ThreadPoolExecutor, evqe.py:232-236): entry i of every array belongs to context ctxs[i] and
  * has the meaning of the corresponding qb_evaluate_expectation argument.  Every context evaluates its share on its own host

@@ -1,6 +1,7 @@
 // C-ABI implementation (include/queasars_b200.h): contexts, plans, Hamiltonians, batched evaluation.
 // No CPU fallback: every compute entry point needs a CUDA device and fails with QB_ERR_CUDA otherwise.
 #include <algorithm>
+#include <cmath>
 #include <condition_variable>
 #include <cstdio>
 #include <cstdlib>
@@ -14,6 +15,8 @@
 #include <string>
 #include <thread>
 #include <vector>
+
+#include <cub/device/device_radix_sort.cuh>
 
 #include "qb_kernels.cuh"
 
@@ -126,7 +129,12 @@ struct Ham {
     std::vector<int> generic_groups;  // indices into `groups`
     DevBuf tile_groups, tile_z, tile_wr, tile_wi;
     int tile_n_eff = 0;
+    // data of the exact CVaR (qb_evaluate_cvar), built on first use: E(k) in basis order (every alpha), and for alpha < 1 the
+    // stable ascending (E, k) order as sorted position -> basis index with E at each sorted position
+    DevBuf cvar_energy, cvar_perm, cvar_sorted;
+    int cvar_energy_n_eff = 0, cvar_order_n_eff = 0;
     ~Ham() {
+        cvar_energy.release(), cvar_perm.release(), cvar_sorted.release();
         tile_groups.release(), tile_z.release(), tile_wr.release(), tile_wi.release();
         diag_z.release(), diag_c.release(), table.release();
         for (auto& g : groups) g->z.release(), g->wr.release(), g->wi.release();
@@ -815,6 +823,71 @@ size_t max_batch_for(qb_context* ctx, const Plan* pl) {
     return std::min<size_t>(65535, std::max<size_t>(1, limit / state_bytes));  // 65535: grid.y of the batched launches
 }
 
+// E(k) of the Hamiltonian's diagonal terms for k < 2^n_eff into `table` (asynchronous on the context's stream)
+int fill_diag_table(qb_context* ctx, const Ham& ham, double* table, int n_eff) {
+    const uint64_t size = uint64_t(1) << n_eff;
+    if (ham.n_diag == 0) {
+        QB_CUDA(cudaMemsetAsync(table, 0, sizeof(double) * size, ctx->stream));
+        return QB_OK;
+    }
+    const int blocks = int(std::min<uint64_t>(uint64_t(ctx->sm_count) * 8, std::max<uint64_t>(1, size / 256)));
+    for (int lo = 0; lo < ham.n_diag; lo += kTableTermChunk) {  // term order is kept: chunk after chunk accumulates onto the table
+        const int cnt = std::min(kTableTermChunk, ham.n_diag - lo);
+        qb::diag_table_kernel<<<blocks, 256, size_t(cnt) * (sizeof(uint64_t) + sizeof(double)), ctx->stream>>>(
+            table, size, 0, ham.diag_z.as<uint64_t>() + lo, ham.diag_c.as<double>() + lo, cnt, lo ? 1 : 0);
+        QB_TRY(check_launch(ctx, "diag_table_kernel"));
+    }
+    return QB_OK;
+}
+
+size_t workspace_limit_of(const qb_context* ctx) { return ctx->workspace_limit ? ctx->workspace_limit : ctx->default_workspace; }
+
+// Build (once per Hamiltonian and state width) what qb_evaluate_cvar reads: E(k) in basis order (8 B per amplitude); with `sorted`
+// also a stable ascending radix sort of (E(k), k) -> perm (sorted position -> k, 4 B) and E_sorted (8 B).  CUB's radix sort is
+// stable and treats -0.0 == +0.0, which is numpy.argsort(kind="stable") on float64.  The sort needs the input indices and CUB's
+// sort storage for a moment.
+int ensure_cvar_order(qb_context* ctx, Ham& ham, int n_eff, bool sorted) {
+    const uint64_t size = uint64_t(1) << n_eff;
+    const size_t limit = workspace_limit_of(ctx);
+    if (ham.cvar_energy_n_eff != n_eff) {
+        if (sizeof(double) * size > limit)
+            return fail(QB_ERR_MEMORY, "the CVaR energies of a " + std::to_string(n_eff) + "-qubit Hamiltonian need " +
+                                           std::to_string(sizeof(double) * size) + " bytes, the workspace is " + std::to_string(limit) + " bytes");
+        ham.cvar_energy_n_eff = ham.cvar_order_n_eff = 0;
+        QB_TRY(ham.cvar_energy.reserve(sizeof(double) * size));
+        QB_TRY(fill_diag_table(ctx, ham, ham.cvar_energy.as<double>(), n_eff));
+        QB_CUDA(cudaStreamSynchronize(ctx->stream));
+        ham.cvar_energy_n_eff = n_eff;
+    }
+    if (!sorted || ham.cvar_order_n_eff == n_eff) return QB_OK;
+    size_t sort_bytes = 0;
+    QB_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, static_cast<const double*>(nullptr), static_cast<double*>(nullptr),
+                                            static_cast<const uint32_t*>(nullptr), static_cast<uint32_t*>(nullptr), int64_t(size), 0,
+                                            int(sizeof(double) * 8), ctx->stream));
+    const size_t index_at = (sort_bytes + 255) & ~size_t(255);
+    const size_t kept = (sizeof(double) * 2 + sizeof(uint32_t)) * size, need = kept + index_at + sizeof(uint32_t) * size;
+    if (need > limit)
+        return fail(QB_ERR_MEMORY, "the CVaR order data of a " + std::to_string(n_eff) + "-qubit Hamiltonian needs " + std::to_string(need) +
+                                       " bytes to build (" + std::to_string(kept) + " kept), the workspace is " + std::to_string(limit) + " bytes");
+    QB_TRY(ham.cvar_sorted.reserve(sizeof(double) * size));
+    QB_TRY(ham.cvar_perm.reserve(sizeof(uint32_t) * size));
+    DevBuf temp;
+    QB_TRY(temp.reserve(index_at + sizeof(uint32_t) * size));
+    uint32_t* index = reinterpret_cast<uint32_t*>(static_cast<unsigned char*>(temp.p) + index_at);
+    const int blocks = int(std::min<uint64_t>(uint64_t(ctx->sm_count) * 8, std::max<uint64_t>(1, size / 256)));
+    qb::iota_u32_kernel<<<blocks, 256, 0, ctx->stream>>>(index, size);
+    int rc = check_launch(ctx, "iota_u32_kernel");
+    if (rc == QB_OK) {
+        cudaError_t e = cub::DeviceRadixSort::SortPairs(temp.p, sort_bytes, ham.cvar_energy.as<double>(), ham.cvar_sorted.as<double>(), index,
+                                                        ham.cvar_perm.as<uint32_t>(), int64_t(size), 0, int(sizeof(double) * 8), ctx->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+        if (e != cudaSuccess) rc = fail(QB_ERR_CUDA, std::string("cub::DeviceRadixSort::SortPairs: ") + cudaGetErrorString(e));
+    }
+    temp.release();
+    if (rc == QB_OK) ham.cvar_order_n_eff = n_eff;
+    return rc;
+}
+
 }  // namespace
 
 // =====================================================================================================
@@ -1122,16 +1195,9 @@ int qb_hamiltonian_create(qb_context* ctx, int n_qubits, int n_terms, const uint
     QB_CUDA(cudaStreamSynchronize(ctx->stream));
     if (build_table && ham->n_diag > 0) {
         const int n_eff = std::max(n_qubits, QB_TILE_BITS);
-        const uint64_t size = uint64_t(1) << n_eff;
-        QB_TRY(ham->table.reserve(sizeof(double) * size));
+        QB_TRY(ham->table.reserve(sizeof(double) * (uint64_t(1) << n_eff)));
         ham->table_n_eff = n_eff;
-        const int blocks = int(std::min<uint64_t>(uint64_t(ctx->sm_count) * 8, std::max<uint64_t>(1, size / 256)));
-        for (int lo = 0; lo < ham->n_diag; lo += kTableTermChunk) {  // term order is kept: chunk after chunk accumulates onto the table
-            const int cnt = std::min(kTableTermChunk, ham->n_diag - lo);
-            qb::diag_table_kernel<<<blocks, 256, size_t(cnt) * (sizeof(uint64_t) + sizeof(double)), ctx->stream>>>(
-                ham->table.as<double>(), size, 0, ham->diag_z.as<uint64_t>() + lo, ham->diag_c.as<double>() + lo, cnt, lo ? 1 : 0);
-            QB_TRY(check_launch(ctx, "diag_table_kernel"));
-        }
+        QB_TRY(fill_diag_table(ctx, *ham, ham->table.as<double>(), n_eff));
         QB_CUDA(cudaStreamSynchronize(ctx->stream));
     }
     {   // schedule the non-diagonal x-mask groups into tile sweeps
@@ -1430,6 +1496,79 @@ int qb_sample(qb_context* ctx, int batch, const int64_t* plan_ids, const double*
         const int64_t* sorted = static_cast<const int64_t*>(ctx->pin_out.p);
         for (int pos = 0; pos < n; ++pos)
             std::memcpy(out_indices + size_t(lo + b.order[pos]) * shots, sorted + size_t(pos) * shots, sizeof(int64_t) * size_t(shots));
+    }
+    return QB_OK;
+}
+
+int qb_evaluate_cvar(qb_context* ctx, int batch, const int64_t* plan_ids, const double* params, const int64_t* param_offsets,
+                     int64_t ham_id, double alpha, double* out_values) {
+    if (!ctx || !plan_ids || !param_offsets || !out_values) return fail(QB_ERR_INVALID, "null argument");
+    if (!(alpha > 0.0 && alpha <= 1.0)) return fail(QB_ERR_INVALID, "alpha must be in the range (0, 1]");
+    if (batch <= 0) return QB_OK;
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    QB_ON_DEVICE(ctx);
+    Ham* ham = find_ham(ctx, ham_id);
+    if (!ham) return fail(QB_ERR_NOT_FOUND, "unknown Hamiltonian id");
+    if (!ham->diagonal) return fail(QB_ERR_INVALID, "CVaR needs a diagonal Hamiltonian; this one has non-diagonal terms");
+    Plan* first = find_plan(ctx, plan_ids[0]);
+    if (!first) return fail(QB_ERR_NOT_FOUND, "unknown plan id " + std::to_string(plan_ids[0]));
+    // every chunk below is launched against order data of 2^first->n_eff entries: all plans must match it and the Hamiltonian
+    for (int i = 0; i < batch; ++i) {
+        const Plan* pl = find_plan(ctx, plan_ids[i]);
+        if (!pl) return fail(QB_ERR_NOT_FOUND, "unknown plan id " + std::to_string(plan_ids[i]));
+        if (pl->n_qubits != ham->n_qubits)
+            return fail(QB_ERR_INVALID, "Hamiltonian acts on " + std::to_string(ham->n_qubits) + " qubits, circuit " + std::to_string(i) +
+                                            " on " + std::to_string(pl->n_qubits));
+        if (pl->n_eff != first->n_eff || pl->dtype != first->dtype)
+            return fail(QB_ERR_INVALID, "all plans of one CVaR call must share state width and dtype");
+    }
+    // alpha ~ 1 (numpy.isclose(alpha, 1)): the greedy fill in basis order, no sort (expectation.lower_tail_expectation_arrays)
+    const bool sorted = std::fabs(alpha - 1.0) > 1e-8 + 1e-5;
+    QB_TRY(ensure_cvar_order(ctx, *ham, first->n_eff, sorted));
+    const uint32_t* perm = sorted ? ham->cvar_perm.as<uint32_t>() : nullptr;
+    const double* energy = sorted ? ham->cvar_sorted.as<double>() : ham->cvar_energy.as<double>();
+    // the statevectors share the workspace with the CVaR data the Hamiltonian holds
+    const size_t state_bytes = (size_t(1) << first->n_eff) * amp_bytes(first->dtype);
+    const size_t limit = workspace_limit_of(ctx), kept = ham->cvar_energy.cap + ham->cvar_perm.cap + ham->cvar_sorted.cap;
+    if (kept + state_bytes > limit)
+        return fail(QB_ERR_MEMORY, "CVaR data (" + std::to_string(kept) + " bytes) and one statevector (" + std::to_string(state_bytes) +
+                                       " bytes) do not fit the workspace of " + std::to_string(limit) + " bytes");
+    const int chunk = int(std::min<size_t>({size_t(batch), max_batch_for(ctx, first), (limit - kept) / state_bytes}));
+    for (int lo = 0; lo < batch; lo += chunk) {
+        const int n = std::min(chunk, batch - lo);
+        DeviceBatch& b = ctx->oneshot;
+        QB_TRY(build_batch(ctx, b, n, plan_ids + lo, nullptr, nullptr, 1, 0));
+        QB_TRY(batch_upload_params(ctx, b, params, param_offsets + lo));
+        QB_TRY(launch_circuits(ctx, b, nullptr));
+        const uint64_t size = uint64_t(1) << b.n_eff;
+        const uint64_t n_chunks = size >> qb::kChunkBits;
+        QB_TRY(ctx->scratch.reserve(sizeof(double) * (2 * size_t(n) * n_chunks + size_t(n))));
+        double* d_mass = ctx->scratch.as<double>();
+        double* d_pe = d_mass + size_t(n) * n_chunks;  // right after the masses: one scan launch covers both
+        double* d_out = d_pe + size_t(n) * n_chunks;
+        dim3 cgrid(unsigned(std::min<uint64_t>((n_chunks + 7) / 8, 2048)), unsigned(n));
+        const unsigned fgrid = unsigned((n + 7) / 8);
+        if (b.dtype == QB_C128) {
+            qb::cvar_chunk_kernel<double><<<cgrid, 256, 0, ctx->stream>>>(b.states.as<double2>(), size, perm, energy, n_chunks, d_mass, d_pe);
+            QB_TRY(check_launch(ctx, "cvar_chunk_kernel"));
+            qb::scan_chunks_kernel<<<2 * n, 1024, 0, ctx->stream>>>(d_mass, n_chunks);
+            QB_TRY(check_launch(ctx, "scan_chunks_kernel"));
+            qb::cvar_finish_kernel<double><<<fgrid, 256, 0, ctx->stream>>>(b.states.as<double2>(), size, perm, energy, d_mass, d_pe, n_chunks,
+                                                                           alpha, n, d_out);
+        } else {
+            qb::cvar_chunk_kernel<float><<<cgrid, 256, 0, ctx->stream>>>(b.states.as<float2>(), size, perm, energy, n_chunks, d_mass, d_pe);
+            QB_TRY(check_launch(ctx, "cvar_chunk_kernel"));
+            qb::scan_chunks_kernel<<<2 * n, 1024, 0, ctx->stream>>>(d_mass, n_chunks);
+            QB_TRY(check_launch(ctx, "scan_chunks_kernel"));
+            qb::cvar_finish_kernel<float><<<fgrid, 256, 0, ctx->stream>>>(b.states.as<float2>(), size, perm, energy, d_mass, d_pe, n_chunks,
+                                                                          alpha, n, d_out);
+        }
+        QB_TRY(check_launch(ctx, "cvar_finish_kernel"));
+        QB_TRY(ctx->pin_out.reserve(sizeof(double) * size_t(n)));
+        QB_CUDA(cudaMemcpyAsync(ctx->pin_out.p, d_out, sizeof(double) * size_t(n), cudaMemcpyDeviceToHost, ctx->stream));
+        QB_CUDA(cudaStreamSynchronize(ctx->stream));
+        const double* sorted_out = static_cast<const double*>(ctx->pin_out.p);
+        for (int pos = 0; pos < n; ++pos) out_values[lo + b.order[pos]] = sorted_out[pos];
     }
     return QB_OK;
 }

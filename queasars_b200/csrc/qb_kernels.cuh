@@ -9,6 +9,7 @@
 //   expect_group_kernel K4     Re sum_k psi_k conj(psi_{k^x}) W_x(k) for one x-mask group of a Pauli sum
 //   expect_tile_kernel  K4     the same for all groups that fit one 2^11 tile: one read of the state per tile sweep
 //   chunk_prob_kernel / scan_chunks_kernel / sample_kernel   K5  prefix-sum CDF sampling
+//   cvar_chunk_kernel / scan_chunks_kernel / cvar_finish_kernel  K6  exact CVaR(alpha) of a diagonal Hamiltonian (sorted lower tail)
 //   swap_p2p_kernel            global <-> local qubit swap of a sharded state fused with its all-to-all (peer-memory stores)
 //
 // What the arithmetic follows ([upstream] = un-vendored qiskit 2.4.2, see oracle/qiskit_semantics.py):
@@ -1114,6 +1115,98 @@ sample_kernel(const typename Cx<T>::type* __restrict__ states, uint64_t state_st
     if (found < 0) found = int64_t(lo * kChunk + kChunk - 1);  // rounding at the very top of a chunk
     if (uint64_t(found) >= valid_size) found = int64_t(valid_size - 1);
     if (lane == 0) out[blockIdx.y * uint64_t(shots) + shot] = found;
+}
+
+// ---------------------------------------------------------------------------------------------------
+// exact CVaR(alpha) of a diagonal Hamiltonian (K6): the lower alpha-tail of |psi_k|^2 in (E(k), k) order, weighted by E(k)
+// (expectation.lower_tail_expectation_arrays on the full distribution).  `perm` = sorted position -> basis index and
+// `energy` = E at each sorted position (the Hamiltonian's order data); perm == nullptr walks basis order with energy = E(k)
+// (the unsorted greedy rule of alpha ~ 1).  chunk sums -> scan_chunks_kernel on both sums -> one warp per entry finishes.
+// Every sum runs in a fixed order (lane, then warp_sum / warp scan): bit-identical across runs and batch compositions.
+// ---------------------------------------------------------------------------------------------------
+template <typename T>
+__device__ __forceinline__ double cvar_prob(const typename Cx<T>::type* __restrict__ st, const uint32_t* __restrict__ perm, uint64_t pos) {
+    const auto a = st[perm ? uint64_t(perm[pos]) : pos];
+    return double(a.x) * double(a.x) + double(a.y) * double(a.y);
+}
+
+// grid.x covers chunks (one warp per 512 sorted positions), grid.y = batch entry: chunk mass and chunk sum p * E
+template <typename T>
+__global__ void __launch_bounds__(256)
+cvar_chunk_kernel(const typename Cx<T>::type* __restrict__ states, uint64_t state_stride, const uint32_t* __restrict__ perm,
+                  const double* __restrict__ energy, uint64_t n_chunks, double* __restrict__ chunk_mass, double* __restrict__ chunk_pe) {
+    const int lane = threadIdx.x & 31;
+    const uint64_t warps_per_grid = uint64_t(gridDim.x) * (blockDim.x >> 5);
+    const auto* st = states + blockIdx.y * state_stride;
+    for (uint64_t ch = blockIdx.x * uint64_t(blockDim.x >> 5) + (threadIdx.x >> 5); ch < n_chunks; ch += warps_per_grid) {
+        double m = 0.0, s = 0.0;
+#pragma unroll 4
+        for (int i = 0; i < kChunk / 32; ++i) {
+            const uint64_t pos = ch * kChunk + i * 32 + lane;
+            const double p = cvar_prob<T>(st, perm, pos);
+            m += p;
+            s = fma(p, energy[pos], s);
+        }
+        m = warp_sum(m);
+        s = warp_sum(s);
+        if (lane == 0) chunk_mass[blockIdx.y * n_chunks + ch] = m, chunk_pe[blockIdx.y * n_chunks + ch] = s;
+    }
+}
+
+__global__ void iota_u32_kernel(uint32_t* __restrict__ out, uint64_t size) {
+    for (uint64_t k = blockIdx.x * uint64_t(blockDim.x) + threadIdx.x; k < size; k += uint64_t(gridDim.x) * blockDim.x) out[k] = uint32_t(k);
+}
+
+// one warp per batch entry; mass_cdf / pe_cdf are the inclusive scans of the chunk sums.  The stop entry is the first k whose running
+// mass reaches alpha - (atol + rtol * alpha) (numpy.isclose); out = (sum_{i<k} p_i E_i + min(alpha - cum_{k-1}, p_k) E_k) / alpha.
+template <typename T>
+__global__ void __launch_bounds__(256)
+cvar_finish_kernel(const typename Cx<T>::type* __restrict__ states, uint64_t state_stride, const uint32_t* __restrict__ perm,
+                   const double* __restrict__ energy, const double* __restrict__ mass_cdf, const double* __restrict__ pe_cdf, uint64_t n_chunks,
+                   double alpha, int batch, double* __restrict__ out) {
+    const int lane = threadIdx.x & 31;
+    const int entry = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (entry >= batch) return;
+    const auto* st = states + entry * state_stride;
+    const double* cdf = mass_cdf + entry * n_chunks;
+    const double* pcdf = pe_cdf + entry * n_chunks;
+    const double bound = alpha - (1e-8 + 1e-5 * alpha);
+    if (cdf[n_chunks - 1] < bound) {  // the whole distribution weighs less than the bound: every entry is taken
+        if (lane == 0) out[entry] = pcdf[n_chunks - 1] / alpha;
+        return;
+    }
+    uint64_t lo = 0, hi = n_chunks - 1;
+    while (lo < hi) {
+        const uint64_t mid = (lo + hi) >> 1;
+        if (cdf[mid] >= bound) hi = mid;
+        else lo = mid + 1;
+    }
+    double run = lo ? cdf[lo - 1] : 0.0, acc = lo ? pcdf[lo - 1] : 0.0;
+    for (int i = 0; i < kChunk / 32; ++i) {
+        const uint64_t pos = lo * kChunk + i * 32 + lane;
+        const double p = cvar_prob<T>(st, perm, pos);
+        const double e = energy[pos];
+        double inc = p, pe = p * e;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const double nb = __shfl_up_sync(0xffffffffu, inc, o);
+            const double nbe = __shfl_up_sync(0xffffffffu, pe, o);
+            if (lane >= o) inc += nb, pe += nbe;
+        }
+        // the last entry of the chunk stops the walk when the in-chunk running sum misses the bound by rounding only
+        const bool hit = run + inc >= bound || (i == kChunk / 32 - 1 && lane == 31);
+        const unsigned ballot = __ballot_sync(0xffffffffu, hit);
+        const double excl = __shfl_up_sync(0xffffffffu, inc, 1), excl_pe = __shfl_up_sync(0xffffffffu, pe, 1);
+        if (ballot) {
+            if (lane == __ffs(ballot) - 1) {
+                const double before = run + (lane ? excl : 0.0);
+                out[entry] = (acc + (lane ? excl_pe : 0.0) + fmin(alpha - before, p) * e) / alpha;
+            }
+            return;
+        }
+        run += __shfl_sync(0xffffffffu, inc, 31);
+        acc += __shfl_sync(0xffffffffu, pe, 31);
+    }
 }
 
 // ---------------------------------------------------------------------------------------------------

@@ -439,6 +439,16 @@ class Engine:
         _native.check(self._lib.qb_sample(self._ctx, len(plans), _native.ptr(ids), _native.ptr(flat), _native.ptr(offsets), int(shots), _native.ptr(uniforms), _native.ptr(out)))
         return out
 
+    def cvar(self, plans: Sequence[PlanHandle], params: Sequence[Sequence[float]], ham: HamiltonianHandle, alpha: float) -> np.ndarray:
+        """Exact CVaR(alpha) of the diagonal ``ham`` on every circuit's full distribution |psi|^2, no shots
+        (``qb_evaluate_cvar``: ``expectation.lower_tail_expectation_arrays`` over all 2^n basis states)."""
+        if not plans:
+            return np.zeros(0)
+        ids, flat, offsets = self._pack(plans, params)  # (raises ValueError for a length mismatch, as in expectation / sample)
+        out = np.empty(len(plans), dtype=np.float64)
+        _native.check(self._lib.qb_evaluate_cvar(self._ctx, len(plans), _native.ptr(ids), _native.ptr(flat), _native.ptr(offsets), ham.ham_id, float(alpha), _native.ptr(out)))
+        return out
+
     def statevector(self, plan: PlanHandle, params: Sequence[float]) -> np.ndarray:
         vals = np.ascontiguousarray(np.asarray(params, dtype=np.float64).reshape(-1))
         if vals.size != plan.n_params:

@@ -9,6 +9,11 @@ non-SparsePauliOp operator on the sampler route, qubit-count mismatch of ``initi
 result semantics, but evaluating the whole list in one batched GPU submission instead of one primitive pub
 per circuit.  Inputs are never mutated; outputs are fresh Python floats.
 
+``sampler_shots=None`` on the two sampler evaluators means exact values: CVaR(alpha) of the full distribution |psi|^2 of the
+statevector instead of a shot histogram (``B200SamplerV2.cvar_values``; with alpha close to 1 the operator evaluator returns
+sum_k |psi_k|^2 E(k)), so the objective carries no shot noise.  It needs a diagonal energy on the device: a ``SparsePauliOp`` of
+Z terms, or a bitstring evaluator exposing ``diagonal_terms``.
+
 Differences that are deliberate and documented in DESIGN.md:
   * the first constructor argument must be a ``B200EstimatorV2`` / ``B200SamplerV2`` (it carries device,
     dtype and seed); any other primitive type raises ``TypeError`` -- to drive a foreign primitive use the
@@ -141,13 +146,23 @@ class B200OperatorCircuitEvaluator(BaseCircuitEvaluator, _WithInitialState):
 
 
 class _SamplerEvaluator(BaseCircuitEvaluator, _WithInitialState):
-    def __init__(self, sampler: B200SamplerV2, sampler_shots: int, alpha: float):
+    def __init__(self, sampler: B200SamplerV2, sampler_shots: Optional[int], alpha: float):
         if not isinstance(sampler, B200SamplerV2):
             raise TypeError(f"{type(self).__name__} needs a B200SamplerV2 (it carries device / dtype / seed)")
         self._sampler = sampler
-        self._sampler_shots = int(sampler_shots)
+        self._sampler_shots = None if sampler_shots is None else int(sampler_shots)  # None: exact values, no shots
         ex.check_alpha(alpha)
         self._alpha = float(alpha)
+
+    def _exact(self, circuits, parameter_values, operator, kind: str) -> list[float]:
+        pairs = [(c, p) for c, p in zip(self._prepend(circuits), parameter_values) if c is not None and p is not None]
+        try:
+            values = self._sampler._exact(kind, [c for c, _ in pairs], [p for _, p in pairs], operator, self._alpha)
+        except (ValueError, TypeError, NotImplementedError):
+            raise
+        except Exception as exc:
+            raise CircuitEvaluatorException(str(exc)) from exc
+        return [float(v) for v in values]
 
     def _distributions(self, circuits, parameter_values):
         try:
@@ -176,6 +191,8 @@ class B200OperatorSamplerCircuitEvaluator(_SamplerEvaluator):
         self._initial_state_circuit = initial_state_circuit
 
     def evaluate_circuits(self, circuits: list, parameter_values: list[list[float]]) -> list[float]:
+        if self._sampler_shots is None:  # exact: sum p E for alpha ~ 1 (as the sampled branch below), the sorted lower tail otherwise
+            return self._exact(circuits, parameter_values, self._operator, "exp" if ex._close(self._alpha, 1) else "cvar")
         # the quasi-distributions of measure_quasi_distributions (circuit_evaluation.py:29-59) as (states, counts) arrays in
         # ascending state order -- the same entries, in the same order, as the dict route, without 10 000-entry dicts
         pairs = [(c, p) for c, p in zip(self._prepend(circuits), parameter_values) if c is not None and p is not None]
@@ -227,8 +244,15 @@ class B200BitstringCircuitEvaluator(_SamplerEvaluator):
 
             z, c = bitstring_evaluator.diagonal_terms
             self._diagonal_op = SparsePauliOp._raw(n, [0] * len(z), [int(v) for v in z], [float(v) for v in c])
+        elif self._sampler_shots is None:
+            raise ValueError(
+                "exact evaluation (sampler_shots=None) needs a BitstringEvaluator with diagonal_terms "
+                "(DiagonalEnergyBitstringEvaluator): the exact distribution would call the evaluator on all 2^n bitstrings"
+            )
 
     def evaluate_circuits(self, circuits: list, parameter_values: list[list[float]]) -> list[float]:
+        if self._sampler_shots is None:
+            return self._exact(circuits, parameter_values, self._diagonal_op, "cvar")
         n = self.n_qubits
         vectorised = getattr(self._bitstring_evaluator, "evaluate_states", None)
         if vectorised is None:  # the reference contract: one call of the user's function per distinct bitstring

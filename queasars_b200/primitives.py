@@ -26,6 +26,7 @@ import numpy as np
 
 from . import _native
 from . import containers as ct
+from . import expectation as ex
 from .batching import CoalescingQueue
 from .engine import Engine, HamiltonianHandle, PlanHandle
 from .gate_list import from_circuit_or_none, from_circuit
@@ -605,7 +606,63 @@ class B200SamplerV2(_B200Primitive):
             raise ValueError("all circuits of one sampler submission must act on the same number of qubits")
         return np.asarray(self._submit(("smp", int(shots), widths.pop()), (circuits, parameter_values)))
 
+    def cvar_values(self, circuits, parameter_values, operator, alpha: float) -> np.ndarray:
+        """Exact (shot-free) CVaR(alpha) of the diagonal ``operator`` on every circuit's full distribution |psi|^2:
+        ``expectation.lower_tail_expectation_arrays(|psi|^2, E, alpha)`` over all 2^n basis states, computed on the device
+        (fast path of the sampler evaluators with ``sampler_shots=None``).  float64 array [len(circuits)]."""
+        return self._exact("cvar", circuits, parameter_values, operator, float(alpha))
+
+    def _exact(self, kind: str, circuits, parameter_values, operator, alpha: float) -> np.ndarray:
+        """``kind`` "cvar": ``Engine.cvar``; "exp": sum_k |psi_k|^2 E(k) through ``Engine.expectation`` (the fused diagonal
+        expectation of the last sweep)."""
+        circuits, parameter_values = list(circuits), list(parameter_values)
+        if len(circuits) != len(parameter_values):
+            raise ValueError(f"{len(circuits)} circuits but {len(parameter_values)} parameter vectors")
+        ex.check_alpha(alpha)
+        if not circuits:
+            return np.zeros(0)
+        widths = {_width(c) for c in circuits}
+        if len(widths) != 1:
+            raise ValueError("all circuits of one sampler submission must act on the same number of qubits")
+        width = widths.pop()
+        if width != int(operator.num_qubits):
+            raise ValueError(f"the circuits act on {width} qubits, the operator on {int(operator.num_qubits)}")
+        if self._needs_sharding(width):
+            raise NotImplementedError(
+                f"exact CVaR / expectation values need the whole {width}-qubit statevector on one device; a state that must be sharded "
+                "over several GPUs is only supported with shots"
+            )
+        fp = _operator_fingerprint(operator)
+        if not self.hamiltonian_for(operator, build_table=(False if kind == "cvar" else None), fingerprint=fp).diagonal:
+            raise ValueError("Operator string contains non-diagonal terms")
+        return np.asarray(self._submit((kind, id(operator), fp, alpha, width), (operator, circuits, parameter_values)), dtype=np.float64)
+
+    def _execute_exact(self, key, payloads):
+        kind, _, fp, alpha, _ = key
+        operator = payloads[0][0]
+        circuits, values, sizes = [], [], []
+        for _, circs, vals in payloads:
+            sizes.append(len(circs))
+            circuits.extend(circs)
+            values.extend(vals)
+        resolved = self._resolve_all(circuits, values, probabilities_only=True)
+
+        def call(slot, plans, params):
+            engine = self.engines[slot]
+            if kind == "cvar":
+                return list(engine.cvar(plans, params, self.hamiltonian_for(operator, build_table=False, slot=slot, fingerprint=fp), alpha))
+            return list(engine.expectation(plans, params, self.hamiltonian_for(operator, slot=slot, fingerprint=fp)))
+
+        flat = self._run_per_device(resolved, call)
+        out, pos = [], 0
+        for n in sizes:
+            out.append(np.asarray(flat[pos : pos + n], dtype=np.float64))
+            pos += n
+        return out
+
     def _execute(self, key, payloads):
+        if key[0] in ("cvar", "exp"):
+            return self._execute_exact(key, payloads)
         shots = key[1]
         circuits, values, sizes = [], [], []
         for circs, vals in payloads:
