@@ -185,6 +185,27 @@ int qb_statevector(qb_context* ctx, int64_t plan_id, const double* params, int n
 int qb_evaluate_cvar(qb_context* ctx, int batch, const int64_t* plan_ids, const double* params,
                      const int64_t* param_offsets, int64_t ham_id, double alpha, double* out_values);
 
+/* --- observable sets ------------------------------------------------------------------------------------
+ * Several observables H_j = sum_t c_{j,t} P_t evaluated on one simulated state (EstimatorV2 pubs with an array of observables).
+ * Observable j owns the terms term_offsets[j] .. term_offsets[j+1]-1 of the mask / coefficient arrays (term_offsets[0] == 0).
+ * qb_observables_create builds the union of the distinct (x, z) strings of all observables, the rows that combine them
+ * (duplicate strings of one observable summed, ascending union order), and plans the strings' x-mask groups into tile sweeps as
+ * qb_hamiltonian_create does.  coeff_im may be null: every P_t is Hermitian, so only Re(c_{j,t}) enters Re<psi|H_j|psi>.
+ * QB_ERR_INVALID for n_obs < 1, decreasing offsets or a string outside the register.
+ * qb_evaluate_observables: out_values[i * n_obs + j] = Re <psi_i|H_j|psi_i> = sum_t Re(c_{j,t}) <psi_i|P_t|psi_i> (row-major,
+ * batch x n_obs), the semantics of qb_evaluate_expectation per observable.  Every distinct string is reduced once per state:
+ * one read of the state per tile sweep of x-mask groups (plus two reads per 8 strings of a group wider than a tile), each
+ * string into its own per-CTA partials, summed in a fixed order -- no atomics, bit-identical across runs, batch compositions
+ * and workspace limits.  A list that does not fit the workspace is evaluated in chunks; QB_ERR_MEMORY (with byte counts) only
+ * when one statevector and its scratch do not fit.  QB_ERR_INVALID when a plan's width differs from the set's or a plan's
+ * width or dtype from the first plan's. */
+int qb_observables_create(qb_context* ctx, int n_qubits, int n_obs, const int64_t* term_offsets /* n_obs + 1 */,
+                          const uint64_t* x_masks, const uint64_t* z_masks, const double* coeff_re, const double* coeff_im,
+                          int64_t* obs_id);
+int qb_observables_destroy(qb_context* ctx, int64_t obs_id);
+int qb_evaluate_observables(qb_context* ctx, int batch, const int64_t* plan_ids, const double* params,
+                            const int64_t* param_offsets, int64_t obs_id, double* out_values /* batch * n_obs, row-major */);
+
 /* One evaluate_circuits() list split over several GPUs of one process (the device sets of queasars_b200/primitives.py: the
  * reference wraps ONE primitive in a ThreadPoolExecutor, evqe.py:232-236): entry i of every array belongs to context ctxs[i] and
  * has the meaning of the corresponding qb_evaluate_expectation argument.  Every context evaluates its share on its own host

@@ -53,6 +53,9 @@ def _declare(lib):
         "qb_context_sm_count": [c_void_p],
         "qb_sample": [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p],
         "qb_evaluate_cvar": [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int64, c_double, c_void_p],
+        "qb_observables_create": [c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, P(c_int64)],
+        "qb_observables_destroy": [c_void_p, c_int64],
+        "qb_evaluate_observables": [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int64, c_void_p],
         "qb_statevector": [c_void_p, c_int64, c_void_p, c_int, c_void_p],
         "qb_batch_create": [c_void_p, c_int, c_void_p, c_int64, P(c_int64)],
         "qb_batch_set_params": [c_void_p, c_int64, c_void_p, c_void_p],
@@ -92,6 +95,7 @@ EXPORTED_SYMBOLS = (
     "qb_device_count qb_context_create qb_context_destroy qb_last_error qb_context_stream qb_context_launch_count "
     "qb_context_set_workspace_limit qb_context_workspace qb_context_synchronize qb_context_set_index_width qb_plan_create qb_plan_destroy qb_plan_set_prefix qb_hamiltonian_create "
     "qb_hamiltonian_destroy qb_hamiltonian_diag_energies qb_evaluate_expectation qb_sample qb_evaluate_cvar qb_statevector "
+    "qb_observables_create qb_observables_destroy qb_evaluate_observables "
     "qb_evaluate_expectation_multi qb_evaluate_expectation_submit qb_evaluate_expectation_collect qb_context_sm_count "
     "qb_batch_create qb_batch_set_params qb_batch_run qb_batch_run_timed qb_batch_read qb_batch_destroy qb_batch_stats "
     "qb_apply_plan_device qb_expectation_device qb_sample_device qb_swap_global_p2p qb_record_sizes "

@@ -49,31 +49,41 @@ class DataBin:
 
 
 class ShotRegister:
-    """Shot outcomes of one classical register (upstream ``BitArray``): basis-state indices per shot."""
+    """Shot outcomes of one classical register (upstream ``BitArray``): basis-state indices per shot.  ``shape``: the pub's
+    parameter shape; ``indices`` is then ``shape + (num_shots,)`` and ``loc`` picks one position of it (``loc=None`` pools
+    every position, as upstream's ``BitArray`` does)."""
 
-    def __init__(self, indices: np.ndarray, num_bits: int):
-        self._indices = np.asarray(indices, dtype=np.int64).reshape(-1)
+    def __init__(self, indices: np.ndarray, num_bits: int, shape: tuple = ()):
+        self.shape = tuple(int(s) for s in shape)
+        self._indices = np.asarray(indices, dtype=np.int64).reshape(self.shape + (-1,) if self.shape else (-1,))
         self.num_bits = int(num_bits)
 
     @property
     def num_shots(self) -> int:
-        return int(self._indices.size)
+        return int(self._indices.shape[-1])
 
     @property
     def indices(self) -> np.ndarray:
         return self._indices
 
-    def get_int_counts(self) -> dict[int, int]:
-        vals, cnts = np.unique(self._indices, return_counts=True)
+    def _select(self, loc) -> np.ndarray:
+        if loc is None:
+            return self._indices.reshape(-1)
+        if not self.shape:
+            raise IndexError("a register of shape () has no positions to select")
+        return np.asarray(self._indices[loc], dtype=np.int64).reshape(-1)
+
+    def get_int_counts(self, loc=None) -> dict[int, int]:
+        vals, cnts = np.unique(self._select(loc), return_counts=True)
         return {int(v): int(c) for v, c in zip(vals, cnts)}
 
-    def get_counts(self) -> dict[str, int]:
+    def get_counts(self, loc=None) -> dict[str, int]:
         width = self.num_bits
-        return {format(v, f"0{width}b"): c for v, c in self.get_int_counts().items()}
+        return {format(v, f"0{width}b"): c for v, c in self.get_int_counts(loc).items()}
 
-    def get_bitstrings(self) -> list[str]:
+    def get_bitstrings(self, loc=None) -> list[str]:
         width = self.num_bits
-        return [format(int(v), f"0{width}b") for v in self._indices]
+        return [format(int(v), f"0{width}b") for v in self._select(loc)]
 
 
 class PubResult:

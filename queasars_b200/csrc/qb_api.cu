@@ -141,6 +141,17 @@ struct Ham {
     }
 };
 
+// A set of observables evaluated together (qb_evaluate_observables): the union of their distinct Pauli strings, grouped by
+// x mask and planned into tile sweeps like a Hamiltonian's groups, plus the CSR rows that combine string values into observables.
+struct Obs {
+    int n_qubits = 0, n_obs = 0, n_terms = 0, n_eff = 0;
+    std::vector<qb::ExpTileSweep> tile_sweeps;
+    std::vector<std::pair<int, int>> sweep_terms;  // device term range of every tile sweep
+    std::vector<qb::TermGroup> generic;            // groups whose x mask does not fit a tile (term ranges on the device)
+    DevBuf groups, z, im, sign, row_begin, cols, coeff;
+    ~Obs() { groups.release(), z.release(), im.release(), sign.release(), row_begin.release(), cols.release(), coeff.release(); }
+};
+
 // A set of circuit evaluations resident on the device.
 struct DeviceBatch {
     int batch = 0, n_eff = 0, n_qubits = 0, dtype = 0, tile_bits = QB_TILE_BITS, reg_bits = 4, max_sweeps = 0;
@@ -257,6 +268,7 @@ struct qb_context {
     std::mutex mu;
     std::map<int64_t, std::unique_ptr<Plan>> plans;
     std::map<int64_t, std::unique_ptr<Ham>> hams;
+    std::map<int64_t, std::unique_ptr<Obs>> observables;
     std::map<int64_t, std::unique_ptr<DeviceBatch>> batches;
     HostBuf pin_in, pin_out, pin_entries;
     cudaEvent_t pin_entries_done = nullptr;
@@ -888,6 +900,115 @@ int ensure_cvar_order(qb_context* ctx, Ham& ham, int n_eff, bool sorted) {
     return rc;
 }
 
+// Pauli strings grouped by x mask, groups in first-appearance order: xs[g] and the string indices of each group
+int group_by_xmask(int n_qubits, int n_terms, const uint64_t* x_masks, const uint64_t* z_masks, std::vector<uint64_t>& xs,
+                   std::vector<std::vector<int>>& members) {
+    for (int t = 0; t < n_terms; ++t) {
+        if ((x_masks[t] | z_masks[t]) >> n_qubits) return fail(QB_ERR_INVALID, "Pauli term acts outside the register");
+        size_t g = 0;
+        for (; g < xs.size(); ++g)
+            if (xs[g] == x_masks[t]) break;
+        if (g == xs.size()) xs.push_back(x_masks[t]), members.emplace_back();
+        members[g].push_back(t);
+    }
+    return QB_OK;
+}
+
+// Schedule x-mask groups into tile sweeps: every sweep takes, in order, the pending groups whose flipped qubits still fit one
+// 2^kExpTileBits tile next to qubits 0 .. QB_LOW_BITS-1; a group that does not fit a tile on its own is left to a generic kernel.
+// Group records of the sweeps are laid out sweep after sweep, in `sweep_groups` order (group_begin / group_end count them).
+struct TilePlan {
+    std::vector<qb::ExpTileSweep> sweeps;
+    std::vector<std::vector<int>> sweep_groups;  // group indices of every sweep
+    std::vector<uint32_t> xloc;                  // per group: x mask in the tile-local bit positions of its sweep
+    std::vector<int> generic;                    // groups whose x mask does not fit a tile
+};
+
+TilePlan plan_tile_sweeps(int n_eff, const std::vector<uint64_t>& xmask, std::vector<int> pending) {
+    const int K = qb::kExpTileBits, low = QB_LOW_BITS;
+    TilePlan tp;
+    tp.xloc.assign(xmask.size(), 0);
+    int n_records = 0;
+    while (!pending.empty()) {
+        uint64_t tile = (uint64_t(1) << low) - 1;
+        std::vector<int> chosen, rest;
+        for (int g : pending) {
+            const uint64_t want = tile | xmask[g];
+            if (__builtin_popcountll(want) <= K) tile = want, chosen.push_back(g);
+            else rest.push_back(g);
+        }
+        if (chosen.empty()) {  // the first pending group alone does not fit a tile: generic kernel
+            tp.generic.push_back(pending.front());
+            pending.erase(pending.begin());
+            continue;
+        }
+        for (int q = 0; __builtin_popcountll(tile) < K; ++q) tile |= uint64_t(1) << q;
+        qb::ExpTileSweep sw{};
+        int pos_of[64];
+        for (int q = 0, i = 0; q < n_eff; ++q)
+            if ((tile >> q) & 1) pos_of[q] = i, sw.tile_qubits[i++] = q;
+        sw.group_begin = n_records;
+        for (int g : chosen)
+            for (int q = 0; q < n_eff; ++q)
+                if ((xmask[g] >> q) & 1) tp.xloc[g] |= 1u << pos_of[q];
+        n_records += int(chosen.size());
+        sw.group_end = n_records;
+        tp.sweeps.push_back(sw);
+        tp.sweep_groups.push_back(chosen);
+        pending = rest;
+    }
+    return tp;
+}
+
+Obs* find_obs(qb_context* ctx, int64_t id) {
+    auto it = ctx->observables.find(id);
+    return it == ctx->observables.end() ? nullptr : it->second.get();
+}
+
+// partial-sum scratch of one term-resolved launch: terms beyond it are evaluated in further launches over the same state
+constexpr size_t kTermPartialBytes = size_t(256) << 20;
+
+// <P_t> of every string of `ob` for the n resident states of `b` into d_terms[pos * n_terms + slot]
+template <typename T>
+int launch_terms_t(qb_context* ctx, const DeviceBatch& b, const Obs& ob, double* d_partials, size_t partial_bytes, double* d_terms) {
+    using C = typename qb::Cx<T>::type;
+    const int n = b.batch;
+    const uint64_t size = uint64_t(1) << b.n_eff;
+    const C* states = b.states.as<C>();
+    // terms [lo, hi) in pieces whose partials (n states x terms x count) fit the scratch; a term's value does not depend on the piece
+    auto pieces = [&](int lo, int hi, uint64_t count, const std::function<int(int, int)>& run) -> int {
+        const int per = int(std::max<uint64_t>(1, std::min<uint64_t>(uint64_t(hi - lo), partial_bytes / (sizeof(double) * count * uint64_t(n)))));
+        for (int t0 = lo; t0 < hi; t0 += per) {
+            const int t1 = std::min(hi, t0 + per);
+            QB_TRY(run(t0, t1));
+            qb::reduce_term_partials_kernel<<<dim3(unsigned(t1 - t0), unsigned(n)), 256, 0, ctx->stream>>>(
+                d_partials, int64_t(count), t1 - t0, ob.sign.as<double>(), t0, d_terms, ob.n_terms);
+            QB_TRY(check_launch(ctx, "reduce_term_partials_kernel"));
+        }
+        return QB_OK;
+    };
+    const uint64_t tiles = size >> qb::kExpTileBits;
+    const size_t smem = sizeof(C) << qb::kExpTileBits;
+    for (size_t s = 0; s < ob.tile_sweeps.size(); ++s) {
+        const auto& sw = ob.tile_sweeps[s];
+        QB_TRY(pieces(ob.sweep_terms[s].first, ob.sweep_terms[s].second, tiles, [&](int t0, int t1) {
+            qb::expect_terms_tile_kernel<T><<<dim3(unsigned(tiles), unsigned(n)), 256, smem, ctx->stream>>>(
+                states, size, b.n_eff, sw, ob.groups.as<qb::TermGroup>(), ob.z.as<uint64_t>(), ob.im.as<int8_t>(), t0, t1, d_partials);
+            return check_launch(ctx, "expect_terms_tile_kernel");
+        }));
+    }
+    const uint64_t blocks = std::min<uint64_t>(1024, std::max<uint64_t>(1, size / 256));
+    for (const auto& g : ob.generic) {
+        if (g.xmask >> b.n_eff) return fail(QB_ERR_INVALID, "Pauli term flips a qubit outside the statevector");
+        QB_TRY(pieces(g.term_begin, g.term_end, blocks, [&](int t0, int t1) {
+            qb::expect_terms_group_kernel<T><<<dim3(unsigned(blocks), unsigned(n)), 256, 0, ctx->stream>>>(
+                states, size, size, g.xmask, ob.z.as<uint64_t>(), ob.im.as<int8_t>(), t0, t1, t0, t1 - t0, d_partials);
+            return check_launch(ctx, "expect_terms_group_kernel");
+        }));
+    }
+    return QB_OK;
+}
+
 }  // namespace
 
 // =====================================================================================================
@@ -971,6 +1092,7 @@ int qb_context_destroy(qb_context* ctx) {
     ctx->batches.clear();
     ctx->plans.clear();
     ctx->hams.clear();
+    ctx->observables.clear();
     ctx->pin_in.release(), ctx->pin_out.release(), ctx->scratch.release();
     if (ctx->pin_in_done) cudaEventDestroy(ctx->pin_in_done);
     if (ctx->pin_entries_done) cudaEventDestroy(ctx->pin_entries_done);
@@ -1155,14 +1277,7 @@ int qb_hamiltonian_create(qb_context* ctx, int n_qubits, int n_terms, const uint
     // group by x mask, keeping first-appearance order; weights w = coeff * i^{#Y}
     std::vector<uint64_t> xs;
     std::vector<std::vector<int>> members;
-    for (int t = 0; t < n_terms; ++t) {
-        if ((x_masks[t] | z_masks[t]) >> n_qubits) return fail(QB_ERR_INVALID, "Pauli term acts outside the register");
-        size_t g = 0;
-        for (; g < xs.size(); ++g)
-            if (xs[g] == x_masks[t]) break;
-        if (g == xs.size()) xs.push_back(x_masks[t]), members.emplace_back();
-        members[g].push_back(t);
-    }
+    QB_TRY(group_by_xmask(n_qubits, n_terms, x_masks, z_masks, xs, members));
     std::vector<uint64_t> dz;
     std::vector<double> dc;
     for (size_t g = 0; g < xs.size(); ++g) {
@@ -1201,12 +1316,16 @@ int qb_hamiltonian_create(qb_context* ctx, int n_qubits, int n_terms, const uint
         QB_CUDA(cudaStreamSynchronize(ctx->stream));
     }
     {   // schedule the non-diagonal x-mask groups into tile sweeps
-        const int K = qb::kExpTileBits, low = QB_LOW_BITS;
-        const int n_eff = std::max(n_qubits, K);
+        const int n_eff = std::max(n_qubits, qb::kExpTileBits);
         ham->tile_n_eff = n_eff;
+        std::vector<uint64_t> gx(ham->groups.size());
         std::vector<int> pending;
-        for (size_t g = 0; g < ham->groups.size(); ++g)
-            if (ham->groups[g]->xmask != 0) pending.push_back(int(g));
+        for (size_t g = 0; g < ham->groups.size(); ++g) {
+            gx[g] = ham->groups[g]->xmask;
+            if (gx[g] != 0) pending.push_back(int(g));
+        }
+        TilePlan tp = plan_tile_sweeps(n_eff, gx, pending);
+        ham->tile_sweeps = tp.sweeps, ham->tile_sweep_groups = tp.sweep_groups, ham->generic_groups = tp.generic;
         std::vector<qb::ExpTileGroup> tgroups;
         std::vector<uint64_t> tz;
         std::vector<double> twr, twi;
@@ -1226,29 +1345,10 @@ int qb_hamiltonian_create(qb_context* ctx, int n_qubits, int n_terms, const uint
                 host_z[slot].push_back(z_masks[t]), host_wr[slot].push_back(r), host_wi[slot].push_back(i);
             }
         }
-        while (!pending.empty()) {
-            uint64_t tile = (uint64_t(1) << low) - 1;
-            std::vector<int> chosen, rest;
-            for (int g : pending) {
-                const uint64_t want = tile | ham->groups[g]->xmask;
-                if (__builtin_popcountll(want) <= K) tile = want, chosen.push_back(g);
-                else rest.push_back(g);
-            }
-            if (chosen.empty()) {  // the first pending group alone does not fit a tile: generic kernel
-                ham->generic_groups.push_back(pending.front());
-                pending.erase(pending.begin());
-                continue;
-            }
-            for (int q = 0; __builtin_popcountll(tile) < K; ++q) tile |= uint64_t(1) << q;
-            qb::ExpTileSweep sw{};
-            int pos_of[64];
-            for (int q = 0, i = 0; q < n_eff; ++q)
-                if ((tile >> q) & 1) pos_of[q] = i, sw.tile_qubits[i++] = q;
-            sw.group_begin = int(tgroups.size());
+        for (const auto& chosen : tp.sweep_groups)
             for (int g : chosen) {
                 qb::ExpTileGroup tg{};
-                for (int q = 0; q < n_eff; ++q)
-                    if ((ham->groups[g]->xmask >> q) & 1) tg.xloc |= 1u << pos_of[q];
+                tg.xloc = tp.xloc[g];
                 tg.term_begin = int(tz.size());
                 tz.insert(tz.end(), host_z[g].begin(), host_z[g].end());
                 twr.insert(twr.end(), host_wr[g].begin(), host_wr[g].end());
@@ -1257,11 +1357,6 @@ int qb_hamiltonian_create(qb_context* ctx, int n_qubits, int n_terms, const uint
                 tg.trivial = (host_z[g].size() == 1 && host_z[g][0] == 0) ? 1 : 0;
                 tgroups.push_back(tg);
             }
-            sw.group_end = int(tgroups.size());
-            ham->tile_sweeps.push_back(sw);
-            ham->tile_sweep_groups.push_back(chosen);
-            pending = rest;
-        }
         if (!tgroups.empty()) {
             QB_TRY(upload(ctx, ham->tile_groups, tgroups.data(), sizeof(qb::ExpTileGroup) * tgroups.size()));
             QB_TRY(upload(ctx, ham->tile_z, tz.data(), sizeof(uint64_t) * tz.size()));
@@ -1310,6 +1405,96 @@ int qb_hamiltonian_diag_energies(qb_context* ctx, int64_t ham_id, int64_t n_stat
     QB_CUDA(cudaStreamSynchronize(ctx->stream));
     std::memcpy(out_energies, ctx->pin_out.p, bytes);
     return QB_OK;
+}
+
+// ---- observable sets ----------------------------------------------------------------------------------
+int qb_observables_create(qb_context* ctx, int n_qubits, int n_obs, const int64_t* term_offsets, const uint64_t* x_masks,
+                          const uint64_t* z_masks, const double* coeff_re, const double* coeff_im, int64_t* obs_id) {
+    (void)coeff_im;  // every string is Hermitian, <P_t> is real: Re(c <P_t>) = Re(c) <P_t>
+    if (!ctx || !term_offsets || !obs_id) return fail(QB_ERR_INVALID, "null argument");
+    if (n_qubits < 1 || n_qubits > 40) return fail(QB_ERR_INVALID, "bad observable width");
+    if (n_obs < 1) return fail(QB_ERR_INVALID, "an observable set needs at least one observable");
+    if (term_offsets[0] != 0) return fail(QB_ERR_INVALID, "term_offsets[0] must be 0");
+    for (int j = 0; j < n_obs; ++j)
+        if (term_offsets[j + 1] < term_offsets[j]) return fail(QB_ERR_INVALID, "term_offsets must not decrease");
+    const int64_t total = term_offsets[n_obs];
+    if (total > (int64_t(1) << 30)) return fail(QB_ERR_INVALID, "too many terms");
+    if (total > 0 && (!x_masks || !z_masks || !coeff_re)) return fail(QB_ERR_INVALID, "null argument");
+    // union of the distinct (x, z) strings in first-appearance order; CSR rows over union indices, duplicates summed
+    std::map<std::pair<uint64_t, uint64_t>, int> index_of;
+    std::vector<uint64_t> ux, uz;
+    std::vector<int64_t> row_begin(size_t(n_obs) + 1, 0);
+    std::vector<int32_t> cols;
+    std::vector<double> coeff;
+    for (int j = 0; j < n_obs; ++j) {
+        std::map<int, double> row;  // union index -> coefficient (ascending term order)
+        for (int64_t t = term_offsets[j]; t < term_offsets[j + 1]; ++t) {
+            if ((x_masks[t] | z_masks[t]) >> n_qubits) return fail(QB_ERR_INVALID, "Pauli term acts outside the register");
+            auto ins = index_of.emplace(std::make_pair(x_masks[t], z_masks[t]), int(ux.size()));
+            if (ins.second) ux.push_back(x_masks[t]), uz.push_back(z_masks[t]);
+            row[ins.first->second] += coeff_re[t];
+        }
+        for (const auto& e : row) cols.push_back(e.first), coeff.push_back(e.second);
+        row_begin[j + 1] = int64_t(cols.size());
+    }
+    auto ob = std::make_unique<Obs>();
+    ob->n_qubits = n_qubits, ob->n_obs = n_obs, ob->n_terms = int(ux.size());
+    ob->n_eff = std::max(n_qubits, qb::kExpTileBits);
+    std::vector<uint64_t> xs;
+    std::vector<std::vector<int>> members;
+    QB_TRY(group_by_xmask(n_qubits, ob->n_terms, ux.data(), uz.data(), xs, members));
+    std::vector<int> pending(xs.size());
+    std::iota(pending.begin(), pending.end(), 0);
+    for (size_t g = 0; g < xs.size(); ++g)  // the diagonal group (|psi_k|^2, no partner) first
+        if (xs[g] == 0) std::rotate(pending.begin(), pending.begin() + g, pending.begin() + g + 1);
+    const TilePlan tp = plan_tile_sweeps(ob->n_eff, xs, pending);
+    // device order of the strings: sweep after sweep, group after group, then the generic groups
+    std::vector<int> slot_of(ux.size());
+    std::vector<uint64_t> dz;
+    std::vector<int8_t> dim;
+    std::vector<double> dsign;
+    std::vector<qb::TermGroup> records;
+    auto place = [&](int g) {
+        qb::TermGroup rec{};
+        rec.xmask = xs[g], rec.xloc = tp.xloc[g], rec.term_begin = int(dz.size()), rec.real_only = 1;
+        for (int u : members[g]) {
+            const int ny = __builtin_popcountll(ux[u] & uz[u]) & 3;
+            slot_of[u] = int(dz.size());
+            dz.push_back(uz[u]), dim.push_back(int8_t(ny & 1)), dsign.push_back((ny == 1 || ny == 2) ? -1.0 : 1.0);
+            if (ny & 1) rec.real_only = 0;
+        }
+        rec.term_end = int(dz.size());
+        return rec;
+    };
+    ob->tile_sweeps = tp.sweeps;
+    for (const auto& chosen : tp.sweep_groups) {
+        const int first = int(dz.size());
+        for (int g : chosen) records.push_back(place(g));
+        ob->sweep_terms.emplace_back(first, int(dz.size()));
+    }
+    for (int g : tp.generic) ob->generic.push_back(place(g));
+    for (auto& c : cols) c = slot_of[c];
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    QB_ON_DEVICE(ctx);
+    QB_TRY(upload(ctx, ob->groups, records.data(), sizeof(qb::TermGroup) * records.size()));
+    QB_TRY(upload(ctx, ob->z, dz.data(), sizeof(uint64_t) * dz.size()));
+    QB_TRY(upload(ctx, ob->im, dim.data(), dim.size()));
+    QB_TRY(upload(ctx, ob->sign, dsign.data(), sizeof(double) * dsign.size()));
+    QB_TRY(upload(ctx, ob->row_begin, row_begin.data(), sizeof(int64_t) * row_begin.size()));
+    QB_TRY(upload(ctx, ob->cols, cols.data(), sizeof(int32_t) * cols.size()));
+    QB_TRY(upload(ctx, ob->coeff, coeff.data(), sizeof(double) * coeff.size()));
+    QB_CUDA(cudaStreamSynchronize(ctx->stream));
+    *obs_id = ctx->next_id++;
+    ctx->observables[*obs_id] = std::move(ob);
+    return QB_OK;
+}
+
+int qb_observables_destroy(qb_context* ctx, int64_t obs_id) {
+    if (!ctx) return fail(QB_ERR_INVALID, "null context");
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    QB_ON_DEVICE(ctx);
+    cudaStreamSynchronize(ctx->stream);
+    return ctx->observables.erase(obs_id) ? QB_OK : fail(QB_ERR_NOT_FOUND, "unknown observable set id");
 }
 
 // ---- resident batches -----------------------------------------------------------------------------------
@@ -1569,6 +1754,65 @@ int qb_evaluate_cvar(qb_context* ctx, int batch, const int64_t* plan_ids, const 
         QB_CUDA(cudaStreamSynchronize(ctx->stream));
         const double* sorted_out = static_cast<const double*>(ctx->pin_out.p);
         for (int pos = 0; pos < n; ++pos) out_values[lo + b.order[pos]] = sorted_out[pos];
+    }
+    return QB_OK;
+}
+
+int qb_evaluate_observables(qb_context* ctx, int batch, const int64_t* plan_ids, const double* params, const int64_t* param_offsets,
+                            int64_t obs_id, double* out_values) {
+    if (!ctx || !plan_ids || !param_offsets || !out_values) return fail(QB_ERR_INVALID, "null argument");
+    if (batch <= 0) return QB_OK;
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    QB_ON_DEVICE(ctx);
+    const Obs* ob = find_obs(ctx, obs_id);
+    if (!ob) return fail(QB_ERR_NOT_FOUND, "unknown observable set id");
+    const Plan* first = find_plan(ctx, plan_ids[0]);
+    if (!first) return fail(QB_ERR_NOT_FOUND, "unknown plan id " + std::to_string(plan_ids[0]));
+    for (int i = 0; i < batch; ++i) {
+        const Plan* pl = find_plan(ctx, plan_ids[i]);
+        if (!pl) return fail(QB_ERR_NOT_FOUND, "unknown plan id " + std::to_string(plan_ids[i]));
+        if (pl->n_qubits != ob->n_qubits)
+            return fail(QB_ERR_INVALID, "observables act on " + std::to_string(ob->n_qubits) + " qubits, circuit " + std::to_string(i) + " on " +
+                                            std::to_string(pl->n_qubits));
+        if (pl->n_eff != first->n_eff || pl->dtype != first->dtype)
+            return fail(QB_ERR_INVALID, "all plans of one observables call must share state width and dtype");
+    }
+    // per state: the statevector, its string values, its observable values and the partials of at least one string
+    const uint64_t size = uint64_t(1) << first->n_eff;
+    const uint64_t count = std::max<uint64_t>(size >> qb::kExpTileBits, std::min<uint64_t>(1024, std::max<uint64_t>(1, size / 256)));
+    const size_t state_bytes = size_t(size) * amp_bytes(first->dtype);
+    const size_t values_bytes = sizeof(double) * (size_t(ob->n_terms) + size_t(ob->n_obs));
+    const size_t per_state = state_bytes + values_bytes + sizeof(double) * size_t(count);
+    const size_t limit = workspace_limit_of(ctx);
+    if (per_state > limit)
+        return fail(QB_ERR_MEMORY, "one statevector (" + std::to_string(state_bytes) + " bytes) and its observable scratch (" +
+                                       std::to_string(per_state - state_bytes) + " bytes) do not fit the workspace of " + std::to_string(limit) + " bytes");
+    const int chunk = int(std::min<size_t>({size_t(batch), max_batch_for(ctx, first), limit / per_state}));
+    const size_t n_out = size_t(ob->n_obs);
+    for (int lo = 0; lo < batch; lo += chunk) {
+        const int n = std::min(chunk, batch - lo);
+        DeviceBatch& b = ctx->oneshot;
+        QB_TRY(build_batch(ctx, b, n, plan_ids + lo, nullptr, nullptr, 1, 0));
+        QB_TRY(batch_upload_params(ctx, b, params, param_offsets + lo));
+        QB_TRY(launch_circuits(ctx, b, nullptr));
+        const size_t terms_bytes = sizeof(double) * size_t(n) * size_t(ob->n_terms), out_bytes = sizeof(double) * size_t(n) * n_out;
+        const size_t room = limit - size_t(n) * state_bytes - terms_bytes - out_bytes;  // >= n * count * 8 by the chunk size
+        const size_t partial_bytes = std::max(sizeof(double) * size_t(count) * size_t(n), std::min(kTermPartialBytes, room));
+        QB_TRY(ctx->scratch.reserve(terms_bytes + out_bytes + partial_bytes + 16));
+        double* d_terms = ctx->scratch.as<double>();
+        double* d_out = d_terms + size_t(n) * size_t(ob->n_terms);
+        double* d_partials = d_out + size_t(n) * n_out;
+        QB_TRY(b.dtype == QB_C128 ? launch_terms_t<double>(ctx, b, *ob, d_partials, partial_bytes, d_terms)
+                                  : launch_terms_t<float>(ctx, b, *ob, d_partials, partial_bytes, d_terms));
+        qb::combine_observables_kernel<<<dim3(unsigned((n_out + 127) / 128), unsigned(n)), 128, 0, ctx->stream>>>(
+            d_terms, ob->n_terms, ob->row_begin.as<int64_t>(), ob->cols.as<int32_t>(), ob->coeff.as<double>(), ob->n_obs, d_out);
+        QB_TRY(check_launch(ctx, "combine_observables_kernel"));
+        QB_TRY(ctx->pin_out.reserve(out_bytes));
+        QB_CUDA(cudaMemcpyAsync(ctx->pin_out.p, d_out, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+        QB_CUDA(cudaStreamSynchronize(ctx->stream));
+        const double* sorted = static_cast<const double*>(ctx->pin_out.p);
+        for (int pos = 0; pos < n; ++pos)
+            std::memcpy(out_values + size_t(lo + b.order[pos]) * n_out, sorted + size_t(pos) * n_out, sizeof(double) * n_out);
     }
     return QB_OK;
 }

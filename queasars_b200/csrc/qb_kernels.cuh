@@ -1023,6 +1023,213 @@ reduce_partials_kernel(const double* partials, int64_t stride, int64_t count, do
 }
 
 // ---------------------------------------------------------------------------------------------------
+// term-resolved expectation (qb_evaluate_observables): <P_t> of every distinct Pauli string P_t = i^{#Y} X^x Z^z of a set of
+// observables, one value per string, from one read of the state per tile sweep of x-mask groups.  With the pair product
+// p_k = psi_k conj(psi_{k^x}):   <P_t> = sign_t * sum_k (-1)^{pc(k & z_t)} * (#Y_t odd ? Im p_k : Re p_k),
+// sign_t = -1 for #Y = 1, 2 (mod 4), +1 otherwise (applied by reduce_term_partials_kernel).  Every CTA writes one partial per
+// (term, CTA); the second stage sums them in a fixed order: no atomics, and a term's value depends on neither the other terms
+// of its launch nor the batch it is evaluated in.
+// ---------------------------------------------------------------------------------------------------
+constexpr int kTermChunk = 8;  // accumulators held in registers per pass over the thread's amplitudes
+
+struct TermGroup {
+    uint64_t xmask;     // flipped qubits
+    uint32_t xloc;      // x mask in tile-local bit positions (tile sweeps)
+    int32_t term_begin, term_end;
+    int32_t real_only;  // no string of the group has an odd number of Y: Im p_k is never read
+};
+
+// block reduction of kTermChunk accumulators (fixed tree per term); thread c < nc writes term c's CTA total to out[c * stride]
+__device__ __forceinline__ void term_chunk_store(double (&acc)[kTermChunk], int nc, double* s_red, double* __restrict__ out, uint64_t stride) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int c = 0; c < kTermChunk; ++c) {
+        const double v = warp_sum(acc[c]);
+        if (lane == 0) s_red[warp * kTermChunk + c] = v;
+    }
+    __syncthreads();
+    if (threadIdx.x < nc) {
+        const int nw = blockDim.x >> 5;
+        double total = 0.0;
+        for (int w = 0; w < nw; ++w) total += s_red[w * kTermChunk + threadIdx.x];
+        out[threadIdx.x * stride] = total;
+    }
+    __syncthreads();
+}
+
+// terms [lo, hi) of one group over the thread's kPerThread pair products; kk[i] = global index of amplitude i
+template <int kPerThread>
+__device__ __forceinline__ void term_chunks(const double (&pr)[kPerThread], const double (&pi)[kPerThread], const uint64_t (&kk)[kPerThread],
+                                            const uint64_t* __restrict__ z, const int8_t* __restrict__ im, int lo, int hi, int t0,
+                                            double* s_red, double* __restrict__ part, uint64_t count) {
+    for (int c0 = lo; c0 < hi; c0 += kTermChunk) {
+        const int nc = min(kTermChunk, hi - c0);
+        uint64_t zc[kTermChunk];
+        uint32_t ic = 0;  // bit c: term c reads Im p_k
+        double acc[kTermChunk];
+#pragma unroll
+        for (int c = 0; c < kTermChunk; ++c) {
+            zc[c] = c < nc ? z[c0 + c] : 0;
+            ic |= (c < nc && im[c0 + c] != 0) ? 1u << c : 0u;
+            acc[c] = 0.0;
+        }
+#pragma unroll
+        for (int i = 0; i < kPerThread; ++i)
+#pragma unroll
+            for (int c = 0; c < kTermChunk; ++c) {
+                const double v = ((ic >> c) & 1u) ? pi[i] : pr[i];
+                acc[c] += (__popcll(kk[i] & zc[c]) & 1) ? -v : v;
+            }
+        term_chunk_store(acc, nc, s_red, part + uint64_t(c0 - t0) * count, count);
+    }
+}
+
+// grid = (tiles, batch entries), block = 256, dynamic smem = 2^kExpTileBits amplitudes.  Terms [t0, t1) of the sweep's groups;
+// partials[((entry * (t1 - t0)) + t - t0) * tiles + tile].
+template <typename T>
+__global__ void __launch_bounds__(256)
+expect_terms_tile_kernel(const typename Cx<T>::type* __restrict__ states, uint64_t state_stride, int n_eff, ExpTileSweep sw,
+                         const TermGroup* __restrict__ groups, const uint64_t* __restrict__ z, const int8_t* __restrict__ im, int t0, int t1,
+                         double* __restrict__ partials) {
+    using C = typename Cx<T>::type;
+    extern __shared__ __align__(16) unsigned char dsm[];
+    C* tile = reinterpret_cast<C*>(dsm);
+    __shared__ double s_red[8 * kTermChunk];
+    constexpr int kPerThread = (1 << kExpTileBits) / 256;
+    const int tid = threadIdx.x;
+    uint64_t tile_mask = 0;
+#pragma unroll
+    for (int i = 0; i < kExpTileBits; ++i) tile_mask |= 1ull << sw.tile_qubits[i];
+    uint64_t base = 0;
+    {
+        uint64_t t = blockIdx.x;
+        for (int q = 0; q < n_eff; ++q)
+            if (!((tile_mask >> q) & 1ull)) {
+                base |= (t & 1ull) << q;
+                t >>= 1;
+            }
+    }
+    // element e = tid + 256 * i : the low 8 tile bits come from tid, the high ones from i
+    uint64_t g_lo = 0;
+#pragma unroll
+    for (int b = 0; b < 8; ++b) g_lo |= uint64_t((tid >> b) & 1) << sw.tile_qubits[b];
+    uint64_t kk[kPerThread];
+#pragma unroll
+    for (int i = 0; i < kPerThread; ++i) {
+        kk[i] = base | g_lo;
+#pragma unroll
+        for (int b = 8; b < kExpTileBits; ++b) kk[i] |= uint64_t((i >> (b - 8)) & 1) << sw.tile_qubits[b];
+    }
+    const C* __restrict__ st = states + blockIdx.y * state_stride;
+    C mine[kPerThread];
+#pragma unroll
+    for (int i = 0; i < kPerThread; ++i) {
+        mine[i] = ld_state(st + kk[i]);
+        tile[tid + 256 * i] = mine[i];
+    }
+    __syncthreads();
+    const uint64_t count = gridDim.x;
+    double* part = partials + uint64_t(blockIdx.y) * uint64_t(t1 - t0) * count + blockIdx.x;
+    for (int g = sw.group_begin; g < sw.group_end; ++g) {
+        const TermGroup grp = groups[g];
+        const int lo = max(grp.term_begin, t0), hi = min(grp.term_end, t1);
+        if (lo >= hi) continue;
+        double pr[kPerThread], pi[kPerThread];
+        const uint32_t hi_bits = grp.xloc >> 8;
+        if (grp.xloc == 0u) {
+            // diagonal group: p_k = |psi_k|^2
+#pragma unroll
+            for (int i = 0; i < kPerThread; ++i) {
+                pr[i] = fma(double(mine[i].x), double(mine[i].x), double(mine[i].y) * double(mine[i].y));
+                pi[i] = 0.0;
+            }
+        } else if (grp.real_only && (grp.xloc & 255u) == 0u && (hi_bits == 1u || hi_bits == 2u || hi_bits == 4u)) {
+            // the flipped bit is one of the thread's own element bits: the partner sits in this thread's registers (no
+            // shared-memory read), and only the real part of the pair product is needed
+#define QB_REG_PAIRS(S)                                                                                                \
+    _Pragma("unroll") for (int i = 0; i < kPerThread; ++i) {                                                            \
+        pr[i] = fma(double(mine[i].x), double(mine[i ^ S].x), double(mine[i].y) * double(mine[i ^ S].y));               \
+        pi[i] = 0.0;                                                                                                    \
+    }
+            if (hi_bits == 1u) { QB_REG_PAIRS(1) } else if (hi_bits == 2u) { QB_REG_PAIRS(2) } else { QB_REG_PAIRS(4) }
+#undef QB_REG_PAIRS
+        } else {
+#pragma unroll
+            for (int i = 0; i < kPerThread; ++i) {
+                const C a = mine[i];
+                const C b = tile[(tid + 256 * i) ^ grp.xloc];
+                pr[i] = fma(double(a.x), double(b.x), double(a.y) * double(b.y));
+                pi[i] = grp.real_only ? 0.0 : fma(double(a.y), double(b.x), -double(a.x) * double(b.y));
+            }
+        }
+        term_chunks(pr, pi, kk, z, im, lo, hi, t0, s_red, part, count);
+    }
+}
+
+// One group whose x mask does not fit a tile: two reads of the state per chunk of kTermChunk terms.
+// grid = (blocks, batch entries), block = 256; terms [lo, hi) of the group, partials as above with count = blocks.
+template <typename T>
+__global__ void __launch_bounds__(256)
+expect_terms_group_kernel(const typename Cx<T>::type* __restrict__ states, uint64_t state_stride, uint64_t size, uint64_t xmask,
+                          const uint64_t* __restrict__ z, const int8_t* __restrict__ im, int lo, int hi, int t0, int nt,
+                          double* __restrict__ partials) {
+    __shared__ double s_red[8 * kTermChunk];
+    const auto* state = states + blockIdx.y * state_stride;
+    const uint64_t count = gridDim.x;
+    double* part = partials + uint64_t(blockIdx.y) * uint64_t(nt) * count + blockIdx.x;
+    for (int c0 = lo; c0 < hi; c0 += kTermChunk) {
+        const int nc = min(kTermChunk, hi - c0);
+        uint64_t zc[kTermChunk];
+        uint32_t ic = 0;  // bit c: term c reads Im p_k
+        double acc[kTermChunk];
+#pragma unroll
+        for (int c = 0; c < kTermChunk; ++c) {
+            zc[c] = c < nc ? z[c0 + c] : 0;
+            ic |= (c < nc && im[c0 + c] != 0) ? 1u << c : 0u;
+            acc[c] = 0.0;
+        }
+        for (uint64_t k = blockIdx.x * uint64_t(blockDim.x) + threadIdx.x; k < size; k += uint64_t(gridDim.x) * blockDim.x) {
+            const auto a = state[k];
+            const auto b = state[k ^ xmask];
+            const double pr = fma(double(a.x), double(b.x), double(a.y) * double(b.y));
+            const double pi = fma(double(a.y), double(b.x), -double(a.x) * double(b.y));
+#pragma unroll
+            for (int c = 0; c < kTermChunk; ++c) {
+                const double v = ((ic >> c) & 1u) ? pi : pr;
+                acc[c] += (__popcll(k & zc[c]) & 1) ? -v : v;
+            }
+        }
+        term_chunk_store(acc, nc, s_red, part + uint64_t(c0 - t0) * count, count);
+    }
+}
+
+// terms[entry * terms_stride + t0 + t] = sign[t0 + t] * sum_i partials[(entry * nt + t) * count + i]  (fixed order)
+// grid = (nt, batch entries)
+__global__ void __launch_bounds__(256)
+reduce_term_partials_kernel(const double* __restrict__ partials, int64_t count, int nt, const double* __restrict__ sign, int t0,
+                            double* __restrict__ terms, int64_t terms_stride) {
+    __shared__ double s_red[8];
+    const double* p = partials + (int64_t(blockIdx.y) * nt + blockIdx.x) * count;
+    double acc = 0.0;
+    for (int64_t i = threadIdx.x; i < count; i += blockDim.x) acc += p[i];
+    const double total = block_sum(acc, s_red);
+    if (threadIdx.x == 0) terms[blockIdx.y * terms_stride + t0 + blockIdx.x] = sign[t0 + blockIdx.x] * total;
+}
+
+// out[entry * n_obs + j] = sum_e coeff[e] * terms[entry * n_terms + cols[e]] over row j's entries (ascending term order)
+// grid = (ceil(n_obs / 128), batch entries), block = 128
+__global__ void __launch_bounds__(128)
+combine_observables_kernel(const double* __restrict__ terms, int n_terms, const int64_t* __restrict__ row_begin,
+                           const int32_t* __restrict__ cols, const double* __restrict__ coeff, int n_obs, double* __restrict__ out) {
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n_obs) return;
+    const double* t = terms + int64_t(blockIdx.y) * n_terms;
+    double s = 0.0;
+    for (int64_t e = row_begin[j]; e < row_begin[j + 1]; ++e) s = fma(coeff[e], t[cols[e]], s);
+    out[int64_t(blockIdx.y) * n_obs + j] = s;
+}
+
+// ---------------------------------------------------------------------------------------------------
 // sampling: |psi|^2 chunk sums -> inclusive scan of chunk sums -> per-shot two-level search
 // ---------------------------------------------------------------------------------------------------
 constexpr int kChunkBits = 9;  // 512 amplitudes per chunk

@@ -87,6 +87,13 @@ class HamiltonianHandle:
         self.z_masks, self.coeffs, self.n_terms = z_masks, coeffs, n_terms
 
 
+class ObservablesHandle:
+    __slots__ = ("obs_id", "n_qubits", "n_obs", "diagonal", "n_terms", "__weakref__")
+
+    def __init__(self, obs_id, n_qubits, n_obs, diagonal, n_terms):
+        self.obs_id, self.n_qubits, self.n_obs, self.diagonal, self.n_terms = obs_id, n_qubits, n_obs, diagonal, n_terms
+
+
 def operator_terms(operator):
     """``SparsePauliOp``-like -> (n_qubits, x_masks, z_masks, coeffs) via the Qiskit API ``to_list()``
     (labels little-endian, right-most char = qubit 0)."""
@@ -120,6 +127,44 @@ def merge_duplicate_terms(x, z, c):
     np.add.at(summed, inverse, c)
     order = np.argsort(first)
     return uniq[order, 0].copy(), uniq[order, 1].copy(), summed[order]
+
+
+def observable_union(x, z, c, offsets):
+    """The combination ``qb_observables_create`` builds from observable j's terms ``offsets[j] .. offsets[j+1]-1``: the distinct
+    (x, z) strings in first-appearance order and CSR rows over them -> (ux, uz, row_begin, cols, coeffs), each row in ascending
+    string order with the real parts of duplicate strings summed (every string is Hermitian, so Re(c) is all that counts)."""
+    index_of: dict = {}
+    ux, uz, row_begin, cols, coeffs = [], [], [0], [], []
+    for j in range(len(offsets) - 1):
+        row: dict = {}
+        for t in range(int(offsets[j]), int(offsets[j + 1])):
+            key = (int(x[t]), int(z[t]))
+            u = index_of.setdefault(key, len(ux))
+            if u == len(ux):
+                ux.append(key[0]), uz.append(key[1])
+            row[u] = row.get(u, 0.0) + float(np.real(c[t]))
+        for u in sorted(row):
+            cols.append(u), coeffs.append(row[u])
+        row_begin.append(len(cols))
+    return (np.asarray(ux, dtype=np.uint64), np.asarray(uz, dtype=np.uint64), np.asarray(row_begin, dtype=np.int64),
+            np.asarray(cols, dtype=np.int64), np.asarray(coeffs, dtype=np.float64))
+
+
+def observable_terms(operators):
+    """Operators of one width -> (n_qubits, x, z, coeffs, offsets): the concatenated terms, duplicates merged per operator."""
+    operators = list(operators)
+    if not operators:
+        raise ValueError("an observable set needs at least one observable")
+    xs, zs, cs, offsets, width = [], [], [], [0], None
+    for op in operators:
+        n, x, z, c = operator_terms(op)
+        if width is not None and n != width:
+            raise ValueError(f"observables of one set must act on the same number of qubits ({width} and {n})")
+        width = n
+        x, z, c = merge_duplicate_terms(x, z, c)
+        xs.append(np.asarray(x, dtype=np.uint64)), zs.append(np.asarray(z, dtype=np.uint64)), cs.append(np.asarray(c, dtype=complex))
+        offsets.append(offsets[-1] + len(c))
+    return int(width), np.concatenate(xs), np.concatenate(zs), np.concatenate(cs), np.asarray(offsets, dtype=np.int64)
 
 
 @functools.lru_cache(maxsize=256)
@@ -296,6 +341,30 @@ class Engine:
         if engine_finalizer.alive:
             lib.qb_hamiltonian_destroy(ctx, ham_id)
 
+    def observables(self, operators: Sequence) -> ObservablesHandle:
+        """Device form of several observables of one width, evaluated together by ``expectation_many``: the union of their
+        distinct Pauli strings, grouped by x mask (``qb_observables_create``)."""
+        width, x, z, c, offs = observable_terms(operators)
+        x = np.ascontiguousarray(x, dtype=np.uint64)
+        z = np.ascontiguousarray(z, dtype=np.uint64)
+        cre = np.ascontiguousarray(c.real, dtype=np.float64)
+        cim = np.ascontiguousarray(c.imag, dtype=np.float64)
+        pad = lambda a: a if a.size else np.zeros(1, dtype=a.dtype)  # (valid pointers for a set of empty operators)
+        obs_id = c_int64()
+        _native.check(
+            self._lib.qb_observables_create(self._ctx, width, len(offs) - 1, _native.ptr(offs), _native.ptr(pad(x)), _native.ptr(pad(z)),
+                                            _native.ptr(pad(cre)), _native.ptr(pad(cim)), byref(obs_id))
+        )
+        n_terms = len(observable_union(x, z, c, offs)[0])
+        handle = ObservablesHandle(obs_id.value, width, len(offs) - 1, not bool(np.any(x)), n_terms)
+        weakref.finalize(handle, self._release_observables, self._lib, self._ctx, obs_id.value, self._finalizer)
+        return handle
+
+    @staticmethod
+    def _release_observables(lib, ctx, obs_id, engine_finalizer):
+        if engine_finalizer.alive:
+            lib.qb_observables_destroy(ctx, obs_id)
+
     # ------------------------------------------------------------------ batched evaluation
     @staticmethod
     def _pack(plans: Sequence[PlanHandle], params: Sequence[Sequence[float]]):
@@ -447,6 +516,16 @@ class Engine:
         ids, flat, offsets = self._pack(plans, params)  # (raises ValueError for a length mismatch, as in expectation / sample)
         out = np.empty(len(plans), dtype=np.float64)
         _native.check(self._lib.qb_evaluate_cvar(self._ctx, len(plans), _native.ptr(ids), _native.ptr(flat), _native.ptr(offsets), ham.ham_id, float(alpha), _native.ptr(out)))
+        return out
+
+    def expectation_many(self, plans: Sequence[PlanHandle], params: Sequence[Sequence[float]], handle: ObservablesHandle) -> np.ndarray:
+        """Re <psi_i|H_j|psi_i> of every circuit and every observable of ``handle``: float64 array [len(plans), n_obs], each
+        distinct Pauli string reduced once per state (``qb_evaluate_observables``)."""
+        if not plans:
+            return np.zeros((0, handle.n_obs))
+        ids, flat, offsets = self._pack(plans, params)
+        out = np.empty((len(plans), handle.n_obs), dtype=np.float64)
+        _native.check(self._lib.qb_evaluate_observables(self._ctx, len(plans), _native.ptr(ids), _native.ptr(flat), _native.ptr(offsets), handle.obs_id, _native.ptr(out)))
         return out
 
     def statevector(self, plan: PlanHandle, params: Sequence[float]) -> np.ndarray:

@@ -12,8 +12,14 @@ Semantics follow [upstream] ``StatevectorEstimator`` / ``StatevectorSampler`` (q
     ``default_rng(seed).normal(evs, precision)`` from a fresh generator per pub, ``stds = precision``
   * sampler: ``Generator.choice`` = ``cumsum(|psi|^2)`` CDF + ``searchsorted(uniforms, side='right')`` with
     ``uniforms = default_rng(seed).random(shots)``, a fresh generator per pub when ``seed`` is an int.
-Only zero-dimensional pubs (one parameter vector per pub) are used by QUEASARS; 2-D ``parameter_values`` are
-accepted and produce array-shaped ``evs`` / one register per row.
+QUEASARS itself only sends zero-dimensional pubs (one parameter vector, one observable).  Arrays are accepted too:
+  * estimator: an observables array of several elements (``ObservablesArray``, nested lists of ``SparsePauliOp``s,
+    ``{label: coeff}`` dicts or labels) is broadcast against the parameter shape, ``evs.shape ==
+    np.broadcast_shapes(obs_shape, param_shape)``; every distinct parameter row is simulated once and all distinct
+    observables are reduced from that one state (``expectation_values_many``).  A pub with exactly one observable keeps
+    the single-observable route, and ``[H]`` gives the parameter shape (upstream: ``(1,)``).
+  * sampler: ``parameter_values`` of shape S give one submission over all rows and ``data.meas`` of shape S
+    (``get_counts(loc=None)`` pools every position, as upstream's ``BitArray``).
 """
 from __future__ import annotations
 
@@ -28,7 +34,7 @@ from . import _native
 from . import containers as ct
 from . import expectation as ex
 from .batching import CoalescingQueue
-from .engine import Engine, HamiltonianHandle, PlanHandle
+from .engine import Engine, HamiltonianHandle, ObservablesHandle, PlanHandle
 from .gate_list import from_circuit_or_none, from_circuit
 
 _engines: dict = {}
@@ -255,6 +261,24 @@ class _B200Primitive:
             self._ham_cache[key] = (operator, handle, fp)
         return handle
 
+    def observables_for(self, operators: Sequence, slot: int = 0, fingerprints=None) -> ObservablesHandle:
+        """Device form of a set of observables on device ``slot``, cached like ``hamiltonian_for``: by the operators' identities,
+        guarded by their fingerprints against in-place edits."""
+        operators = tuple(operators)
+        key = ("obs", tuple(id(op) for op in operators), slot)
+        fps = tuple(_operator_fingerprint(op) for op in operators) if fingerprints is None else tuple(fingerprints)
+        with self._lock:
+            hit = self._ham_cache.get(key)
+            if hit is not None and len(hit[0]) == len(operators) and all(a is b for a, b in zip(hit[0], operators)) and hit[2] == fps:
+                return hit[1]
+        engines = self.engines
+        handle = engines[slot].observables(operators)
+        with self._lock:
+            if len(self._ham_cache) > 64 * len(engines):
+                self._ham_cache.clear()
+            self._ham_cache[key] = (operators, handle, fps)
+        return handle
+
     # ------------------------------------------------------------------ splitting a submission over the devices
     def _assign(self, entries: Sequence, costs: Sequence[float]) -> list:
         """entries[i] = cache entry of circuit i (or None) -> device slot per entry.  Greedy longest-processing-time over
@@ -454,7 +478,63 @@ class B200EstimatorV2(_B200Primitive):
                 return np.asarray(engines[0].expectation([r[1] for r in resolved], [r[2] for r in resolved], ham), dtype=np.float64)
         return np.asarray(self._submit(("exp", id(operator), fp), (operator, circuits, parameter_values)))
 
+    def expectation_values_many(self, circuits, parameter_values, observables) -> np.ndarray:
+        """Exact <H_j> of every (circuit_i, params_i) and every observable H_j: float64 array [len(circuits), len(observables)].
+        Each circuit is simulated once and every distinct Pauli string of the set is reduced once per state."""
+        circuits, parameter_values, observables = list(circuits), list(parameter_values), list(observables)
+        if len(circuits) != len(parameter_values):
+            raise ValueError(f"{len(circuits)} circuits but {len(parameter_values)} parameter vectors")
+        if not observables:
+            raise ValueError("at least one observable is needed")
+        widths = {int(op.num_qubits) for op in observables}
+        if len(widths) != 1:
+            raise ValueError("all observables of one set must act on the same number of qubits")
+        width = widths.pop()
+        for c in circuits:
+            if _width(c) != width:
+                raise ValueError(f"a circuit acts on {_width(c)} qubits, the observables on {width}")
+        if not circuits:
+            return np.zeros((0, len(observables)))
+        fps = tuple(_operator_fingerprint(op) for op in observables)
+        if not self._needs_sharding(width):
+            self.observables_for(observables, fingerprints=fps)  # validates the set (and builds its device form) before anything is queued
+        key = ("many", tuple(id(op) for op in observables), fps)
+        return np.asarray(self._submit(key, (observables, circuits, parameter_values)), dtype=np.float64).reshape(len(circuits), len(observables))
+
+    def _execute_many(self, key, payloads):
+        observables = payloads[0][0]
+        fps = key[2]
+        circuits, values, sizes = [], [], []
+        for _, circs, vals in payloads:
+            sizes.append(len(circs))
+            circuits.extend(circs)
+            values.extend(vals)
+        width = int(observables[0].num_qubits)
+        if self._needs_sharding(width):
+            # one statevector over the whole device set per row, every observable evaluated on it (sharded.py)
+            flat = []
+            with self._shard_lock:
+                sv = self._sharded_state(width)
+                for circuit, vals in zip(circuits, values):
+                    gates, bound = self._bound_gates(circuit, vals)
+                    sv.reset()
+                    sv.run(gates, bound)
+                    flat.append(np.asarray([sv.expectation(op) for op in observables], dtype=np.float64))
+        else:
+            diagonal = self.observables_for(observables, fingerprints=fps).diagonal
+            resolved = self._resolve_all(circuits, values, probabilities_only=diagonal)
+            flat = self._run_per_device(
+                resolved, lambda slot, plans, params: list(self.engines[slot].expectation_many(plans, params, self.observables_for(observables, slot, fps)))
+            )
+        out, pos = [], 0
+        for n in sizes:
+            out.append(np.asarray(flat[pos : pos + n], dtype=np.float64).reshape(n, len(observables)))
+            pos += n
+        return out
+
     def _execute(self, key, payloads):
+        if key[0] == "many":
+            return self._execute_many(key, payloads)
         operator = payloads[0][0]
         circuits, values, sizes = [], [], []
         for _, circs, vals in payloads:
@@ -544,6 +624,19 @@ class B200EstimatorV2(_B200Primitive):
             for pub in coerced:
                 prec = pub.precision if pub.precision is not None else self.default_precision
                 rows, shape = _param_rows(pub.parameter_values)
+                try:
+                    ops, obs_shape = _observables_array(pub.observables)
+                except TypeError:  # not an observables array this module reads: the single-observable route decides
+                    ops, obs_shape = [None], ()
+                if len(ops) != 1:
+                    evs = self._many_evs(pub.circuit, rows, shape, ops, obs_shape)
+                    evs = self._noisy(evs, float(prec or 0.0))
+                    shape = evs.shape
+                    results.append(
+                        ct.PubResult(ct.DataBin(evs=evs, stds=np.full(shape, float(prec or 0.0)), shape=shape),
+                                     metadata={"target_precision": prec, "circuit_metadata": {}})
+                    )
+                    continue
                 evs = self.expectation_values([pub.circuit] * len(rows), list(rows), _single_observable(pub.observables))
                 evs = self._noisy(np.asarray(evs, dtype=np.float64), float(prec or 0.0)).reshape(shape)
                 stds = np.full(shape, float(prec or 0.0))
@@ -553,6 +646,68 @@ class B200EstimatorV2(_B200Primitive):
             return ct.FinishedJob(ct.PrimitiveResult(results, metadata={"version": 2, "backend": "queasars_b200"}))
         except Exception as exc:  # surfaced by job.result(), like a PrimitiveJob would
             return ct.FinishedJob(error=exc)
+
+    def _many_evs(self, circuit, rows: np.ndarray, param_shape: tuple, ops: list, obs_shape: tuple) -> np.ndarray:
+        """evs of a pub with several observables: V2 broadcasting of the observable shape against the parameter shape; every
+        distinct parameter row is simulated once and evaluated with all distinct observables in one call."""
+        shape = np.broadcast_shapes(obs_shape, param_shape)  # (ValueError for shapes that do not broadcast)
+        width = _width(circuit)
+        for op in ops:
+            if int(op.num_qubits) != width:
+                raise ValueError(f"an observable acts on {int(op.num_qubits)} qubits, the circuit on {width}")
+        uniq_rows, row_of = np.unique(rows, axis=0, return_inverse=True) if len(rows) > 1 else (rows, np.zeros(len(rows), dtype=np.int64))
+        row_of = np.asarray(row_of).reshape(-1)
+        keys, distinct, op_of = {}, [], []
+        for op in ops:
+            x, z, c = _op_masks(op)
+            k = (x.tobytes(), z.tobytes(), c.tobytes())
+            if k not in keys:
+                keys[k] = len(distinct)
+                distinct.append(op)
+            op_of.append(keys[k])
+        vals = self.expectation_values_many([circuit] * len(uniq_rows), list(uniq_rows), distinct)
+        p_idx = np.broadcast_to(row_of.reshape(param_shape), shape)
+        o_idx = np.broadcast_to(np.asarray(op_of, dtype=np.int64).reshape(obs_shape), shape)
+        return np.asarray(vals[p_idx, o_idx], dtype=np.float64)
+
+
+def _op_masks(op):
+    from .engine import operator_terms
+
+    _, x, z, c = operator_terms(op)
+    return np.asarray(x, dtype=np.uint64), np.asarray(z, dtype=np.uint64), np.asarray(c, dtype=complex)
+
+
+def _as_operator(obs):
+    """One element of an observables array: a ``SparsePauliOp``(-like), a ``{label: coeff}`` dict or a Pauli label."""
+    from .operators import SparsePauliOp
+
+    if isinstance(obs, dict):
+        if not obs:
+            raise ValueError("an observable given as a dict needs at least one term")
+        return SparsePauliOp.from_list(list(obs.items()))
+    if isinstance(obs, str):
+        return SparsePauliOp(obs)
+    if hasattr(obs, "num_qubits") and (hasattr(obs, "to_list") or hasattr(obs, "masks")):
+        return obs
+    raise TypeError(f"cannot interpret {type(obs).__name__} as an observable")
+
+
+def _observables_array(observables) -> tuple[list, tuple]:
+    """A pub's observables -> (operators in row-major order, shape).  Accepts qiskit's ``ObservablesArray`` (``tolist()`` gives
+    ``{label: coeff}`` dicts), nested lists / tuples, dicts, ``SparsePauliOp``s and Pauli labels."""
+    obs = observables
+    if hasattr(obs, "tolist") and not hasattr(obs, "to_list"):  # ObservablesArray / object ndarray
+        obs = obs.tolist()
+    if not isinstance(obs, (list, tuple)):
+        return [_as_operator(obs)], ()
+    if not obs:
+        raise ValueError("an observables array needs at least one observable")
+    parts = [_observables_array(o) for o in obs]
+    inner = parts[0][1]
+    if any(p[1] != inner for p in parts):
+        raise ValueError("observables array is ragged: its nested lists differ in shape")
+    return [op for p in parts for op in p[0]], (len(obs),) + inner
 
 
 def _single_observable(observables):
@@ -710,12 +865,13 @@ class B200SamplerV2(_B200Primitive):
             for pub in coerced:
                 n_shots = int(pub.shots if pub.shots is not None else self.default_shots)
                 rows, shape = _param_rows(pub.parameter_values)
-                if shape != ():
-                    raise NotImplementedError("B200SamplerV2 supports one parameter vector per pub")
                 _check_measure_all(pub.circuit)
-                idx = self.sample_indices([pub.circuit], [rows[0]], n_shots)[0]
-                reg = ct.ShotRegister(idx, int(pub.circuit.num_qubits))
-                results.append(ct.SamplerPubResult(ct.DataBin(meas=reg, shape=()), metadata={"shots": n_shots, "circuit_metadata": {}}))
+                if shape == ():
+                    idx = self.sample_indices([pub.circuit], [rows[0]], n_shots)[0]
+                else:  # a parameter array: one submission over all rows, one register position per row
+                    idx = self.sample_indices([pub.circuit] * len(rows), list(rows), n_shots).reshape(shape + (n_shots,))
+                reg = ct.ShotRegister(idx, int(pub.circuit.num_qubits), shape)
+                results.append(ct.SamplerPubResult(ct.DataBin(meas=reg, shape=shape), metadata={"shots": n_shots, "circuit_metadata": {}}))
             return ct.FinishedJob(ct.PrimitiveResult(results, metadata={"version": 2, "backend": "queasars_b200"}))
         except Exception as exc:
             return ct.FinishedJob(error=exc)
