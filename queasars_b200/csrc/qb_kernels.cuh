@@ -1284,6 +1284,10 @@ scan_chunks_kernel(double* __restrict__ chunk_sums, uint64_t n_chunks) {
 }
 
 // one warp per shot: index = first k with cdf(k) / total > u   (searchsorted(cdf / cdf[-1], u, side='right'))
+// searchsorted never returns an index of probability zero for u < 1 (such an entry repeats its predecessor's cdf).  The warp
+// scan below sums in tree order, so at a cdf boundary a zero-probability lane can see a larger running sum than the non-zero
+// lane before it: only lanes with pr > 0 may be hits, and the fallback for a chunk whose running sum misses u by rounding is
+// its last entry with pr > 0.
 template <typename T>
 __global__ void __launch_bounds__(256)
 sample_kernel(const typename Cx<T>::type* __restrict__ states, uint64_t state_stride, const double* __restrict__ chunk_cdf,
@@ -1303,7 +1307,7 @@ sample_kernel(const typename Cx<T>::type* __restrict__ states, uint64_t state_st
         else lo = mid + 1;
     }
     double run = lo ? cdf[lo - 1] : 0.0;
-    int64_t found = -1;
+    int64_t found = -1, last_nz = -1;
     for (int i = 0; i < kChunk / 32 && found < 0; ++i) {
         const uint64_t k = lo * kChunk + i * 32 + lane;
         const auto a = st[k];
@@ -1314,12 +1318,15 @@ sample_kernel(const typename Cx<T>::type* __restrict__ states, uint64_t state_st
             const double nb = __shfl_up_sync(0xffffffffu, inc, o);
             if (lane >= o) inc += nb;
         }
-        const bool hit = ((run + inc) / total > u);
+        const bool hit = pr > 0.0 && ((run + inc) / total > u);
         const unsigned ballot = __ballot_sync(0xffffffffu, hit);
+        const unsigned nonzero = __ballot_sync(0xffffffffu, pr > 0.0);
         if (ballot) found = int64_t(lo * kChunk + i * 32 + (__ffs(ballot) - 1));
+        else if (nonzero) last_nz = int64_t(lo * kChunk + i * 32 + (31 - __clz(nonzero)));
         run += __shfl_sync(0xffffffffu, inc, 31);
     }
-    if (found < 0) found = int64_t(lo * kChunk + kChunk - 1);  // rounding at the very top of a chunk
+    if (found < 0) found = last_nz;  // rounding at the very top of a chunk
+    if (found < 0) found = int64_t(lo * kChunk + kChunk - 1);  // (no mass in the chunk: only for u outside [0, 1))
     if (uint64_t(found) >= valid_size) found = int64_t(valid_size - 1);
     if (lane == 0) out[blockIdx.y * uint64_t(shots) + shot] = found;
 }
