@@ -246,7 +246,9 @@ int qb_batch_run_timed(qb_context* ctx, int64_t batch_id, int max_launches, floa
 /* --- device-pointer entry points (parity tests, sharded multi-GPU path) -------------------------------
  * Operate on a caller-owned device statevector of 2^n_local amplitudes.  `index_offset` is OR-ed into the
  * amplitude index seen by QB_K_EXT operands and by the diagonal table lookup, so a rank holding the shard
- * with global-qubit bits `rank << n_local` evaluates controls on global qubits correctly. */
+ * with global-qubit bits `rank << n_local` evaluates controls on global qubits correctly.  A plan whose width is below
+ * its sweep tile (2^tile_bits amplitudes) is refused by qb_apply_plan_device with QB_ERR_INVALID: its sweeps would cover
+ * more than the caller's buffer. */
 int qb_apply_plan_device(qb_context* ctx, int64_t plan_id, const double* params_host, int n_params,
                          void* d_state, int init_zero_state, uint64_t index_offset);
 int qb_expectation_device(qb_context* ctx, int64_t ham_id, int dtype, int n_local, const void* d_state,
@@ -257,6 +259,22 @@ int qb_expectation_device(qb_context* ctx, int64_t ham_id, int dtype, int n_loca
  * rank its shots with re-scaled uniforms ([upstream] StatevectorSampler / Generator.choice semantics per shard). */
 int qb_sample_device(qb_context* ctx, int dtype, int n_local, const void* d_state, int shots,
                      const double* uniforms, int64_t* out_indices);
+/* One radix-digit pass of the exact CVaR of a sharded state (sort-free weighted selection, queasars_b200/sharded.py) on a
+ * caller-owned shard of 2^n_local amplitudes whose physical indices are `index_offset | k`.  Entries are keyed by
+ * (energy_key(E(k)), logical k) with E(k) of the diagonal Hamiltonian `ham_id` (built with physical z masks), summed like
+ * qb_hamiltonian_diag_energies, and energy_key the order-preserving 64-bit image of the double (-0.0 keyed as +0.0).  Only
+ * entries matching the prefix are counted: energy key >> e_free == e_prefix (e_free = 64: no energy constraint) and
+ * (physical index & idx_mask) == idx_value.  The digit is bits [e_free - digit_bits, e_free) of the energy key (digit_kind 0) or
+ * the physical index bits digit_positions[0..digit_bits) (digit_kind 1; the logical index bits of the digit, lowest first),
+ * digit_bits <= 8.  Per bucket b of the digit: out_sums[b] = mass, out_sums[256 + b] = sum p * E (fixed summation order: the
+ * same on every call), out_ints[b] = count, [256 + b] / [512 + b] = min / max energy key, [768 + b] = least physical index.
+ * cache_mode 1 also writes (p, E) of every entry as two doubles into d_cache (2^n_local * 16 B, e.g. the idle spare shard
+ * buffer); cache_mode 2 reads them from there and does not touch d_state.  QB_ERR_INVALID for a non-diagonal Hamiltonian, a
+ * bad bit map or a bad digit.  Synchronous. */
+int qb_cvar_select_device(qb_context* ctx, int64_t ham_id, int dtype, int n_local, const void* d_state, uint64_t index_offset,
+                          void* d_cache, int cache_mode, uint64_t e_prefix, int e_free, int digit_kind, int digit_bits,
+                          const int32_t* digit_positions, uint64_t idx_mask, uint64_t idx_value, double* out_sums,
+                          uint64_t* out_ints);
 
 /* Global <-> local qubit swap of a state sharded over `world` = 2^n_global GPUs of one node (BASELINE config C5), fused with its
  * all-to-all: the calling rank streams its shard `d_state` once and stores every amplitude directly into the rank that owns it

@@ -67,6 +67,8 @@ def _declare(lib):
         "qb_apply_plan_device": [c_void_p, c_int64, c_void_p, c_int, c_void_p, c_int, c_uint64],
         "qb_expectation_device": [c_void_p, c_int64, c_int, c_int, c_void_p, c_uint64, P(c_double)],
         "qb_sample_device": [c_void_p, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p],
+        "qb_cvar_select_device": [c_void_p, c_int64, c_int, c_int, c_void_p, c_uint64, c_void_p, c_int, c_uint64, c_int, c_int, c_int, c_void_p,
+                                  c_uint64, c_uint64, c_void_p, c_void_p],
         "qb_swap_global_p2p": [c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p],
         "qb_device_alloc": [c_void_p, c_uint64, P(c_void_p)],
         "qb_device_free": [c_void_p, c_void_p],
@@ -98,7 +100,7 @@ EXPORTED_SYMBOLS = (
     "qb_observables_create qb_observables_destroy qb_evaluate_observables "
     "qb_evaluate_expectation_multi qb_evaluate_expectation_submit qb_evaluate_expectation_collect qb_context_sm_count "
     "qb_batch_create qb_batch_set_params qb_batch_run qb_batch_run_timed qb_batch_read qb_batch_destroy qb_batch_stats "
-    "qb_apply_plan_device qb_expectation_device qb_sample_device qb_swap_global_p2p qb_record_sizes "
+    "qb_apply_plan_device qb_expectation_device qb_sample_device qb_cvar_select_device qb_swap_global_p2p qb_record_sizes "
     "qb_device_alloc qb_device_free qb_device_read qb_enable_peer_access qb_ipc_export qb_ipc_open qb_ipc_close"
 ).split()
 

@@ -1848,6 +1848,12 @@ int qb_apply_plan_device(qb_context* ctx, int64_t plan_id, const double* params_
     if (!ctx || !d_state) return fail(QB_ERR_INVALID, "null argument");
     std::lock_guard<std::mutex> lock(ctx->mu);
     QB_ON_DEVICE(ctx);
+    const Plan* pl = find_plan(ctx, plan_id);
+    if (!pl) return fail(QB_ERR_NOT_FOUND, "unknown plan id");
+    // the sweeps cover 2^n_eff amplitudes; a caller-owned state holds exactly 2^n_qubits
+    if (pl->n_eff != pl->n_qubits)
+        return fail(QB_ERR_INVALID, "a caller-owned state of " + std::to_string(pl->n_qubits) + " qubits is smaller than one " +
+                                        std::to_string(pl->n_eff) + "-qubit sweep tile");
     DeviceBatch b;
     QB_TRY(build_batch(ctx, b, 1, &plan_id, nullptr, d_state, init_zero_state, index_offset));
     const int64_t offs[2] = {0, n_params};
@@ -1909,6 +1915,71 @@ int qb_sample_device(qb_context* ctx, int dtype, int n_local, const void* d_stat
     QB_TRY(check_launch(ctx, "sample_kernel"));
     QB_CUDA(cudaMemcpyAsync(out_indices, d_indices, u_bytes, cudaMemcpyDeviceToHost, ctx->stream));
     QB_CUDA(cudaStreamSynchronize(ctx->stream));
+    return QB_OK;
+}
+
+int qb_cvar_select_device(qb_context* ctx, int64_t ham_id, int dtype, int n_local, const void* d_state, uint64_t index_offset, void* d_cache,
+                          int cache_mode, uint64_t e_prefix, int e_free, int digit_kind, int digit_bits, const int32_t* digit_positions,
+                          uint64_t idx_mask, uint64_t idx_value, double* out_sums, uint64_t* out_ints) {
+    if (!ctx || !out_sums || !out_ints || (cache_mode != 2 && !d_state)) return fail(QB_ERR_INVALID, "null argument");
+    if (n_local < 8 || n_local > 36) return fail(QB_ERR_INVALID, "n_local out of range");
+    if (dtype != QB_C128 && dtype != QB_C64) return fail(QB_ERR_INVALID, "dtype must be QB_C128 or QB_C64");
+    if (cache_mode < 0 || cache_mode > 2 || (cache_mode && !d_cache)) return fail(QB_ERR_INVALID, "cache_mode must be 0, or 1 / 2 with a cache buffer");
+    if (digit_bits < 1 || digit_bits > qb::kSelBits) return fail(QB_ERR_INVALID, "digit_bits must be in 1.." + std::to_string(qb::kSelBits));
+    if (e_free < 0 || e_free > 64) return fail(QB_ERR_INVALID, "e_free must be in 0..64");
+    if (e_free > 0 && e_free < 64 && (e_prefix >> (64 - e_free)) != 0) return fail(QB_ERR_INVALID, "e_prefix has bits beyond 64 - e_free");
+    if ((idx_value & ~idx_mask) != 0) return fail(QB_ERR_INVALID, "idx_value has bits outside idx_mask");
+    qb::SelectArgs a{};
+    a.e_prefix = e_prefix, a.idx_mask = idx_mask, a.idx_value = idx_value, a.e_free = e_free, a.digit_kind = digit_kind, a.bits = digit_bits;
+    if (digit_kind == 0) {
+        if (e_free < digit_bits) return fail(QB_ERR_INVALID, "energy digit below the energy key's open bits");
+    } else if (digit_kind == 1) {
+        if (!digit_positions) return fail(QB_ERR_INVALID, "null digit_positions");
+        uint64_t seen = idx_mask;
+        for (int j = 0; j < digit_bits; ++j) {
+            const int p = digit_positions[j];
+            if (p < 0 || p > 63 || ((seen >> p) & 1)) return fail(QB_ERR_INVALID, "bad bit map: digit positions must be distinct, unfixed bit positions");
+            seen |= uint64_t(1) << p;
+            a.pos[j] = p;
+        }
+    } else {
+        return fail(QB_ERR_INVALID, "digit_kind must be 0 (energy) or 1 (logical index)");
+    }
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    QB_ON_DEVICE(ctx);
+    Ham* ham = find_ham(ctx, ham_id);
+    if (!ham) return fail(QB_ERR_NOT_FOUND, "unknown Hamiltonian id");
+    if (!ham->diagonal) return fail(QB_ERR_INVALID, "CVaR needs a diagonal Hamiltonian; this one has non-diagonal terms");
+    const uint64_t size = uint64_t(1) << n_local;
+    // the grid depends on the device and the shard size only: the CTA-order reduction is the same on every call
+    const int n_cta = int(std::min<uint64_t>(uint64_t(ctx->sm_count) * 4, std::max<uint64_t>(1, size / (32 * qb::kSelWarps * 16))));
+    constexpr int B = qb::kSelBuckets;
+    const size_t part_bytes = sizeof(double) * 2 * B * size_t(n_cta), sums_bytes = sizeof(double) * 2 * B, ints_bytes = sizeof(uint64_t) * 4 * B;
+    QB_TRY(ctx->scratch.reserve(part_bytes + sums_bytes + ints_bytes));
+    double* d_part = ctx->scratch.as<double>();
+    double* d_sums = d_part + 2 * B * size_t(n_cta);
+    unsigned long long* d_ints = reinterpret_cast<unsigned long long*>(d_sums + 2 * B);
+    QB_CUDA(cudaMemsetAsync(d_ints, 0, sizeof(uint64_t) * B, ctx->stream));                  // count
+    QB_CUDA(cudaMemsetAsync(d_ints + B, 0xff, sizeof(uint64_t) * B, ctx->stream));           // emin
+    QB_CUDA(cudaMemsetAsync(d_ints + 2 * B, 0, sizeof(uint64_t) * B, ctx->stream));          // emax
+    QB_CUDA(cudaMemsetAsync(d_ints + 3 * B, 0xff, sizeof(uint64_t) * B, ctx->stream));       // kmin
+    const uint64_t* z = ham->diag_z.as<uint64_t>();
+    const double* c = ham->diag_c.as<double>();
+    double2* cache = static_cast<double2*>(d_cache);
+    if (dtype == QB_C128)
+        qb::cvar_select_kernel<double><<<n_cta, 32 * qb::kSelWarps, 0, ctx->stream>>>(static_cast<const double2*>(d_state), cache, cache_mode, size,
+                                                                                       index_offset, z, c, ham->n_diag, a, d_part, d_part + B * size_t(n_cta), d_ints);
+    else
+        qb::cvar_select_kernel<float><<<n_cta, 32 * qb::kSelWarps, 0, ctx->stream>>>(static_cast<const float2*>(d_state), cache, cache_mode, size,
+                                                                                      index_offset, z, c, ham->n_diag, a, d_part, d_part + B * size_t(n_cta), d_ints);
+    QB_TRY(check_launch(ctx, "cvar_select_kernel"));
+    qb::cvar_select_reduce_kernel<<<2 * B, 256, 0, ctx->stream>>>(d_part, n_cta, d_sums);
+    QB_TRY(check_launch(ctx, "cvar_select_reduce_kernel"));
+    QB_TRY(ctx->pin_out.reserve(sums_bytes + ints_bytes));
+    QB_CUDA(cudaMemcpyAsync(ctx->pin_out.p, d_sums, sums_bytes + ints_bytes, cudaMemcpyDeviceToHost, ctx->stream));  // d_ints follows d_sums
+    QB_CUDA(cudaStreamSynchronize(ctx->stream));
+    std::memcpy(out_sums, ctx->pin_out.p, sums_bytes);
+    std::memcpy(out_ints, static_cast<const unsigned char*>(ctx->pin_out.p) + sums_bytes, ints_bytes);
     return QB_OK;
 }
 

@@ -10,6 +10,7 @@
 //   expect_tile_kernel  K4     the same for all groups that fit one 2^11 tile: one read of the state per tile sweep
 //   chunk_prob_kernel / scan_chunks_kernel / sample_kernel   K5  prefix-sum CDF sampling
 //   cvar_chunk_kernel / scan_chunks_kernel / cvar_finish_kernel  K6  exact CVaR(alpha) of a diagonal Hamiltonian (sorted lower tail)
+//   cvar_select_kernel / cvar_select_reduce_kernel  K8  one radix-digit pass of the exact CVaR of a sharded state (weighted select)
 //   swap_p2p_kernel            global <-> local qubit swap of a sharded state fused with its all-to-all (peer-memory stores)
 //
 // What the arithmetic follows ([upstream] = un-vendored qiskit 2.4.2, see oracle/qiskit_semantics.py):
@@ -1421,6 +1422,129 @@ cvar_finish_kernel(const typename Cx<T>::type* __restrict__ states, uint64_t sta
         run += __shfl_sync(0xffffffffu, inc, 31);
         acc += __shfl_sync(0xffffffffu, pe, 31);
     }
+}
+
+// ---------------------------------------------------------------------------------------------------
+// exact CVaR(alpha) of a SHARDED state (K8): one radix-digit pass of a sort-free weighted selection over one shard.
+// The stable ascending (E(k), logical k) order is the order of the composite key (energy_key(E(k)), logical k); the stop entry
+// of the greedy fill is the smallest key whose inclusive mass reaches the bound.  The host fixes the key digit by digit: every
+// pass histograms, over the entries that match the prefix fixed so far, the next digit -- per bucket the mass, sum p * E, the
+// count, min / max of the energy key and the least physical index -- and the host keeps the bucket in which the bound falls.
+//   digit_kind 0: bits [e_free - bits, e_free) of the energy key;  1: logical index bits, read from physical positions pos[]
+// Determinism: per warp and iteration the entries of one digit are summed by their lowest lane in lane order, the per-warp
+// histograms are added in warp order, and per-CTA partials are reduced in CTA order (cvar_select_reduce_kernel).  Count, min
+// and max are integers (atomics are order-free).  cache_mode 1 writes (p, E) of every entry into `cache` (the spare shard
+// buffer, 16 B per amplitude), mode 2 reads them from there instead of the state and the Hamiltonian.
+// ---------------------------------------------------------------------------------------------------
+constexpr int kSelBits = 8;
+constexpr int kSelBuckets = 1 << kSelBits;
+constexpr int kSelWarps = 8;
+
+struct SelectArgs {
+    uint64_t e_prefix;             // fixed high bits of the energy key (its low e_free bits are open)
+    uint64_t idx_mask, idx_value;  // physical index bits fixed by the logical-index prefix
+    int32_t e_free;                // 64: no energy constraint (alpha ~ 1 orders by the logical index alone)
+    int32_t digit_kind, bits;
+    int32_t pos[kSelBits];         // index digit: physical positions of its logical bits, lowest first
+};
+
+// order-preserving 64-bit key of a double; -0.0 gets the key of +0.0 (radix sort / numpy stable argsort treat them as tied)
+__device__ __forceinline__ uint64_t energy_key(double e) {
+    uint64_t u = uint64_t(__double_as_longlong(e));
+    if (u == 0x8000000000000000ull) u = 0;
+    return (u >> 63) ? ~u : (u | 0x8000000000000000ull);
+}
+
+// grid = n_cta (fixed by the device and the shard size), block = 32 * kSelWarps.  part_* = [bucket][cta];
+// ints = [count | emin | emax | kmin][bucket], initialised by the caller (0, ~0, 0, ~0)
+template <typename T>
+__global__ void __launch_bounds__(32 * kSelWarps)
+cvar_select_kernel(const typename Cx<T>::type* __restrict__ state, double2* __restrict__ cache, int cache_mode, uint64_t size,
+                   uint64_t index_offset, const uint64_t* __restrict__ z, const double* __restrict__ c, int n_terms, SelectArgs a,
+                   double* __restrict__ part_mass, double* __restrict__ part_pe, unsigned long long* __restrict__ ints) {
+    __shared__ double h_m[kSelWarps][kSelBuckets], h_s[kSelWarps][kSelBuckets];
+    __shared__ double st_p[kSelWarps][32], st_e[kSelWarps][32];
+    __shared__ unsigned long long st_k[kSelWarps][32];
+    __shared__ unsigned long long s_cnt[kSelBuckets], s_min[kSelBuckets], s_max[kSelBuckets], s_kmin[kSelBuckets];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    for (int b = threadIdx.x; b < kSelBuckets; b += blockDim.x) {
+        for (int w = 0; w < kSelWarps; ++w) h_m[w][b] = 0.0, h_s[w][b] = 0.0;
+        s_cnt[b] = 0, s_min[b] = ~0ull, s_max[b] = 0, s_kmin[b] = ~0ull;
+    }
+    __syncthreads();
+    const unsigned dmask = (1u << a.bits) - 1u;
+    const uint64_t stride = uint64_t(gridDim.x) * kSelWarps * 32;
+    // size is a multiple of 32: every lane of a warp runs the same iterations (the warp-synchronous steps below need it)
+    for (uint64_t k = (uint64_t(blockIdx.x) * kSelWarps + warp) * 32 + lane; k < size; k += stride) {
+        double p, e;
+        if (cache_mode == 2) {
+            const double2 v = cache[k];
+            p = v.x, e = v.y;
+        } else {
+            const auto amp = state[k];
+            p = double(amp.x) * double(amp.x) + double(amp.y) * double(amp.y);
+            e = 0.0;  // diag_table_kernel's loop: the same double, so ties are the ones the single-GPU route sees
+            const uint64_t kk = k | index_offset;
+            for (int t = 0; t < n_terms; ++t) e += (__popcll(kk & z[t]) & 1) ? -c[t] : c[t];
+            if (cache_mode == 1) cache[k] = make_double2(p, e);
+        }
+        const uint64_t kk = k | index_offset;
+        const uint64_t key = energy_key(e);
+        const bool ok = (kk & a.idx_mask) == a.idx_value && (a.e_free >= 64 || (key >> a.e_free) == a.e_prefix);
+        unsigned d = 0;
+        if (a.digit_kind == 0) {
+            d = unsigned(key >> (a.e_free - a.bits)) & dmask;
+        } else {
+#pragma unroll
+            for (int j = 0; j < kSelBits; ++j)  // (unrolled: constant indices keep a.pos in registers, off the stack)
+                if (j < a.bits) d |= unsigned((kk >> a.pos[j]) & 1) << j;
+        }
+        const unsigned peers = __match_any_sync(0xffffffffu, ok ? d : 0xffffffffu);
+        st_p[warp][lane] = p, st_e[warp][lane] = e, st_k[warp][lane] = kk;
+        __syncwarp();
+        if (ok && lane == __ffs(peers) - 1) {  // the lowest lane of every digit sums its peers in lane order
+            double m = 0.0, s = 0.0;
+            uint64_t lo = ~0ull, hi = 0, kmin = ~0ull;
+            for (unsigned rest = peers; rest; rest &= rest - 1) {
+                const int l = __ffs(rest) - 1;
+                const double pl = st_p[warp][l], el = st_e[warp][l];
+                const uint64_t kl = energy_key(el);
+                m += pl, s += pl * el;
+                lo = kl < lo ? kl : lo, hi = kl > hi ? kl : hi;
+                kmin = st_k[warp][l] < kmin ? st_k[warp][l] : kmin;
+            }
+            h_m[warp][d] += m, h_s[warp][d] += s;
+            atomicAdd(&s_cnt[d], (unsigned long long)__popc(peers));
+            atomicMin(&s_min[d], (unsigned long long)lo);
+            atomicMax(&s_max[d], (unsigned long long)hi);
+            atomicMin(&s_kmin[d], (unsigned long long)kmin);
+        }
+        __syncwarp();
+    }
+    __syncthreads();
+    for (int b = threadIdx.x; b < kSelBuckets; b += blockDim.x) {
+        double m = 0.0, s = 0.0;
+        for (int w = 0; w < kSelWarps; ++w) m += h_m[w][b], s += h_s[w][b];
+        part_mass[uint64_t(b) * gridDim.x + blockIdx.x] = m;
+        part_pe[uint64_t(b) * gridDim.x + blockIdx.x] = s;
+        if (s_cnt[b]) {
+            atomicAdd(&ints[b], s_cnt[b]);
+            atomicMin(&ints[kSelBuckets + b], s_min[b]);
+            atomicMax(&ints[2 * kSelBuckets + b], s_max[b]);
+            atomicMin(&ints[3 * kSelBuckets + b], s_kmin[b]);
+        }
+    }
+}
+
+// out[row] = sum over CTAs (in CTA order, then block_sum's fixed tree) of part[row * n_cta + i];  grid = 2 * kSelBuckets rows
+__global__ void __launch_bounds__(256)
+cvar_select_reduce_kernel(const double* __restrict__ part, int n_cta, double* __restrict__ out) {
+    __shared__ double s_red[8];
+    const double* p = part + uint64_t(blockIdx.x) * n_cta;
+    double acc = 0.0;
+    for (int i = threadIdx.x; i < n_cta; i += blockDim.x) acc += p[i];
+    const double total = block_sum(acc, s_red);
+    if (threadIdx.x == 0) out[blockIdx.x] = total;
 }
 
 // ---------------------------------------------------------------------------------------------------

@@ -558,6 +558,19 @@ class Engine:
         _native.check(self._lib.qb_expectation_device(self._ctx, ham.ham_id, _dtype_code(dtype), int(n_local), c_void_p(state_ptr), int(index_offset), byref(out)))
         return out.value
 
+    def cvar_select_device(self, ham: HamiltonianHandle, dtype, n_local: int, state_ptr: int, index_offset: int, cache_ptr: int, cache_mode: int,
+                           e_prefix: int, e_free: int, digit_kind: int, positions: Sequence[int], idx_mask: int, idx_value: int):
+        """One select pass of the sharded exact CVaR on a caller-owned shard (``qb_cvar_select_device``, include/queasars_b200.h) ->
+        (sums float64 [2, 256]: mass, sum p * E;  ints uint64 [4, 256]: count, min / max energy key, least physical index)."""
+        pos = np.zeros(8, dtype=np.int32)
+        pos[: len(positions)] = list(positions)
+        bits = len(positions) if digit_kind == 1 else 8
+        sums = np.empty((2, 256), dtype=np.float64)
+        ints = np.empty((4, 256), dtype=np.uint64)
+        _native.check(self._lib.qb_cvar_select_device(self._ctx, ham.ham_id, _dtype_code(dtype), int(n_local), c_void_p(state_ptr), int(index_offset),
+                                                      c_void_p(cache_ptr or None), int(cache_mode), int(e_prefix), int(e_free), int(digit_kind), int(bits),
+                                                      _native.ptr(pos), int(idx_mask), int(idx_value), _native.ptr(sums), _native.ptr(ints)))
+        return sums, ints
 
     def swap_global_p2p(self, dtype, n_local: int, state_ptr: int, peer_ptrs: Sequence[int], rank: int, local_positions: Sequence[int]):
         """Launch the fused swap + all-to-all kernel (asynchronous on the engine's stream; see include/queasars_b200.h)."""

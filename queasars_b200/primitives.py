@@ -764,7 +764,11 @@ class B200SamplerV2(_B200Primitive):
     def cvar_values(self, circuits, parameter_values, operator, alpha: float) -> np.ndarray:
         """Exact (shot-free) CVaR(alpha) of the diagonal ``operator`` on every circuit's full distribution |psi|^2:
         ``expectation.lower_tail_expectation_arrays(|psi|^2, E, alpha)`` over all 2^n basis states, computed on the device
-        (fast path of the sampler evaluators with ``sampler_shots=None``).  float64 array [len(circuits)]."""
+        (fast path of the sampler evaluators with ``sampler_shots=None``).  float64 array [len(circuits)].
+
+        Circuits too wide for one GPU run as one statevector sharded over the device set, one at a time, and the CVaR comes from
+        the sort-free weighted select of ``sharded._ShardedLogic.cvar`` (same definition, same stop entry, ties in logical basis
+        order); that route needs at least two devices and raises ``NotImplementedError`` on one."""
         return self._exact("cvar", circuits, parameter_values, operator, float(alpha))
 
     def _exact(self, kind: str, circuits, parameter_values, operator, alpha: float) -> np.ndarray:
@@ -782,33 +786,47 @@ class B200SamplerV2(_B200Primitive):
         width = widths.pop()
         if width != int(operator.num_qubits):
             raise ValueError(f"the circuits act on {width} qubits, the operator on {int(operator.num_qubits)}")
-        if self._needs_sharding(width):
-            raise NotImplementedError(
-                f"exact CVaR / expectation values need the whole {width}-qubit statevector on one device; a state that must be sharded "
-                "over several GPUs is only supported with shots"
-            )
         fp = _operator_fingerprint(operator)
-        if not self.hamiltonian_for(operator, build_table=(False if kind == "cvar" else None), fingerprint=fp).diagonal:
+        sharded = self._needs_sharding(width)
+        if not self.hamiltonian_for(operator, build_table=(False if kind == "cvar" or sharded else None), fingerprint=fp).diagonal:
             raise ValueError("Operator string contains non-diagonal terms")
+        if sharded and len(self.engines) < 2:
+            raise NotImplementedError(
+                f"exact CVaR / expectation values of a {width}-qubit state that must be sharded need a device set of at least two GPUs "
+                "(devices=[...] or 'all'); on one device use shots"
+            )
         return np.asarray(self._submit((kind, id(operator), fp, alpha, width), (operator, circuits, parameter_values)), dtype=np.float64)
 
     def _execute_exact(self, key, payloads):
-        kind, _, fp, alpha, _ = key
+        kind, _, fp, alpha, width = key
         operator = payloads[0][0]
         circuits, values, sizes = [], [], []
         for _, circs, vals in payloads:
             sizes.append(len(circs))
             circuits.extend(circs)
             values.extend(vals)
-        resolved = self._resolve_all(circuits, values, probabilities_only=True)
+        if self._needs_sharding(width):
+            # one statevector over the whole device set, circuit after circuit (sharded.py): the select passes of
+            # _ShardedLogic.cvar, or <H> for alpha ~ 1 on the operator evaluator; the duplicate-merged terms of the device Hamiltonian
+            ham = self.hamiltonian_for(operator, build_table=False, fingerprint=fp)
+            flat = []
+            with self._shard_lock:
+                sv = self._sharded_state(width)
+                for circuit, vals in zip(circuits, values):
+                    gates, bound = self._bound_gates(circuit, vals)
+                    sv.reset()
+                    sv.run(gates, bound)
+                    flat.append(sv.cvar(ham.z_masks, ham.coeffs, alpha)[0] if kind == "cvar" else sv.diagonal_expectation(ham.z_masks, ham.coeffs))
+        else:
+            resolved = self._resolve_all(circuits, values, probabilities_only=True)
 
-        def call(slot, plans, params):
-            engine = self.engines[slot]
-            if kind == "cvar":
-                return list(engine.cvar(plans, params, self.hamiltonian_for(operator, build_table=False, slot=slot, fingerprint=fp), alpha))
-            return list(engine.expectation(plans, params, self.hamiltonian_for(operator, slot=slot, fingerprint=fp)))
+            def call(slot, plans, params):
+                engine = self.engines[slot]
+                if kind == "cvar":
+                    return list(engine.cvar(plans, params, self.hamiltonian_for(operator, build_table=False, slot=slot, fingerprint=fp), alpha))
+                return list(engine.expectation(plans, params, self.hamiltonian_for(operator, slot=slot, fingerprint=fp)))
 
-        flat = self._run_per_device(resolved, call)
+            flat = self._run_per_device(resolved, call)
         out, pos = [], 0
         for n in sizes:
             out.append(np.asarray(flat[pos : pos + n], dtype=np.float64))

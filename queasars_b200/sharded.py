@@ -27,7 +27,7 @@ Two drivers share the schedule (``_ShardedLogic``):
                                ``cudaDeviceEnablePeerAccess`` instead of IPC, reductions on the host.
 
 The shard-local arithmetic is delegated to a *backend* object (``apply``, ``diagonal_expectation``, ``pauli_expectation``,
-``sample``, ``swap_p2p``); the product default drives the CUDA engine.  Tests inject a NumPy backend to exercise the
+``sample``, ``cvar_select``, ``swap_p2p``); the product default drives the CUDA engine.  Tests inject a NumPy backend to exercise the
 multi-rank host logic on CPU with the gloo backend.
 """
 from __future__ import annotations
@@ -49,12 +49,31 @@ def _state_ptr(state) -> int:
     return state.data_ptr() if hasattr(state, "data_ptr") else int(state)
 
 
+_SIGN = np.uint64(1 << 63)
+
+
+def energy_keys(energies) -> np.ndarray:
+    """Order-preserving uint64 image of float64 energies (``energy_key`` of qb_kernels.cuh): ascending keys are ascending
+    energies, and -0.0 gets the key of +0.0 (a radix sort and ``numpy.argsort(kind="stable")`` treat them as tied)."""
+    u = np.ascontiguousarray(energies, dtype=np.float64).view(np.uint64).copy()
+    u[u == _SIGN] = 0
+    return np.where((u >> np.uint64(63)) == 1, ~u, u | _SIGN)
+
+
+def energy_from_key(key: int) -> float:
+    """Inverse of ``energy_keys`` (a key of +-0.0 gives +0.0)."""
+    key = int(key)
+    u = key & ((1 << 63) - 1) if key >> 63 else ~key & ((1 << 64) - 1)
+    return float(np.asarray([u], dtype=np.uint64).view(np.float64)[0])
+
+
 class CudaShardBackend:
     """Runs the shard-local work on the CUDA engine.  ``state`` is a torch tensor (only its ``data_ptr`` and stream are used)
     or a raw device address."""
 
     def __init__(self, engine):
         self.engine = engine
+        self._select_ham = None
 
     @staticmethod
     def _join_torch_stream(state):
@@ -94,6 +113,18 @@ class CudaShardBackend:
         self._join_torch_stream(state)
         return self.engine.sample_device("complex128", n_local, _state_ptr(state), uniforms)
 
+    def cvar_select(self, state, cache, cache_mode: int, z_masks, coeffs, n_total: int, n_local: int, index_offset: int, spec):
+        """One select pass of ``_ShardedLogic.cvar`` on this shard (``qb_cvar_select_device``); ``cache`` is the idle spare buffer."""
+        key = (n_total, tuple(int(z) for z in z_masks), tuple(float(c) for c in coeffs))
+        if self._select_ham is None or self._select_ham[0] != key:  # one Hamiltonian for all passes of a call
+            from .operators import SparsePauliOp
+
+            op = SparsePauliOp._raw(n_total, [0] * len(key[1]), list(key[1]), list(key[2]))
+            self._select_ham = (key, self.engine.hamiltonian(op, build_table=False))
+        self._join_torch_stream(state)
+        return self.engine.cvar_select_device(self._select_ham[1], "complex128", n_local, _state_ptr(state), index_offset,
+                                              0 if cache is None else _state_ptr(cache), cache_mode, *spec)
+
     def swap_p2p(self, state, peer_ptrs: Sequence[int], n_local: int, rank: int, local_positions: Sequence[int]) -> None:
         """Fused swap + all-to-all into the peers' buffers; returns when this rank's stores have been issued and completed."""
         self._join_torch_stream(state)
@@ -108,6 +139,7 @@ class _ShardedLogic:
       _swap(lp)                                   exchange the g rank bits with local positions lp (data movement only)
       _sum_over_shards(fn)                        sum over all shards of fn(rank, state) -> float  (every caller gets the total)
       _shard_masses()                             |shard|^2 of all shards, ndarray [world]
+      _select_pass(z, c, cache_mode, spec)        every shard's bucket arrays of one cvar select pass, in rank order
       _sample_shards(owner, local_u)              physical indices of the shots (owner[s] = shard of shot s), int64 [shots]"""
 
     def _init_logic(self, n_qubits: int, world: int, min_local: int):
@@ -244,6 +276,81 @@ class _ShardedLogic:
                 raise NotImplementedError("a Pauli term flips more qubits than fit one shard next to the rank bits")
             self._swap_all_global(sorted(free[: self.n_global]))
         return float(total)
+
+    def cvar(self, z_masks: Sequence[int], coeffs: Sequence[float], alpha: float, cache: bool = True) -> tuple[float, int]:
+        """Exact CVaR(alpha) of the diagonal Hamiltonian sum_t c_t Z^{z_t} on the whole distribution |psi|^2, no shots:
+        ``expectation.lower_tail_expectation_arrays`` (the single-GPU ``Engine.cvar``) without gathering or sorting anything.
+        Returns (value, logical basis index of the stop entry; -1 when the whole distribution weighs less than the bound).
+
+        The stable ascending (E(k), logical k) order is the order of the composite key (energy_key(E(k)), k) -- for alpha ~ 1
+        the key is k alone -- and the stop entry is the smallest key whose inclusive mass reaches alpha - isclose tolerance: a
+        weighted selection.  Every pass histograms the next 8-bit digit of the key over the entries matching the prefix fixed
+        so far, on every shard (``qb_cvar_select_device``); the host adds the shards' buckets in rank order and keeps the bucket
+        in which the bound falls.  The energy phase ends as soon as that bucket holds one distinct energy, the select as soon
+        as it holds one entry.  Logical index bits are read from their physical positions: no data moves.  The first pass
+        stores (p, E) of every entry in the idle spare buffer, the later ones read it from there.  Every rank makes the same
+        decisions from the same all-gathered numbers, so every caller gets the same result.  ``cache=False`` recomputes p and E
+        from the state on every pass instead (same values)."""
+        from . import expectation as ex
+        from .engine import merge_duplicate_terms
+
+        ex.check_alpha(alpha)
+        _, zs, cs = merge_duplicate_terms(np.zeros(len(z_masks), dtype=np.uint64), np.asarray(z_masks, dtype=np.uint64), np.asarray(coeffs, dtype=np.float64))
+        phys = np.asarray([self._physical_mask(z) for z in zs], dtype=np.uint64)
+        cf = np.ascontiguousarray(np.real(cs), dtype=np.float64)
+        bound = alpha - (1e-8 + 1e-5 * alpha)
+        energy_phase = not ex._close(alpha, 1)
+        e_prefix, e_free = 0, 64  # energy key bits fixed so far (64 open: no constraint)
+        idx_mask = idx_value = 0  # physical index bits fixed by the logical-index prefix
+        hi = self.n_qubits  # logical bits >= hi are fixed
+        below_m = below_s = 0.0  # mass and sum p * E of every entry whose key is below the current prefix range
+        self.cvar_passes = 0
+        while True:
+            if energy_phase:
+                lo, spec = hi, (e_prefix, e_free, 0, (), idx_mask, idx_value)
+            else:
+                lo = max(0, hi - 8)
+                spec = (e_prefix, e_free, 1, [self.position[q] for q in range(lo, hi)], idx_mask, idx_value)
+            parts = self._select_pass(phys, cf, 0 if not cache else 1 if self.cvar_passes == 0 else 2, spec)
+            self.cvar_passes += 1
+            mass, pe = np.zeros(256), np.zeros(256)
+            count = np.zeros(256, dtype=np.uint64)
+            emin, emax, kmin = np.full(256, ~np.uint64(0)), np.zeros(256, dtype=np.uint64), np.full(256, ~np.uint64(0))
+            for sums, ints in parts:  # rank order: every rank adds the same numbers in the same order
+                mass, pe = mass + sums[0], pe + sums[1]
+                count = count + ints[0]
+                emin, emax, kmin = np.minimum(emin, ints[1]), np.maximum(emax, ints[2]), np.minimum(kmin, ints[3])
+            mass_l, pe_l, count_l = mass.tolist(), pe.tolist(), count.tolist()
+            before_m, before_s, run_m, run_s = [], [], below_m, below_s
+            for b in range(256):
+                before_m.append(run_m), before_s.append(run_s)
+                run_m += mass_l[b]
+                run_s += pe_l[b]
+            if self.cvar_passes == 1 and run_m < bound:  # the whole distribution weighs less than the bound: every entry is taken
+                return run_s / alpha, -1
+            hits = [b for b in range(256) if count_l[b] and before_m[b] + mass_l[b] >= bound]
+            if hits:
+                pick = hits[0]
+            else:  # this bucket's parent reached the bound, its digits' sums miss it by rounding only: the last entry with mass stops
+                pick = ([b for b in range(256) if count_l[b] and mass_l[b] > 0] or [b for b in range(256) if count_l[b]])[-1]
+            below_m, below_s = before_m[pick], before_s[pick]
+            if count_l[pick] == 1:
+                p, e = mass_l[pick], energy_from_key(emin[pick])
+                k = int(kmin[pick])
+                logical = sum(((k >> self.position[q]) & 1) << q for q in range(self.n_qubits))
+                return (below_s + min(alpha - below_m, p) * e) / alpha, logical
+            if energy_phase:
+                if emin[pick] == emax[pick]:  # one distinct energy left: ties are ordered by the logical index
+                    e_prefix, e_free, energy_phase = int(emin[pick]), 0, False
+                else:
+                    e_prefix, e_free = (e_prefix << 8) | pick, e_free - 8
+                continue
+            for j, q in enumerate(range(lo, hi)):
+                idx_mask |= 1 << self.position[q]
+                idx_value |= ((pick >> j) & 1) << self.position[q]
+            hi = lo
+            if hi == 0:
+                raise RuntimeError("cvar select: the full logical index matched more than one entry")
 
     def sample(self, shots: int, seed=None, uniforms: Optional[np.ndarray] = None) -> np.ndarray:
         """``shots`` basis-state indices (logical qubit order) drawn from |psi|^2; every caller gets all of them.
@@ -450,6 +557,24 @@ class ShardedStatevector(_ShardedLogic):
         self._dist.all_reduce(masses, group=self.group)
         return masses.cpu().numpy()
 
+    def _select_pass(self, z_masks, coeffs, cache_mode: int, spec) -> list:
+        sums, ints = self.backend.cvar_select(self.state, self.spare, cache_mode, z_masks, coeffs, self.n_qubits, self.n_local, self.index_offset, spec)
+        if self.world == 1:
+            return [(sums, ints)]
+        # all_gather, not all_reduce: every rank adds the shards' buckets in rank order with the same host arithmetic and so takes
+        # the same bucket decision (the bits travel as int64)
+        torch = self._torch
+        mine = np.concatenate([np.ascontiguousarray(sums, dtype=np.float64).reshape(-1).view(np.int64),
+                               np.ascontiguousarray(ints, dtype=np.uint64).reshape(-1).view(np.int64)])
+        t = torch.from_numpy(mine).to(self.device)
+        parts = [torch.empty_like(t) for _ in range(self.world)]
+        self._dist.all_gather(parts, t, group=self.group)
+        out = []
+        for part in parts:
+            a = part.cpu().numpy()
+            out.append((a[:512].view(np.float64).reshape(2, 256), a[512:].view(np.uint64).reshape(4, 256)))
+        return out
+
     def _sample_shards(self, owner: np.ndarray, local_u: np.ndarray) -> np.ndarray:
         physical = np.zeros(owner.size, dtype=np.int64)
         mine = np.nonzero(owner == self.rank)[0]
@@ -553,6 +678,11 @@ class LocalShardedStatevector(_ShardedLogic):
     def _shard_masses(self) -> np.ndarray:
         z, c = np.zeros(1, dtype=np.uint64), np.ones(1)
         return np.asarray(self._each(lambda r: self.backends[r].diagonal_expectation(self._state(r), z, c, self.n_qubits, self.n_local, r << self.n_local)))
+
+    def _select_pass(self, z_masks, coeffs, cache_mode: int, spec) -> list:
+        spare = self._bufs[1 - self._cur]
+        return self._each(lambda r: self.backends[r].cvar_select(self._state(r), spare[r].ptr, cache_mode, z_masks, coeffs, self.n_qubits, self.n_local,
+                                                                 r << self.n_local, spec))
 
     def _sample_shards(self, owner: np.ndarray, local_u: np.ndarray) -> np.ndarray:
         physical = np.zeros(owner.size, dtype=np.int64)
