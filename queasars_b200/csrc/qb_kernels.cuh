@@ -115,9 +115,6 @@ __device__ __forceinline__ double ld_cg(const double* p) {
 #ifndef QB_PLAIN_FAST
 #define QB_PLAIN_FAST 1
 #endif
-#ifndef QB_PLAIN_PRELOAD
-#define QB_PLAIN_PRELOAD 0
-#endif
 #ifndef QB_TABLE_LD
 #define QB_TABLE_LD "ld.global.nc.f64"
 #endif
@@ -290,7 +287,8 @@ constexpr int kMaxInitQubits = 64;
 
 // dispatch word: variant | cpos << 6 | dpos << 11 | dflag << 16 | cb << 17 | tb << 20 | treg << 23
 //   variant bit 5 (dense ops): the matrix's top-left entry is real (gamma == 0) -> 14 instead of 16 multiply-adds per pair
-//   variant 48 + b (uncontrolled dense on register bit b): the whole first column is real (gamma == phi == 0) -> 12
+//   variant 48 + b (uncontrolled dense on register bit b): the whole first column is real (gamma == phi == 0) -> 12; with bit 31
+//         (QB_PLAIN_FAST) the op loop runs it in tangent form instead -> 8 (apply_tangent)
 //   cpos  tile-local position of a thread-bit control; 31 = none (bit 31 of the test word is always set), 30 = an external
 //         control that is 0 for this tile (bit 30 is never set)
 //   dpos  tile-local position of a thread-bit diagonal target; 31 = use dflag (external target, resolved per tile)
@@ -330,22 +328,90 @@ __device__ __forceinline__ void dense_by_bit(uint32_t v, typename Cx<T>::type (&
     }
 }
 
-// the same for the op loop's direct path (real first column), matrix entries already in registers: their shared-memory loads
-// are issued before the two branches instead of behind them
+// Tangent form of a plain op (uncontrolled, real first column): M = [[c, -s E], [s, c E]] = c [[1, -t E], [t, E]] with t = s / c.
+// The body applies the bracket -- 2 multiplies + 6 multiply-adds per pair instead of REAL10's 4 + 8 -- and the sweep multiplies
+// its amplitudes by the product of the c's once before the store (sweep_kernel: stage_tangent, s_scale).  Record (staged in place
+// of the op's matrix): m[0] = E, m[1].x = t.  In place with two temporaries: y is dead once w = E y is formed, x once x' is.
+template <typename T, int R, int B>
+__device__ __forceinline__ void apply_tangent(typename Cx<T>::type (&a)[1 << R], const typename Cx<T>::type* __restrict__ m) {
+    using C = typename Cx<T>::type;
+    const C e = m[0];
+    const T t = m[1].x;
+#pragma unroll
+    for (int j = 0; j < (1 << R); ++j) {
+        if (j & (1 << B)) continue;
+        const C x = a[j], y = a[j | (1 << B)];
+        T w0 = e.x * y.x;
+        T w1 = e.x * y.y;
+        w0 = fma(-e.y, y.y, w0);
+        w1 = fma(e.y, y.x, w1);
+        a[j | (1 << B)].x = fma(t, x.x, w0);
+        a[j | (1 << B)].y = fma(t, x.y, w1);
+        a[j].x = fma(-t, w0, x.x);
+        a[j].y = fma(-t, w1, x.y);
+    }
+}
+
+// the op loop's direct path: a tangent-form plain op on register bit v (< R), two predictable branches
 template <typename T, int R>
-__device__ __forceinline__ void plain_by_bit(uint32_t v, typename Cx<T>::type (&a)[1 << R], const typename Cx<T>::type m00, const typename Cx<T>::type m01,
-                                             const typename Cx<T>::type m10, const typename Cx<T>::type m11) {
+__device__ __forceinline__ void tangent_by_bit(uint32_t v, typename Cx<T>::type (&a)[1 << R], const typename Cx<T>::type* __restrict__ m) {
     if (v & 2u) {
         if constexpr (R > 3) {
-            if (v & 1u) apply_dense<T, R, 3, -1, true, true>(a, m00, m01, m10, m11);
-            else apply_dense<T, R, 2, -1, true, true>(a, m00, m01, m10, m11);
+            if (v & 1u) apply_tangent<T, R, 3>(a, m);
+            else apply_tangent<T, R, 2>(a, m);
         } else {
-            apply_dense<T, R, 2, -1, true, true>(a, m00, m01, m10, m11);
+            apply_tangent<T, R, 2>(a, m);
         }
     } else {
-        if (v & 1u) apply_dense<T, R, 1, -1, true, true>(a, m00, m01, m10, m11);
-        else apply_dense<T, R, 0, -1, true, true>(a, m00, m01, m10, m11);
+        if (v & 1u) apply_tangent<T, R, 1>(a, m);
+        else apply_tangent<T, R, 0>(a, m);
     }
+}
+
+// Amplitudes in tangent form grow by 1 / |c| per op (the norm of M / c), so the sweep keeps a plain op in that form only while
+// the product of the |c|'s of its plain ops so far stays >= kTangentMinScale: amplitudes stay below 2^400 (double) / 2^40 (float),
+// their squares and the pair updates finite.  The bound is a guarantee for any circuit, not a statistic of a workload.
+template <typename T> struct TangentBudget;
+template <> struct TangentBudget<double> { static constexpr double kMinScale = 0x1p-400; };
+template <> struct TangentBudget<float> { static constexpr double kMinScale = 0x1p-40; };
+
+// One warp, after the sweep's matrices are staged: every plain op (bit 31 of its word) within the budget gets its tangent record;
+// one over the budget, or with c == 0, keeps its matrix and drops to the real-top-left body (bits 31 and 4 cleared: variant
+// 48 + b -> 32 + b, which never reads m00.y).  Writes the product of the kept ops' c's (signed) to *s_scale; 1 without one.
+template <typename T>
+__device__ __forceinline__ void stage_tangent(typename Cx<T>::type* s_mat, uint32_t* s_word0, int n_sop, int lane, double* s_scale) {
+    double carry = 1.0, scale = 1.0;
+#pragma unroll 1
+    for (int o0 = 0; o0 < n_sop; o0 += 32) {
+        const int o = o0 + lane;
+        const bool plain = o < n_sop && int32_t(s_word0[o]) < 0;
+        if (!__any_sync(0xffffffffu, plain)) continue;
+        typename Cx<T>::type* m = s_mat + o * 4;
+        const double c = plain ? double(m[0].x) : 1.0;
+        // inclusive prefix product of |c| over the sweep's plain ops, in op order (an op with c == 0 is skipped, not counted)
+        double p = (c != 0.0) ? fabs(c) : 1.0;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            const double q = __shfl_up_sync(0xffffffffu, p, d);
+            if (lane >= d) p *= q;
+        }
+        p *= carry;
+        carry = __shfl_sync(0xffffffffu, p, 31);
+        if (plain && c != 0.0 && p >= TangentBudget<T>::kMinScale) {
+            const double r = 1.0 / c;
+            const double t = double(m[2].x) * r;
+            typename Cx<T>::type e;
+            e.x = T(double(m[3].x) * r), e.y = T(double(m[3].y) * r);
+            m[0] = e;
+            m[1].x = T(t);
+            scale *= c;
+        } else if (plain) {
+            s_word0[o] &= ~(0x80000000u | 16u);
+        }
+    }
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1) scale *= __shfl_xor_sync(0xffffffffu, scale, d);
+    if (lane == 0) *s_scale = scale;
 }
 
 // register-controlled dense gate: c = v - R enumerates (B, CB) as B * (R - 1) + k with CB = the k-th register bit other than B;
@@ -452,6 +518,7 @@ sweep_kernel(const BatchEntry* __restrict__ entries, int sweep_idx, int n_eff, i
     __shared__ uint64_t s_gi[2][8];
     __shared__ double s_red[32];
     __shared__ int s_has_ext;
+    __shared__ double s_scale;  // product of the c's of the sweep's plain ops in tangent form (stage_tangent)
 
     pdl_launch_dependents();  // a dependent launch may start its own staging now; it waits for this grid's stores in pdl_wait()
     const BatchEntry& ge = entries[blockIdx.y];
@@ -579,7 +646,12 @@ sweep_kernel(const BatchEntry* __restrict__ entries, int sweep_idx, int n_eff, i
         }
         if ((ge.index_offset >> n_eff) != 0) p_thread.x = T(0), p_thread.y = T(0);  // rank bits above the local register start in |0>
     }
+    __syncthreads();  // matrices staged
+#if QB_PLAIN_FAST
+    // plain ops to tangent form in place (their words patched before the per-tile word copy reads them)
+    if (tid < 32) stage_tangent<T>(s_mat, s_word0, n_sop, tid, &s_scale);
     __syncthreads();
+#endif
     const bool has_ext = s_has_ext != 0;
 
     C* __restrict__ st = reinterpret_cast<C*>(ge.state);
@@ -702,14 +774,7 @@ sweep_kernel(const BatchEntry* __restrict__ entries, int sweep_idx, int n_eff, i
                 word_next = s_w[o + 1];  // prefetch the next dispatch word behind this op's arithmetic
 #if QB_PLAIN_FAST
                 if (int32_t(word) < 0) {
-#if QB_PLAIN_PRELOAD
-                    const C* m = s_mat + o * 4;
-                    C m00, m10;
-                    m00.x = m[0].x, m00.y = T(0), m10.x = m[2].x, m10.y = T(0);  // (real entries: the imaginary parts are never read)
-                    plain_by_bit<T, R>(word & 3u, a, m00, m[1], m10, m[3]);
-#else
-                    dense_by_bit<T, R, true, true>(word & 3u, a, s_mat + o * 4);
-#endif
+                    tangent_by_bit<T, R>(word & 3u, a, s_mat + o * 4);
                     continue;
                 }
 #endif
@@ -719,6 +784,14 @@ sweep_kernel(const BatchEntry* __restrict__ entries, int sweep_idx, int n_eff, i
 
             // ---- store ----
             if (last) {
+#if QB_PLAIN_FAST
+                // undo the tangent form's factoring of the sweep's plain ops: every state outside the kernel stays as it was
+                const double scale = s_scale;
+                if (scale != 1.0) {
+#pragma unroll
+                    for (int j = 0; j < kNReg; ++j) a[j].x *= T(scale), a[j].y *= T(scale);
+                }
+#endif
                 Idx ix[kNReg];
                 ix[0] = Idx(base) | gthr_last;
 #pragma unroll

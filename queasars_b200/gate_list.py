@@ -156,16 +156,18 @@ def defer_phases(ops: Sequence[KernelOp], drop_final: bool = False) -> list[Kern
 
 
 def dfma_per_amplitude(op: KernelOp) -> float:
-    """FP64 multiply-add-class instructions per amplitude the sweep kernel spends on ``op`` (roofline accounting in bench.py):
-    a dense 2x2 gate costs 16 per amplitude pair, 14 when its top-left entry is real (no global phase), 12 when the bottom-left
-    entry is real as well (phi == 0: the R_Y * D form of the phase-deferred front end); a diagonal 4 per amplitude it touches;
-    a controlled op touches half of the amplitudes."""
+    """FP64 multiply-add-class instructions per amplitude the sweep kernel spends on ``op`` (roofline accounting in bench.py,
+    sweep balancing in the planner): a dense 2x2 gate costs 16 per amplitude pair, 14 when its top-left entry is real (no global
+    phase); an uncontrolled one whose bottom-left entry is real as well (phi == 0: the R_Y * D form of the phase-deferred front
+    end) runs in tangent form, c * [[1, -t E], [t, E]], at 8 per pair, its c folded into one scale per sweep (2 per amplitude,
+    not counted here; the rare op over the sweep's growth budget runs the 14 body instead); a diagonal 4 per amplitude it
+    touches; a controlled op touches half of the amplitudes."""
     if op.kind == DIAG:
         per = 4.0
     else:
         real00 = op.gamma.slot < 0 and op.gamma.const == 0.0
-        real10 = real00 and op.phi.is_zero and op.control < 0  # only the uncontrolled REAL10 bodies are compiled
-        per = 6.0 if real10 else (7.0 if real00 else 8.0)
+        plain = real00 and op.phi.is_zero and op.control < 0  # only uncontrolled gates have the tangent body
+        per = 4.0 if plain else (7.0 if real00 else 8.0)
     return per * (1.0 if op.control < 0 else 0.5)
 
 
