@@ -298,6 +298,22 @@ namespace {
 
 size_t amp_bytes(int dtype) { return dtype == QB_C128 ? 16 : 8; }
 
+size_t workspace_limit_of(const qb_context* ctx) { return ctx->workspace_limit ? ctx->workspace_limit : ctx->default_workspace; }
+
+// f(double()) for complex128 amplitudes, f(float()) for every other dtype code: `using T = decltype(t);` picks the kernel instance
+template <typename F> int with_dtype(int dtype, F&& f) { return dtype == QB_C128 ? f(double()) : f(float()); }
+
+// rows of `row_bytes` between sorted device position pos and caller index order[pos]: scatter_rows puts device rows in caller
+// order, gather_rows caller rows in device order
+void scatter_rows(void* caller, const void* device, const std::vector<int>& order, size_t row_bytes) {
+    for (size_t pos = 0; pos < order.size(); ++pos)
+        std::memcpy(static_cast<char*>(caller) + size_t(order[pos]) * row_bytes, static_cast<const char*>(device) + pos * row_bytes, row_bytes);
+}
+void gather_rows(void* device, const void* caller, const std::vector<int>& order, size_t row_bytes) {
+    for (size_t pos = 0; pos < order.size(); ++pos)
+        std::memcpy(static_cast<char*>(device) + pos * row_bytes, static_cast<const char*>(caller) + size_t(order[pos]) * row_bytes, row_bytes);
+}
+
 // terms of one x-mask group staged in shared memory (24 B each, inside the default 48 KB); longer lists are read from global memory
 constexpr int kMaxStagedTerms = 2000;
 // diagonal terms per diag_table_kernel launch (16 B each in shared memory); longer lists build the table in several launches
@@ -720,15 +736,14 @@ template <typename T> int launch_expectation_t(qb_context* ctx, DeviceBatch& b) 
 
 int launch_expectation(qb_context* ctx, DeviceBatch& b) {
     if (!b.ham) return fail(QB_ERR_INVALID, "batch was created without a Hamiltonian");
-    return b.dtype == QB_C128 ? launch_expectation_t<double>(ctx, b) : launch_expectation_t<float>(ctx, b);
+    return with_dtype(b.dtype, [&](auto t) { return launch_expectation_t<decltype(t)>(ctx, b); });
 }
 
 int batch_read(qb_context* ctx, DeviceBatch& b, double* out_values) {
     QB_TRY(ctx->pin_out.reserve(sizeof(double) * size_t(b.batch)));
     QB_CUDA(cudaMemcpyAsync(ctx->pin_out.p, b.out.p, sizeof(double) * size_t(b.batch), cudaMemcpyDeviceToHost, ctx->stream));
     QB_CUDA(cudaStreamSynchronize(ctx->stream));
-    const double* sorted = static_cast<const double*>(ctx->pin_out.p);
-    for (int pos = 0; pos < b.batch; ++pos) out_values[b.order[pos]] = sorted[pos];
+    scatter_rows(out_values, ctx->pin_out.p, b.order, sizeof(double));
     return QB_OK;
 }
 
@@ -756,7 +771,7 @@ int evaluate_single_graph(qb_context* ctx, int64_t plan_id, Plan* pl, Ham* ham, 
                           const int64_t* param_offsets, double* out_values, bool* handled) {
     *handled = false;
     const size_t state_bytes = (size_t(1) << pl->n_eff) * amp_bytes(pl->dtype) * size_t(copies);
-    const size_t budget = std::min<size_t>(size_t(4) << 30, (ctx->workspace_limit ? ctx->workspace_limit : ctx->default_workspace) / 8);
+    const size_t budget = std::min<size_t>(size_t(4) << 30, workspace_limit_of(ctx) / 8);
     if (!ctx->use_graphs || state_bytes > budget / 4) return QB_OK;
     for (int i = 0; i < copies; ++i)
         if (param_offsets[i + 1] - param_offsets[i] != pl->n_params)
@@ -831,8 +846,7 @@ int evaluate_single_graph(qb_context* ctx, int64_t plan_id, Plan* pl, Ham* ham, 
 
 size_t max_batch_for(qb_context* ctx, const Plan* pl) {
     const size_t state_bytes = (size_t(1) << pl->n_eff) * amp_bytes(pl->dtype);
-    const size_t limit = ctx->workspace_limit ? ctx->workspace_limit : ctx->default_workspace;
-    return std::min<size_t>(65535, std::max<size_t>(1, limit / state_bytes));  // 65535: grid.y of the batched launches
+    return std::min<size_t>(65535, std::max<size_t>(1, workspace_limit_of(ctx) / state_bytes));  // 65535: grid.y of the batched launches
 }
 
 // E(k) of the Hamiltonian's diagonal terms for k < 2^n_eff into `table` (asynchronous on the context's stream)
@@ -851,8 +865,6 @@ int fill_diag_table(qb_context* ctx, const Ham& ham, double* table, int n_eff) {
     }
     return QB_OK;
 }
-
-size_t workspace_limit_of(const qb_context* ctx) { return ctx->workspace_limit ? ctx->workspace_limit : ctx->default_workspace; }
 
 // Build (once per Hamiltonian and state width) what qb_evaluate_cvar reads: E(k) in basis order (8 B per amplitude); with `sorted`
 // also a stable ascending radix sort of (E(k), k) -> perm (sorted position -> k, 4 B) and E_sorted (8 B).  CUB's radix sort is
@@ -1005,6 +1017,53 @@ int launch_terms_t(qb_context* ctx, const DeviceBatch& b, const Obs& ob, double*
                 states, size, size, g.xmask, ob.z.as<uint64_t>(), ob.im.as<int8_t>(), t0, t1, t0, t1 - t0, d_partials);
             return check_launch(ctx, "expect_terms_group_kernel");
         }));
+    }
+    return QB_OK;
+}
+
+// shots from each of the n states (stride `size`): chunk probabilities, their prefix sums, one search per uniform; indices stay
+// below `valid_size`
+template <typename T>
+int launch_sampling_t(qb_context* ctx, const typename qb::Cx<T>::type* states, uint64_t size, int n, uint64_t valid_size, const double* d_uniforms,
+                      int shots, double* d_chunks, int64_t* d_indices) {
+    const uint64_t n_chunks = size >> qb::kChunkBits;
+    dim3 cgrid(unsigned(std::min<uint64_t>((n_chunks + 7) / 8, 2048)), unsigned(n));
+    dim3 sgrid(unsigned((shots + 7) / 8), unsigned(n));
+    qb::chunk_prob_kernel<T><<<cgrid, 256, 0, ctx->stream>>>(states, size, n_chunks, d_chunks);
+    QB_TRY(check_launch(ctx, "chunk_prob_kernel"));
+    qb::scan_chunks_kernel<<<n, 1024, 0, ctx->stream>>>(d_chunks, n_chunks);
+    QB_TRY(check_launch(ctx, "scan_chunks_kernel"));
+    qb::sample_kernel<T><<<sgrid, 256, 0, ctx->stream>>>(states, size, d_chunks, n_chunks, valid_size, d_uniforms, shots, d_indices);
+    return check_launch(ctx, "sample_kernel");
+}
+
+// Every plan of a call whose chunks share one operator's device data must act on the operator's `n_qubits` and share the first
+// plan's state width and dtype.  `acts`: the operator's subject and verb in the message; `call`: the call's name.
+int check_plans(qb_context* ctx, int batch, const int64_t* plan_ids, int n_qubits, const char* acts, const char* call, const Plan** first) {
+    for (int i = 0; i < batch; ++i) {
+        const Plan* pl = find_plan(ctx, plan_ids[i]);
+        if (!pl) return fail(QB_ERR_NOT_FOUND, "unknown plan id " + std::to_string(plan_ids[i]));
+        if (i == 0) *first = pl;
+        if (pl->n_qubits != n_qubits)
+            return fail(QB_ERR_INVALID, std::string(acts) + " on " + std::to_string(n_qubits) + " qubits, circuit " + std::to_string(i) + " on " +
+                                            std::to_string(pl->n_qubits));
+        if (pl->n_eff != (*first)->n_eff || pl->dtype != (*first)->dtype)
+            return fail(QB_ERR_INVALID, std::string("all plans of one ") + call + " call must share state width and dtype");
+    }
+    return QB_OK;
+}
+
+// Runs `batch` circuits through the context's one-shot batch, `chunk` at a time; after each chunk's launches
+// readout(b, lo) reads its resident states, which hold caller entries lo + b.order[pos] in sorted device order.
+template <typename ReadOut>
+int run_oneshot(qb_context* ctx, int batch, const int64_t* plan_ids, const double* params, const int64_t* param_offsets, const Ham* ham, int chunk,
+                ReadOut&& readout) {
+    for (int lo = 0; lo < batch; lo += chunk) {
+        DeviceBatch& b = ctx->oneshot;
+        QB_TRY(build_batch(ctx, b, std::min(chunk, batch - lo), plan_ids + lo, ham, nullptr, 1, 0));
+        QB_TRY(batch_upload_params(ctx, b, params, param_offsets + lo));
+        QB_TRY(launch_circuits(ctx, b, nullptr));
+        QB_TRY(readout(b, lo));
     }
     return QB_OK;
 }
@@ -1614,16 +1673,10 @@ int qb_evaluate_expectation(qb_context* ctx, int batch, const int64_t* plan_ids,
         if (handled) return QB_OK;
     }
     const int chunk = int(std::min<size_t>(size_t(batch), max_batch_for(ctx, first)));
-    for (int lo = 0; lo < batch; lo += chunk) {
-        const int n = std::min(chunk, batch - lo);
-        DeviceBatch& b = ctx->oneshot;
-        QB_TRY(build_batch(ctx, b, n, plan_ids + lo, ham, nullptr, 1, 0));
-        QB_TRY(batch_upload_params(ctx, b, params, param_offsets + lo));
-        QB_TRY(launch_circuits(ctx, b, nullptr));
+    return run_oneshot(ctx, batch, plan_ids, params, param_offsets, ham, chunk, [&](DeviceBatch& b, int lo) {
         QB_TRY(launch_expectation(ctx, b));
-        QB_TRY(batch_read(ctx, b, out_values + lo));
-    }
-    return QB_OK;
+        return batch_read(ctx, b, out_values + lo);
+    });
 }
 
 int qb_sample(qb_context* ctx, int batch, const int64_t* plan_ids, const double* params, const int64_t* param_offsets, int shots,
@@ -1635,12 +1688,8 @@ int qb_sample(qb_context* ctx, int batch, const int64_t* plan_ids, const double*
     Plan* first = find_plan(ctx, plan_ids[0]);
     if (!first) return fail(QB_ERR_NOT_FOUND, "unknown plan id " + std::to_string(plan_ids[0]));
     const int chunk = int(std::min<size_t>(size_t(batch), max_batch_for(ctx, first)));
-    for (int lo = 0; lo < batch; lo += chunk) {
-        const int n = std::min(chunk, batch - lo);
-        DeviceBatch& b = ctx->oneshot;
-        QB_TRY(build_batch(ctx, b, n, plan_ids + lo, nullptr, nullptr, 1, 0));
-        QB_TRY(batch_upload_params(ctx, b, params, param_offsets + lo));
-        QB_TRY(launch_circuits(ctx, b, nullptr));
+    return run_oneshot(ctx, batch, plan_ids, params, param_offsets, nullptr, chunk, [&](DeviceBatch& b, int lo) {
+        const int n = b.batch;
         const uint64_t size = uint64_t(1) << b.n_eff;
         const uint64_t n_chunks = size >> qb::kChunkBits;
         const size_t u_bytes = sizeof(double) * size_t(n) * size_t(shots);
@@ -1654,35 +1703,18 @@ int qb_sample(qb_context* ctx, int batch, const int64_t* plan_ids, const double*
         QB_TRY(ctx->pin_out.reserve(u_bytes));
         // uniforms in sorted (device) order
         double* stage = static_cast<double*>(ctx->pin_in.p);
-        for (int pos = 0; pos < n; ++pos)
-            std::memcpy(stage + size_t(pos) * shots, uniforms + size_t(lo + b.order[pos]) * shots, sizeof(double) * size_t(shots));
+        gather_rows(stage, uniforms + size_t(lo) * shots, b.order, sizeof(double) * size_t(shots));
         QB_CUDA(cudaMemcpyAsync(d_uniforms, stage, u_bytes, cudaMemcpyHostToDevice, ctx->stream));
-        dim3 cgrid(unsigned(std::min<uint64_t>((n_chunks + 7) / 8, 2048)), unsigned(n));
-        dim3 sgrid(unsigned((shots + 7) / 8), unsigned(n));
-        if (b.dtype == QB_C128) {
-            qb::chunk_prob_kernel<double><<<cgrid, 256, 0, ctx->stream>>>(b.states.as<double2>(), size, n_chunks, d_chunks);
-            QB_TRY(check_launch(ctx, "chunk_prob_kernel"));
-            qb::scan_chunks_kernel<<<n, 1024, 0, ctx->stream>>>(d_chunks, n_chunks);
-            QB_TRY(check_launch(ctx, "scan_chunks_kernel"));
-            qb::sample_kernel<double><<<sgrid, 256, 0, ctx->stream>>>(b.states.as<double2>(), size, d_chunks, n_chunks,
-                                                                       uint64_t(1) << b.n_qubits, d_uniforms, shots, d_indices);
-            QB_TRY(check_launch(ctx, "sample_kernel"));
-        } else {
-            qb::chunk_prob_kernel<float><<<cgrid, 256, 0, ctx->stream>>>(b.states.as<float2>(), size, n_chunks, d_chunks);
-            QB_TRY(check_launch(ctx, "chunk_prob_kernel"));
-            qb::scan_chunks_kernel<<<n, 1024, 0, ctx->stream>>>(d_chunks, n_chunks);
-            QB_TRY(check_launch(ctx, "scan_chunks_kernel"));
-            qb::sample_kernel<float><<<sgrid, 256, 0, ctx->stream>>>(b.states.as<float2>(), size, d_chunks, n_chunks,
-                                                                      uint64_t(1) << b.n_qubits, d_uniforms, shots, d_indices);
-            QB_TRY(check_launch(ctx, "sample_kernel"));
-        }
+        QB_TRY(with_dtype(b.dtype, [&](auto t) {
+            using T = decltype(t);
+            return launch_sampling_t<T>(ctx, b.states.as<typename qb::Cx<T>::type>(), size, n, uint64_t(1) << b.n_qubits, d_uniforms, shots, d_chunks,
+                                        d_indices);
+        }));
         QB_CUDA(cudaMemcpyAsync(ctx->pin_out.p, d_indices, u_bytes, cudaMemcpyDeviceToHost, ctx->stream));
         QB_CUDA(cudaStreamSynchronize(ctx->stream));
-        const int64_t* sorted = static_cast<const int64_t*>(ctx->pin_out.p);
-        for (int pos = 0; pos < n; ++pos)
-            std::memcpy(out_indices + size_t(lo + b.order[pos]) * shots, sorted + size_t(pos) * shots, sizeof(int64_t) * size_t(shots));
-    }
-    return QB_OK;
+        scatter_rows(out_indices + size_t(lo) * shots, ctx->pin_out.p, b.order, sizeof(int64_t) * size_t(shots));
+        return QB_OK;
+    });
 }
 
 int qb_evaluate_cvar(qb_context* ctx, int batch, const int64_t* plan_ids, const double* params, const int64_t* param_offsets,
@@ -1695,18 +1727,9 @@ int qb_evaluate_cvar(qb_context* ctx, int batch, const int64_t* plan_ids, const 
     Ham* ham = find_ham(ctx, ham_id);
     if (!ham) return fail(QB_ERR_NOT_FOUND, "unknown Hamiltonian id");
     if (!ham->diagonal) return fail(QB_ERR_INVALID, "CVaR needs a diagonal Hamiltonian; this one has non-diagonal terms");
-    Plan* first = find_plan(ctx, plan_ids[0]);
-    if (!first) return fail(QB_ERR_NOT_FOUND, "unknown plan id " + std::to_string(plan_ids[0]));
     // every chunk below is launched against order data of 2^first->n_eff entries: all plans must match it and the Hamiltonian
-    for (int i = 0; i < batch; ++i) {
-        const Plan* pl = find_plan(ctx, plan_ids[i]);
-        if (!pl) return fail(QB_ERR_NOT_FOUND, "unknown plan id " + std::to_string(plan_ids[i]));
-        if (pl->n_qubits != ham->n_qubits)
-            return fail(QB_ERR_INVALID, "Hamiltonian acts on " + std::to_string(ham->n_qubits) + " qubits, circuit " + std::to_string(i) +
-                                            " on " + std::to_string(pl->n_qubits));
-        if (pl->n_eff != first->n_eff || pl->dtype != first->dtype)
-            return fail(QB_ERR_INVALID, "all plans of one CVaR call must share state width and dtype");
-    }
+    const Plan* first = nullptr;
+    QB_TRY(check_plans(ctx, batch, plan_ids, ham->n_qubits, "Hamiltonian acts", "CVaR", &first));
     // alpha ~ 1 (numpy.isclose(alpha, 1)): the greedy fill in basis order, no sort (expectation.lower_tail_expectation_arrays)
     const bool sorted = std::fabs(alpha - 1.0) > 1e-8 + 1e-5;
     QB_TRY(ensure_cvar_order(ctx, *ham, first->n_eff, sorted));
@@ -1719,12 +1742,8 @@ int qb_evaluate_cvar(qb_context* ctx, int batch, const int64_t* plan_ids, const 
         return fail(QB_ERR_MEMORY, "CVaR data (" + std::to_string(kept) + " bytes) and one statevector (" + std::to_string(state_bytes) +
                                        " bytes) do not fit the workspace of " + std::to_string(limit) + " bytes");
     const int chunk = int(std::min<size_t>({size_t(batch), max_batch_for(ctx, first), (limit - kept) / state_bytes}));
-    for (int lo = 0; lo < batch; lo += chunk) {
-        const int n = std::min(chunk, batch - lo);
-        DeviceBatch& b = ctx->oneshot;
-        QB_TRY(build_batch(ctx, b, n, plan_ids + lo, nullptr, nullptr, 1, 0));
-        QB_TRY(batch_upload_params(ctx, b, params, param_offsets + lo));
-        QB_TRY(launch_circuits(ctx, b, nullptr));
+    return run_oneshot(ctx, batch, plan_ids, params, param_offsets, nullptr, chunk, [&](DeviceBatch& b, int lo) {
+        const int n = b.batch;
         const uint64_t size = uint64_t(1) << b.n_eff;
         const uint64_t n_chunks = size >> qb::kChunkBits;
         QB_TRY(ctx->scratch.reserve(sizeof(double) * (2 * size_t(n) * n_chunks + size_t(n))));
@@ -1733,29 +1752,22 @@ int qb_evaluate_cvar(qb_context* ctx, int batch, const int64_t* plan_ids, const 
         double* d_out = d_pe + size_t(n) * n_chunks;
         dim3 cgrid(unsigned(std::min<uint64_t>((n_chunks + 7) / 8, 2048)), unsigned(n));
         const unsigned fgrid = unsigned((n + 7) / 8);
-        if (b.dtype == QB_C128) {
-            qb::cvar_chunk_kernel<double><<<cgrid, 256, 0, ctx->stream>>>(b.states.as<double2>(), size, perm, energy, n_chunks, d_mass, d_pe);
+        QB_TRY(with_dtype(b.dtype, [&](auto t) {
+            using T = decltype(t);
+            using C = typename qb::Cx<T>::type;
+            qb::cvar_chunk_kernel<T><<<cgrid, 256, 0, ctx->stream>>>(b.states.as<C>(), size, perm, energy, n_chunks, d_mass, d_pe);
             QB_TRY(check_launch(ctx, "cvar_chunk_kernel"));
             qb::scan_chunks_kernel<<<2 * n, 1024, 0, ctx->stream>>>(d_mass, n_chunks);
             QB_TRY(check_launch(ctx, "scan_chunks_kernel"));
-            qb::cvar_finish_kernel<double><<<fgrid, 256, 0, ctx->stream>>>(b.states.as<double2>(), size, perm, energy, d_mass, d_pe, n_chunks,
-                                                                           alpha, n, d_out);
-        } else {
-            qb::cvar_chunk_kernel<float><<<cgrid, 256, 0, ctx->stream>>>(b.states.as<float2>(), size, perm, energy, n_chunks, d_mass, d_pe);
-            QB_TRY(check_launch(ctx, "cvar_chunk_kernel"));
-            qb::scan_chunks_kernel<<<2 * n, 1024, 0, ctx->stream>>>(d_mass, n_chunks);
-            QB_TRY(check_launch(ctx, "scan_chunks_kernel"));
-            qb::cvar_finish_kernel<float><<<fgrid, 256, 0, ctx->stream>>>(b.states.as<float2>(), size, perm, energy, d_mass, d_pe, n_chunks,
-                                                                          alpha, n, d_out);
-        }
-        QB_TRY(check_launch(ctx, "cvar_finish_kernel"));
+            qb::cvar_finish_kernel<T><<<fgrid, 256, 0, ctx->stream>>>(b.states.as<C>(), size, perm, energy, d_mass, d_pe, n_chunks, alpha, n, d_out);
+            return check_launch(ctx, "cvar_finish_kernel");
+        }));
         QB_TRY(ctx->pin_out.reserve(sizeof(double) * size_t(n)));
         QB_CUDA(cudaMemcpyAsync(ctx->pin_out.p, d_out, sizeof(double) * size_t(n), cudaMemcpyDeviceToHost, ctx->stream));
         QB_CUDA(cudaStreamSynchronize(ctx->stream));
-        const double* sorted_out = static_cast<const double*>(ctx->pin_out.p);
-        for (int pos = 0; pos < n; ++pos) out_values[lo + b.order[pos]] = sorted_out[pos];
-    }
-    return QB_OK;
+        scatter_rows(out_values + lo, ctx->pin_out.p, b.order, sizeof(double));
+        return QB_OK;
+    });
 }
 
 int qb_evaluate_observables(qb_context* ctx, int batch, const int64_t* plan_ids, const double* params, const int64_t* param_offsets,
@@ -1766,17 +1778,8 @@ int qb_evaluate_observables(qb_context* ctx, int batch, const int64_t* plan_ids,
     QB_ON_DEVICE(ctx);
     const Obs* ob = find_obs(ctx, obs_id);
     if (!ob) return fail(QB_ERR_NOT_FOUND, "unknown observable set id");
-    const Plan* first = find_plan(ctx, plan_ids[0]);
-    if (!first) return fail(QB_ERR_NOT_FOUND, "unknown plan id " + std::to_string(plan_ids[0]));
-    for (int i = 0; i < batch; ++i) {
-        const Plan* pl = find_plan(ctx, plan_ids[i]);
-        if (!pl) return fail(QB_ERR_NOT_FOUND, "unknown plan id " + std::to_string(plan_ids[i]));
-        if (pl->n_qubits != ob->n_qubits)
-            return fail(QB_ERR_INVALID, "observables act on " + std::to_string(ob->n_qubits) + " qubits, circuit " + std::to_string(i) + " on " +
-                                            std::to_string(pl->n_qubits));
-        if (pl->n_eff != first->n_eff || pl->dtype != first->dtype)
-            return fail(QB_ERR_INVALID, "all plans of one observables call must share state width and dtype");
-    }
+    const Plan* first = nullptr;
+    QB_TRY(check_plans(ctx, batch, plan_ids, ob->n_qubits, "observables act", "observables", &first));
     // per state: the statevector, its string values, its observable values and the partials of at least one string
     const uint64_t size = uint64_t(1) << first->n_eff;
     const uint64_t count = std::max<uint64_t>(size >> qb::kExpTileBits, std::min<uint64_t>(1024, std::max<uint64_t>(1, size / 256)));
@@ -1789,12 +1792,8 @@ int qb_evaluate_observables(qb_context* ctx, int batch, const int64_t* plan_ids,
                                        std::to_string(per_state - state_bytes) + " bytes) do not fit the workspace of " + std::to_string(limit) + " bytes");
     const int chunk = int(std::min<size_t>({size_t(batch), max_batch_for(ctx, first), limit / per_state}));
     const size_t n_out = size_t(ob->n_obs);
-    for (int lo = 0; lo < batch; lo += chunk) {
-        const int n = std::min(chunk, batch - lo);
-        DeviceBatch& b = ctx->oneshot;
-        QB_TRY(build_batch(ctx, b, n, plan_ids + lo, nullptr, nullptr, 1, 0));
-        QB_TRY(batch_upload_params(ctx, b, params, param_offsets + lo));
-        QB_TRY(launch_circuits(ctx, b, nullptr));
+    return run_oneshot(ctx, batch, plan_ids, params, param_offsets, nullptr, chunk, [&](DeviceBatch& b, int lo) {
+        const int n = b.batch;
         const size_t terms_bytes = sizeof(double) * size_t(n) * size_t(ob->n_terms), out_bytes = sizeof(double) * size_t(n) * n_out;
         const size_t room = limit - size_t(n) * state_bytes - terms_bytes - out_bytes;  // >= n * count * 8 by the chunk size
         const size_t partial_bytes = std::max(sizeof(double) * size_t(count) * size_t(n), std::min(kTermPartialBytes, room));
@@ -1802,19 +1801,16 @@ int qb_evaluate_observables(qb_context* ctx, int batch, const int64_t* plan_ids,
         double* d_terms = ctx->scratch.as<double>();
         double* d_out = d_terms + size_t(n) * size_t(ob->n_terms);
         double* d_partials = d_out + size_t(n) * n_out;
-        QB_TRY(b.dtype == QB_C128 ? launch_terms_t<double>(ctx, b, *ob, d_partials, partial_bytes, d_terms)
-                                  : launch_terms_t<float>(ctx, b, *ob, d_partials, partial_bytes, d_terms));
+        QB_TRY(with_dtype(b.dtype, [&](auto t) { return launch_terms_t<decltype(t)>(ctx, b, *ob, d_partials, partial_bytes, d_terms); }));
         qb::combine_observables_kernel<<<dim3(unsigned((n_out + 127) / 128), unsigned(n)), 128, 0, ctx->stream>>>(
             d_terms, ob->n_terms, ob->row_begin.as<int64_t>(), ob->cols.as<int32_t>(), ob->coeff.as<double>(), ob->n_obs, d_out);
         QB_TRY(check_launch(ctx, "combine_observables_kernel"));
         QB_TRY(ctx->pin_out.reserve(out_bytes));
         QB_CUDA(cudaMemcpyAsync(ctx->pin_out.p, d_out, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));
         QB_CUDA(cudaStreamSynchronize(ctx->stream));
-        const double* sorted = static_cast<const double*>(ctx->pin_out.p);
-        for (int pos = 0; pos < n; ++pos)
-            std::memcpy(out_values + size_t(lo + b.order[pos]) * n_out, sorted + size_t(pos) * n_out, sizeof(double) * n_out);
-    }
-    return QB_OK;
+        scatter_rows(out_values + size_t(lo) * n_out, ctx->pin_out.p, b.order, sizeof(double) * n_out);
+        return QB_OK;
+    });
 }
 
 int qb_statevector(qb_context* ctx, int64_t plan_id, const double* params, int n_params, double* out_re_im) {
@@ -1875,8 +1871,7 @@ int qb_expectation_device(qb_context* ctx, int64_t ham_id, int dtype, int n_loca
     QB_TRY(ctx->scratch.reserve(sizeof(double) * (n_part + 16)));
     double* d_part = ctx->scratch.as<double>();
     double* d_out = d_part + n_part;
-    if (dtype == QB_C128) QB_TRY(expectation_state_t<double>(ctx, *ham, d_state, n_local, index_offset, d_part, d_out));
-    else QB_TRY(expectation_state_t<float>(ctx, *ham, d_state, n_local, index_offset, d_part, d_out));
+    QB_TRY(with_dtype(dtype, [&](auto t) { return expectation_state_t<decltype(t)>(ctx, *ham, d_state, n_local, index_offset, d_part, d_out); }));
     QB_CUDA(cudaMemcpyAsync(out_value, d_out, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
     QB_CUDA(cudaStreamSynchronize(ctx->stream));
     return QB_OK;
@@ -1897,22 +1892,10 @@ int qb_sample_device(qb_context* ctx, int dtype, int n_local, const void* d_stat
     int64_t* d_indices = reinterpret_cast<int64_t*>(d_uniforms + shots);
     double* d_chunks = reinterpret_cast<double*>(d_indices + shots);
     QB_CUDA(cudaMemcpyAsync(d_uniforms, uniforms, u_bytes, cudaMemcpyHostToDevice, ctx->stream));
-    dim3 cgrid(unsigned(std::min<uint64_t>((n_chunks + 7) / 8, 2048)), 1);
-    dim3 sgrid(unsigned((shots + 7) / 8), 1);
-    if (dtype == QB_C128) {
-        qb::chunk_prob_kernel<double><<<cgrid, 256, 0, ctx->stream>>>(static_cast<const double2*>(d_state), size, n_chunks, d_chunks);
-        QB_TRY(check_launch(ctx, "chunk_prob_kernel"));
-        qb::scan_chunks_kernel<<<1, 1024, 0, ctx->stream>>>(d_chunks, n_chunks);
-        QB_TRY(check_launch(ctx, "scan_chunks_kernel"));
-        qb::sample_kernel<double><<<sgrid, 256, 0, ctx->stream>>>(static_cast<const double2*>(d_state), size, d_chunks, n_chunks, size, d_uniforms, shots, d_indices);
-    } else {
-        qb::chunk_prob_kernel<float><<<cgrid, 256, 0, ctx->stream>>>(static_cast<const float2*>(d_state), size, n_chunks, d_chunks);
-        QB_TRY(check_launch(ctx, "chunk_prob_kernel"));
-        qb::scan_chunks_kernel<<<1, 1024, 0, ctx->stream>>>(d_chunks, n_chunks);
-        QB_TRY(check_launch(ctx, "scan_chunks_kernel"));
-        qb::sample_kernel<float><<<sgrid, 256, 0, ctx->stream>>>(static_cast<const float2*>(d_state), size, d_chunks, n_chunks, size, d_uniforms, shots, d_indices);
-    }
-    QB_TRY(check_launch(ctx, "sample_kernel"));
+    QB_TRY(with_dtype(dtype, [&](auto t) {
+        using T = decltype(t);
+        return launch_sampling_t<T>(ctx, static_cast<const typename qb::Cx<T>::type*>(d_state), size, 1, size, d_uniforms, shots, d_chunks, d_indices);
+    }));
     QB_CUDA(cudaMemcpyAsync(out_indices, d_indices, u_bytes, cudaMemcpyDeviceToHost, ctx->stream));
     QB_CUDA(cudaStreamSynchronize(ctx->stream));
     return QB_OK;
@@ -1966,13 +1949,12 @@ int qb_cvar_select_device(qb_context* ctx, int64_t ham_id, int dtype, int n_loca
     const uint64_t* z = ham->diag_z.as<uint64_t>();
     const double* c = ham->diag_c.as<double>();
     double2* cache = static_cast<double2*>(d_cache);
-    if (dtype == QB_C128)
-        qb::cvar_select_kernel<double><<<n_cta, 32 * qb::kSelWarps, 0, ctx->stream>>>(static_cast<const double2*>(d_state), cache, cache_mode, size,
-                                                                                       index_offset, z, c, ham->n_diag, a, d_part, d_part + B * size_t(n_cta), d_ints);
-    else
-        qb::cvar_select_kernel<float><<<n_cta, 32 * qb::kSelWarps, 0, ctx->stream>>>(static_cast<const float2*>(d_state), cache, cache_mode, size,
-                                                                                      index_offset, z, c, ham->n_diag, a, d_part, d_part + B * size_t(n_cta), d_ints);
-    QB_TRY(check_launch(ctx, "cvar_select_kernel"));
+    QB_TRY(with_dtype(dtype, [&](auto t) {
+        using T = decltype(t);
+        qb::cvar_select_kernel<T><<<n_cta, 32 * qb::kSelWarps, 0, ctx->stream>>>(static_cast<const typename qb::Cx<T>::type*>(d_state), cache, cache_mode,
+                                                                                  size, index_offset, z, c, ham->n_diag, a, d_part, d_part + B * size_t(n_cta), d_ints);
+        return check_launch(ctx, "cvar_select_kernel");
+    }));
     qb::cvar_select_reduce_kernel<<<2 * B, 256, 0, ctx->stream>>>(d_part, n_cta, d_sums);
     QB_TRY(check_launch(ctx, "cvar_select_reduce_kernel"));
     QB_TRY(ctx->pin_out.reserve(sums_bytes + ints_bytes));
@@ -2007,9 +1989,11 @@ int qb_swap_global_p2p(qb_context* ctx, int dtype, int n_local, const void* d_st
     QB_ON_DEVICE(ctx);
     const uint64_t size = uint64_t(1) << n_local;
     const int blocks = int(std::min<uint64_t>(uint64_t(ctx->sm_count) * 8, std::max<uint64_t>(1, size / (256 * 4))));
-    if (dtype == QB_C128) qb::swap_p2p_kernel<double2><<<blocks, 256, 0, ctx->stream>>>(static_cast<const double2*>(d_state), args, size);
-    else qb::swap_p2p_kernel<float2><<<blocks, 256, 0, ctx->stream>>>(static_cast<const float2*>(d_state), args, size);
-    return check_launch(ctx, "swap_p2p_kernel");
+    return with_dtype(dtype, [&](auto t) {
+        using C = typename qb::Cx<decltype(t)>::type;
+        qb::swap_p2p_kernel<C><<<blocks, 256, 0, ctx->stream>>>(static_cast<const C*>(d_state), args, size);
+        return check_launch(ctx, "swap_p2p_kernel");
+    });
 }
 
 int qb_evaluate_expectation_submit(qb_context* ctx, int batch, const int64_t* plan_ids, const double* params, const int64_t* param_offsets,
@@ -2055,8 +2039,7 @@ int qb_evaluate_expectation_collect(qb_context* ctx, int total, double* out_valu
     if (e != cudaSuccess) return fail(QB_ERR_CUDA, std::string("cudaStreamSynchronize: ") + cudaGetErrorString(e));
     if (size_t(total) != have) return fail(QB_ERR_INVALID, "collect asked for " + std::to_string(total) + " results, " + std::to_string(have) + " are pending");
     const double* res = static_cast<const double*>(ctx->pin_res.p);
-    for (const auto& ch : chunks)
-        for (size_t pos = 0; pos < ch.order.size(); ++pos) out_values[ch.offset + size_t(ch.order[pos])] = res[ch.offset + pos];
+    for (const auto& ch : chunks) scatter_rows(out_values + ch.offset, res + ch.offset, ch.order, sizeof(double));
     return QB_OK;
 }
 
@@ -2103,7 +2086,7 @@ int qb_evaluate_expectation_multi(int n_ctx, qb_context* const* ctxs, const int*
 
 int qb_context_sm_count(qb_context* ctx) { return ctx ? ctx->sm_count : 0; }
 
-uint64_t qb_context_workspace(qb_context* ctx) { return ctx ? (ctx->workspace_limit ? ctx->workspace_limit : ctx->default_workspace) : 0; }
+uint64_t qb_context_workspace(qb_context* ctx) { return ctx ? workspace_limit_of(ctx) : 0; }
 
 // ---- device memory / peer mapping for sharded states --------------------------------------------------
 int qb_device_alloc(qb_context* ctx, uint64_t bytes, void** out_ptr) {

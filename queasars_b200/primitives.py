@@ -433,8 +433,41 @@ class _B200Primitive:
             return self._queue.submit(key, payload)
         return self._execute(key, [payload])[0]
 
-    def _execute(self, key, payloads):  # pragma: no cover - overridden
+    def _execute(self, key, payloads):
+        """Evaluate the payloads (target, circuits, parameter vectors) coalesced under ``key`` as one list: circuit after circuit on
+        one statevector sharded over the device set when they are too wide for one GPU, otherwise split over the devices.  Returns
+        every payload's rows, stacked, in its own order."""
+        circuits, values, sizes = [], [], []
+        for _, circs, vals in payloads:
+            sizes.append(len(circs))
+            circuits.extend(circs)
+            values.extend(vals)
+        width, on_state, on_devices, stack = self._parts(key, payloads[0][0])
+        if self._needs_sharding(width):
+            flat = []
+            with self._shard_lock:
+                sv = self._sharded_state(width)
+                for circuit, vals in zip(circuits, values):
+                    gates, bound = self._bound_gates(circuit, vals)
+                    sv.reset()
+                    sv.run(gates, bound)
+                    flat.append(on_state(sv))
+        else:
+            flat = on_devices(circuits, values)
+        out, pos = [], 0
+        for n in sizes:
+            out.append(stack(flat[pos : pos + n]))
+            pos += n
+        return out
+
+    def _parts(self, key, target):  # pragma: no cover - overridden
+        """What ``_execute`` needs of one kind of submission: (qubit count, ``on_state(sv)`` -> the row of the sharded state just run,
+        ``on_devices(circuits, values)`` -> their rows in submission order, ``stack(rows)`` -> one payload's result)."""
         raise NotImplementedError
+
+
+def _float_rows(rows) -> np.ndarray:
+    return np.asarray(rows, dtype=np.float64)
 
 
 def _param_rows(values) -> tuple[np.ndarray, tuple]:
@@ -501,69 +534,26 @@ class B200EstimatorV2(_B200Primitive):
         key = ("many", tuple(id(op) for op in observables), fps)
         return np.asarray(self._submit(key, (observables, circuits, parameter_values)), dtype=np.float64).reshape(len(circuits), len(observables))
 
-    def _execute_many(self, key, payloads):
-        observables = payloads[0][0]
-        fps = key[2]
-        circuits, values, sizes = [], [], []
-        for _, circs, vals in payloads:
-            sizes.append(len(circs))
-            circuits.extend(circs)
-            values.extend(vals)
-        width = int(observables[0].num_qubits)
-        if self._needs_sharding(width):
-            # one statevector over the whole device set per row, every observable evaluated on it (sharded.py)
-            flat = []
-            with self._shard_lock:
-                sv = self._sharded_state(width)
-                for circuit, vals in zip(circuits, values):
-                    gates, bound = self._bound_gates(circuit, vals)
-                    sv.reset()
-                    sv.run(gates, bound)
-                    flat.append(np.asarray([sv.expectation(op) for op in observables], dtype=np.float64))
-        else:
-            diagonal = self.observables_for(observables, fingerprints=fps).diagonal
-            resolved = self._resolve_all(circuits, values, probabilities_only=diagonal)
-            flat = self._run_per_device(
-                resolved, lambda slot, plans, params: list(self.engines[slot].expectation_many(plans, params, self.observables_for(observables, slot, fps)))
-            )
-        out, pos = [], 0
-        for n in sizes:
-            out.append(np.asarray(flat[pos : pos + n], dtype=np.float64).reshape(n, len(observables)))
-            pos += n
-        return out
+    def _parts(self, key, target):
+        if key[0] == "many":  # target: the observables, every one evaluated on each state
+            observables, fps = target, key[2]
 
-    def _execute(self, key, payloads):
-        if key[0] == "many":
-            return self._execute_many(key, payloads)
-        operator = payloads[0][0]
-        circuits, values, sizes = [], [], []
-        for _, circs, vals in payloads:
-            sizes.append(len(circs))
-            circuits.extend(circs)
-            values.extend(vals)
-        if self._needs_sharding(int(operator.num_qubits)):
-            # one statevector over the whole device set, circuit after circuit (sharded.py): same values, no batch
-            flat = []
-            with self._shard_lock:
-                sv = self._sharded_state(int(operator.num_qubits))
-                for circuit, vals in zip(circuits, values):
-                    gates, bound = self._bound_gates(circuit, vals)
-                    sv.reset()
-                    sv.run(gates, bound)
-                    flat.append(sv.expectation(operator))
-            out, pos = [], 0
-            for n in sizes:
-                out.append(np.asarray(flat[pos : pos + n], dtype=np.float64))
-                pos += n
-            return out
-        fp = key[2]
-        resolved = self._resolve_all(circuits, values, probabilities_only=self.hamiltonian_for(operator, fingerprint=fp).diagonal)
-        flat = self._expectation_on_devices(resolved, operator, fp)
-        out, pos = [], 0
-        for n in sizes:
-            out.append(np.asarray(flat[pos : pos + n], dtype=np.float64))
-            pos += n
-        return out
+            def many_on_devices(circuits, values):
+                diagonal = self.observables_for(observables, fingerprints=fps).diagonal
+                resolved = self._resolve_all(circuits, values, probabilities_only=diagonal)
+                return self._run_per_device(
+                    resolved, lambda slot, plans, params: list(self.engines[slot].expectation_many(plans, params, self.observables_for(observables, slot, fps)))
+                )
+
+            return (int(observables[0].num_qubits), lambda sv: np.asarray([sv.expectation(op) for op in observables], dtype=np.float64), many_on_devices,
+                    lambda rows: np.asarray(rows, dtype=np.float64).reshape(len(rows), len(observables)))
+        operator, fp = target, key[2]
+
+        def on_devices(circuits, values):
+            resolved = self._resolve_all(circuits, values, probabilities_only=self.hamiltonian_for(operator, fingerprint=fp).diagonal)
+            return self._expectation_on_devices(resolved, operator, fp)
+
+        return int(operator.num_qubits), lambda sv: sv.expectation(operator), on_devices, _float_rows
 
     def _expectation_on_devices(self, resolved, operator, fp) -> list:
         """<H> of every resolved (slot, plan, values) entry, in submission order.  One device: one blocking native call.  Several
@@ -759,7 +749,7 @@ class B200SamplerV2(_B200Primitive):
         widths = {_width(c) for c in circuits}
         if len(widths) != 1:
             raise ValueError("all circuits of one sampler submission must act on the same number of qubits")
-        return np.asarray(self._submit(("smp", int(shots), widths.pop()), (circuits, parameter_values)))
+        return np.asarray(self._submit(("smp", int(shots), widths.pop()), (None, circuits, parameter_values)))
 
     def cvar_values(self, circuits, parameter_values, operator, alpha: float) -> np.ndarray:
         """Exact (shot-free) CVaR(alpha) of the diagonal ``operator`` on every circuit's full distribution |psi|^2:
@@ -797,84 +787,49 @@ class B200SamplerV2(_B200Primitive):
             )
         return np.asarray(self._submit((kind, id(operator), fp, alpha, width), (operator, circuits, parameter_values)), dtype=np.float64)
 
-    def _execute_exact(self, key, payloads):
-        kind, _, fp, alpha, width = key
-        operator = payloads[0][0]
-        circuits, values, sizes = [], [], []
-        for _, circs, vals in payloads:
-            sizes.append(len(circs))
-            circuits.extend(circs)
-            values.extend(vals)
-        if self._needs_sharding(width):
-            # one statevector over the whole device set, circuit after circuit (sharded.py): the select passes of
-            # _ShardedLogic.cvar, or <H> for alpha ~ 1 on the operator evaluator; the duplicate-merged terms of the device Hamiltonian
-            ham = self.hamiltonian_for(operator, build_table=False, fingerprint=fp)
-            flat = []
-            with self._shard_lock:
-                sv = self._sharded_state(width)
-                for circuit, vals in zip(circuits, values):
-                    gates, bound = self._bound_gates(circuit, vals)
-                    sv.reset()
-                    sv.run(gates, bound)
-                    flat.append(sv.cvar(ham.z_masks, ham.coeffs, alpha)[0] if kind == "cvar" else sv.diagonal_expectation(ham.z_masks, ham.coeffs))
-        else:
-            resolved = self._resolve_all(circuits, values, probabilities_only=True)
+    def _parts(self, key, target):
+        if key[0] == "smp":
+            _, shots, width = key
 
+            def sample_on_state(sv):
+                rng = self.seed if isinstance(self.seed, np.random.Generator) else np.random.default_rng(self.seed)
+                return sv.sample(shots, uniforms=rng.random(shots))
+
+            def sample_on_devices(circuits, values):
+                resolved = self._resolve_all(circuits, values, probabilities_only=True)
+                # a fresh default_rng(seed) per pub when seed is an int (or None); a shared Generator is consumed in submission order
+                if isinstance(self.seed, np.random.Generator):
+                    uniforms = np.stack([self.seed.random(shots) for _ in resolved])
+                else:
+                    one = np.random.default_rng(self.seed).random(shots) if self.seed is not None else None
+                    uniforms = np.stack([one if one is not None else np.random.default_rng().random(shots) for _ in resolved])
+                rows_of: dict = {}
+                for i, (slot, _, _) in enumerate(resolved):
+                    rows_of.setdefault(slot, []).append(i)
+                return self._run_per_device(
+                    resolved, lambda slot, plans, params: list(self.engines[slot].sample(plans, params, shots, uniforms[rows_of[slot]]))
+                )
+
+            return width, sample_on_state, sample_on_devices, np.stack
+        kind, _, fp, alpha, width = key
+        operator = target
+
+        def on_state(sv):
+            # the select passes of _ShardedLogic.cvar, or <H> for alpha ~ 1 on the operator evaluator; the duplicate-merged terms of
+            # the device Hamiltonian
+            ham = self.hamiltonian_for(operator, build_table=False, fingerprint=fp)
+            return sv.cvar(ham.z_masks, ham.coeffs, alpha)[0] if kind == "cvar" else sv.diagonal_expectation(ham.z_masks, ham.coeffs)
+
+        def on_devices(circuits, values):
             def call(slot, plans, params):
                 engine = self.engines[slot]
                 if kind == "cvar":
                     return list(engine.cvar(plans, params, self.hamiltonian_for(operator, build_table=False, slot=slot, fingerprint=fp), alpha))
                 return list(engine.expectation(plans, params, self.hamiltonian_for(operator, slot=slot, fingerprint=fp)))
 
-            flat = self._run_per_device(resolved, call)
-        out, pos = [], 0
-        for n in sizes:
-            out.append(np.asarray(flat[pos : pos + n], dtype=np.float64))
-            pos += n
-        return out
+            return self._run_per_device(self._resolve_all(circuits, values, probabilities_only=True), call)
 
-    def _execute(self, key, payloads):
-        if key[0] in ("cvar", "exp"):
-            return self._execute_exact(key, payloads)
-        shots = key[1]
-        circuits, values, sizes = [], [], []
-        for circs, vals in payloads:
-            sizes.append(len(circs))
-            circuits.extend(circs)
-            values.extend(vals)
-        if self._needs_sharding(key[2]):
-            rows = []
-            with self._shard_lock:
-                sv = self._sharded_state(key[2])
-                for circuit, vals in zip(circuits, values):
-                    gates, bound = self._bound_gates(circuit, vals)
-                    sv.reset()
-                    sv.run(gates, bound)
-                    rng = self.seed if isinstance(self.seed, np.random.Generator) else np.random.default_rng(self.seed)
-                    rows.append(sv.sample(shots, uniforms=rng.random(shots)))
-            out, pos = [], 0
-            for n in sizes:
-                out.append(np.stack(rows[pos : pos + n]))
-                pos += n
-            return out
-        resolved = self._resolve_all(circuits, values, probabilities_only=True)
-        # a fresh default_rng(seed) per pub when seed is an int (or None); a shared Generator is consumed in submission order
-        if isinstance(self.seed, np.random.Generator):
-            uniforms = np.stack([self.seed.random(shots) for _ in resolved])
-        else:
-            one = np.random.default_rng(self.seed).random(shots) if self.seed is not None else None
-            uniforms = np.stack([one if one is not None else np.random.default_rng().random(shots) for _ in resolved])
-        rows_of: dict = {}
-        for i, (slot, _, _) in enumerate(resolved):
-            rows_of.setdefault(slot, []).append(i)
-        flat = self._run_per_device(
-            resolved, lambda slot, plans, params: list(self.engines[slot].sample(plans, params, shots, uniforms[rows_of[slot]]))
-        )
-        out, pos = [], 0
-        for n in sizes:
-            out.append(np.stack(flat[pos : pos + n]))
-            pos += n
-        return out
+        return width, on_state, on_devices, _float_rows
 
     def run(self, pubs: Iterable, *, shots: Optional[int] = None):
         try:

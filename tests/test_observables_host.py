@@ -238,7 +238,7 @@ def test_coalescing_key(fake_engines):
     for key, _ in keys:
         assert key[0] == "many" and key[1] in ids  # payloads of one call always share a set
     assert sum(count for _, count in keys) == len(cases)
-    assert est._execute_many(("many", keys[0][0][1], keys[0][0][2]), [(set_a, [cases[0][2]], [cases[0][1]])])[0].shape == (1, 3)
+    assert est._execute(("many", keys[0][0][1], keys[0][0][2]), [(set_a, [cases[0][2]], [cases[0][1]])])[0].shape == (1, 3)
     # an in-place edit of a coefficient changes the key and rebuilds the device form
     before = est.observables_for(set_a)
     set_a[0]._c[0] = 2.0
@@ -279,6 +279,60 @@ def test_sharded_route(fake_engines, monkeypatch):
     for row, (instr, values, _) in zip(got, cases):
         assert row == pytest.approx(oracle_evs(instr, values, n, ops), rel=1e-12, abs=1e-12)
     assert not calls(fake_engines, "many")
+
+
+class _ShardedOracle:
+    """Stand-in for ``LocalShardedStatevector``: the oracle's statevector of the last run."""
+
+    def reset(self):
+        self.st = None
+
+    def run(self, gates, params):
+        self.st = _state(gates, params)
+
+    def expectation(self, op):
+        return oq.estimator_expectation(self.st, op.to_list())
+
+    def sample(self, shots, uniforms):
+        return oq.sample_indices(self.st, shots, uniforms=uniforms)
+
+
+def test_sharded_single_operator_route(fake_engines, monkeypatch):
+    n = 4
+    est = pr.B200EstimatorV2(shard_min_qubits=n)
+    op = SparsePauliOp.from_list([(l, 0.5 + k) for k, l in enumerate(labels(n, 11, 4))])
+    cases = [case(n, 2, 90 + s) for s in range(3)]
+    monkeypatch.setattr(est, "_sharded_state", lambda width: _ShardedOracle())
+    got = est.expectation_values([c for _, _, c in cases], [v for _, v, _ in cases], op)
+    assert got.shape == (3,)
+    for ev, (instr, values, _) in zip(got, cases):
+        assert ev == pytest.approx(oracle_evs(instr, values, n, [op])[0], rel=1e-12, abs=1e-12)
+    res = est.run([(cases[0][2], op, [cases[0][1], cases[0][1]])]).result()[0]
+    assert res.data.evs.shape == (2,) and res.data.evs[1] == pytest.approx(got[0], rel=1e-12, abs=1e-12)
+    assert not calls(fake_engines, "expectation") and not calls(fake_engines, "many")
+
+
+def test_sharded_sampler_shots(fake_engines, monkeypatch):
+    n, shots = 4, 96
+    cases = [case(n, 2, 100 + s) for s in range(3)]
+    circuits, values = [c for _, _, c in cases], [v for _, v, _ in cases]
+    states = [oq.statevector(instr, n, v) for instr, v, _ in cases]
+    # an int seed: a fresh generator per circuit, every row drawn from the same uniforms
+    smp = pr.B200SamplerV2(seed=9, shard_min_qubits=n)
+    monkeypatch.setattr(smp, "_sharded_state", lambda width: _ShardedOracle())
+    got = smp.sample_indices(circuits, values, shots)
+    uniforms = np.random.default_rng(9).random(shots)
+    assert got.shape == (3, shots) and got.dtype == np.int64
+    for row, st in zip(got, states):
+        assert row.tolist() == oq.sample_indices(st, shots, uniforms=uniforms).tolist()
+    # a Generator seed: consumed row after row in submission order
+    smp = pr.B200SamplerV2(seed=np.random.default_rng(9), shard_min_qubits=n)
+    monkeypatch.setattr(smp, "_sharded_state", lambda width: _ShardedOracle())
+    got = smp.sample_indices(circuits, values, shots)
+    gen = np.random.default_rng(9)
+    for row, st in zip(got, states):
+        assert row.tolist() == oq.sample_indices(st, shots, uniforms=gen.random(shots)).tolist()
+    assert not any(e.calls for e in fake_engines.values())
 
 
 @pytest.mark.parametrize("shape", [(3,), (2, 2)])
