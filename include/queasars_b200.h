@@ -178,7 +178,8 @@ int qb_statevector(qb_context* ctx, int64_t plan_id, const double* params, int n
  * states, E(k) = sum_t c_t (-1)^{popcount(k & z_t)} -- the lower alpha tail of |psi_i|^2 in stable ascending (E(k), k) order,
  * greedy fill stopped once the mass is numpy.isclose to alpha, divided by alpha.  With alpha isclose to 1 the fill runs in basis
  * order (no sort), as in that function.  The Hamiltonian must be diagonal (QB_ERR_INVALID otherwise, and for alpha outside
- * (0, 1], and when a plan's width or dtype differs from the first plan's or the Hamiltonian's).  Its data is built on first use
+ * (0, 1], when a plan's width or dtype differs from the first plan's or the Hamiltonian's, and for alpha < 1 on more than 32
+ * qubits: the sorted order stores 32-bit basis indices).  Its data is built on first use
  * and kept until the Hamiltonian is destroyed: E in basis order (8 B per amplitude), and for alpha < 1 the sorted order and E
  * sorted (12 B more); QB_ERR_MEMORY when it does not fit the workspace.  Deterministic: bit-identical across runs and
  * independent of the other entries of the batch. */

@@ -871,6 +871,10 @@ int fill_diag_table(qb_context* ctx, const Ham& ham, double* table, int n_eff) {
 // stable and treats -0.0 == +0.0, which is numpy.argsort(kind="stable") on float64.  The sort needs the input indices and CUB's
 // sort storage for a moment.
 int ensure_cvar_order(qb_context* ctx, Ham& ham, int n_eff, bool sorted) {
+    // perm holds basis indices as uint32: above 2^32 entries they would wrap, whatever the workspace holds
+    if (sorted && n_eff > 32)
+        return fail(QB_ERR_INVALID, "the sorted CVaR order of a " + std::to_string(n_eff) +
+                                        "-qubit state needs basis indices wider than 32 bits; only alpha close to 1 (basis order) is supported above 32 qubits");
     const uint64_t size = uint64_t(1) << n_eff;
     const size_t limit = workspace_limit_of(ctx);
     if (ham.cvar_energy_n_eff != n_eff) {
