@@ -186,6 +186,50 @@ int qb_statevector(qb_context* ctx, int64_t plan_id, const double* params, int n
 int qb_evaluate_cvar(qb_context* ctx, int batch, const int64_t* plan_ids, const double* params,
                      const int64_t* param_offsets, int64_t ham_id, double alpha, double* out_values);
 
+/* --- most probable basis states ---------------------------------------------------------------------------
+ * For a state psi of n qubits let p_k = re(psi_k)^2 + im(psi_k)^2, in double (complex64 components converted first) and rounded
+ * without FMA contraction.  The top states are the entries with p_k > 0 and p_k >= min_probability, in descending p, ties in
+ * ascending logical basis index, cut after max_states entries (a cut inside a run of ties keeps its lowest indices).  They are
+ * found without sorting the state: the composite key (~bits(p_k), logical k) -- ascending = that order -- is fixed 8 bits per
+ * pass by a counts-only histogram of the entries matching the prefix fixed so far, until the cut falls on a bucket boundary or
+ * the key is complete; one more pass pair then writes every entry up to that stop key.  Bit-identical across runs, batch
+ * compositions, devices and shard counts: only integer counts are reduced.
+ *
+ * qb_top_select is the state of one such select, shared by the one-GPU call and the sharded drivers.  qb_top_select_init starts
+ * it (QB_ERR_INVALID unless 1 <= n_qubits <= 63 and 1 <= max_states <= 2^20); qb_top_select_pick takes the 256 bucket counts of
+ * the pass the state describes (summed over all shards) and picks the bucket: the one decision rule of every route.  Pure host
+ * functions.  A pass histograms digit bits [p_free - 8, p_free) of the probability key while p_free > 0 (entries whose key >>
+ * p_free equals p_prefix), then logical index bits [max(0, idx_hi - 8), idx_hi) of the entries whose key equals p_prefix and
+ * whose logical bits >= idx_hi equal those of idx_prefix.  Once `done`, every eligible entry with (key, logical k) <=
+ * (stop_key, stop_index) is a top state, `selected` of them (= min(max_states, eligible entries)). */
+typedef struct qb_top_select {
+    uint64_t max_states;
+    uint64_t need;        /* entries still to take inside the current prefix range */
+    uint64_t taken;       /* entries below the current prefix range (all taken) */
+    uint64_t p_prefix;    /* fixed high bits of the probability key; its low p_free bits are open */
+    uint64_t idx_prefix;  /* fixed logical index bits (those >= idx_hi) */
+    uint64_t stop_key, stop_index;
+    uint64_t selected;
+    int32_t n_qubits;
+    int32_t p_free;       /* 64, 56, ..., 0 */
+    int32_t idx_hi;
+    int32_t done;
+    int32_t passes;       /* passes picked so far */
+    int32_t reserved;
+} qb_top_select;
+int qb_top_select_init(qb_top_select* sel, int n_qubits, int64_t max_states);
+int qb_top_select_pick(qb_top_select* sel, const uint64_t counts[256]);
+
+/* The top states of every circuit of a batch (entry i: plan_ids[i] with params[param_offsets[i] ..]).  out_counts[i] = number
+ * found; out_indices[i * max_states + j] (int64 logical basis index) and out_probs[i * max_states + j] (float64 p) for j <
+ * out_counts[i] in the order above; the rest of each row is -1 / 0.  All states of a chunk go through each select pass together;
+ * on one GPU physical and logical indices agree, and the collected entries are put in order by a stable device radix sort by
+ * descending p.  QB_ERR_INVALID for max_states outside [1, 2^20], a negative or non-finite min_probability, or plans that differ
+ * from the first in width or dtype; QB_ERR_MEMORY when one statevector and its max_states * 16 B of output do not fit the
+ * workspace. */
+int qb_top_states(qb_context* ctx, int batch, const int64_t* plan_ids, const double* params, const int64_t* param_offsets,
+                  int64_t max_states, double min_probability, int64_t* out_counts, int64_t* out_indices, double* out_probs);
+
 /* --- observable sets ------------------------------------------------------------------------------------
  * Several observables H_j = sum_t c_{j,t} P_t evaluated on one simulated state (EstimatorV2 pubs with an array of observables).
  * Observable j owns the terms term_offsets[j] .. term_offsets[j+1]-1 of the mask / coefficient arrays (term_offsets[0] == 0).
@@ -276,6 +320,17 @@ int qb_cvar_select_device(qb_context* ctx, int64_t ham_id, int dtype, int n_loca
                           void* d_cache, int cache_mode, uint64_t e_prefix, int e_free, int digit_kind, int digit_bits,
                           const int32_t* digit_positions, uint64_t idx_mask, uint64_t idx_value, double* out_sums,
                           uint64_t* out_ints);
+/* The top states of a sharded state (queasars_b200/sharded.py), on a caller-owned shard of 2^n_local amplitudes whose physical
+ * indices are `index_offset | k`; positions[q] = physical bit position of logical qubit q (sel->n_qubits entries; null: the
+ * identity).  qb_top_select_device runs the pass `sel` describes: out_counts[b] = entries of this shard in bucket b (sum them
+ * over the shards in any order, then qb_top_select_pick).  qb_top_collect_device, once `sel` is done, writes this shard's
+ * entries up to the stop key in physical index order: *out_count of them, out_indices = physical indices, out_probs = p;
+ * QB_ERR_INVALID when more than `capacity` are found.  Synchronous. */
+int qb_top_select_device(qb_context* ctx, int dtype, int n_local, const void* d_state, uint64_t index_offset, double min_probability,
+                         const qb_top_select* sel, const int32_t* positions, uint64_t* out_counts /* 256 */);
+int qb_top_collect_device(qb_context* ctx, int dtype, int n_local, const void* d_state, uint64_t index_offset, double min_probability,
+                          const qb_top_select* sel, const int32_t* positions, int64_t capacity, int64_t* out_count, int64_t* out_indices,
+                          double* out_probs);
 
 /* Global <-> local qubit swap of a state sharded over `world` = 2^n_global GPUs of one node (BASELINE config C5), fused with its
  * all-to-all: the calling rank streams its shard `d_state` once and stores every amplitude directly into the rank that owns it

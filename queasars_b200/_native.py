@@ -26,6 +26,14 @@ class QbError(RuntimeError):
         self.code = code
 
 
+class TopSelect(ctypes.Structure):
+    """``qb_top_select`` (include/queasars_b200.h): the state of one top-states select, advanced by ``qb_top_select_pick``."""
+
+    _fields_ = [("max_states", c_uint64), ("need", c_uint64), ("taken", c_uint64), ("p_prefix", c_uint64), ("idx_prefix", c_uint64),
+                ("stop_key", c_uint64), ("stop_index", c_uint64), ("selected", c_uint64), ("n_qubits", c_int32), ("p_free", c_int32),
+                ("idx_hi", c_int32), ("done", c_int32), ("passes", c_int32), ("reserved", c_int32)]
+
+
 _lib = None
 
 
@@ -77,6 +85,12 @@ def _declare(lib):
         "qb_ipc_export": [c_void_p, c_void_p, c_void_p],
         "qb_ipc_open": [c_void_p, c_void_p, P(c_void_p)],
         "qb_ipc_close": [c_void_p, c_void_p],
+        "qb_top_select_init": [P(TopSelect), c_int, c_int64],
+        "qb_top_select_pick": [P(TopSelect), c_void_p],
+        "qb_top_states": [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int64, c_double, c_void_p, c_void_p, c_void_p],
+        "qb_top_select_device": [c_void_p, c_int, c_int, c_void_p, c_uint64, c_double, P(TopSelect), c_void_p, c_void_p],
+        "qb_top_collect_device": [c_void_p, c_int, c_int, c_void_p, c_uint64, c_double, P(TopSelect), c_void_p, c_int64, P(c_int64), c_void_p,
+                                  c_void_p],
     }
     for name, argtypes in sigs.items():
         fn = getattr(lib, name)
@@ -101,7 +115,8 @@ EXPORTED_SYMBOLS = (
     "qb_evaluate_expectation_multi qb_evaluate_expectation_submit qb_evaluate_expectation_collect qb_context_sm_count "
     "qb_batch_create qb_batch_set_params qb_batch_run qb_batch_run_timed qb_batch_read qb_batch_destroy qb_batch_stats "
     "qb_apply_plan_device qb_expectation_device qb_sample_device qb_cvar_select_device qb_swap_global_p2p qb_record_sizes "
-    "qb_device_alloc qb_device_free qb_device_read qb_enable_peer_access qb_ipc_export qb_ipc_open qb_ipc_close"
+    "qb_device_alloc qb_device_free qb_device_read qb_enable_peer_access qb_ipc_export qb_ipc_open qb_ipc_close "
+    "qb_top_select_init qb_top_select_pick qb_top_states qb_top_select_device qb_top_collect_device"
 ).split()
 
 

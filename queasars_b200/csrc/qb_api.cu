@@ -1072,6 +1072,146 @@ int run_oneshot(qb_context* ctx, int batch, const int64_t* plan_ids, const doubl
     return QB_OK;
 }
 
+// f(uint32_t()) where the sweep kernels use 32-bit amplitude indices (up to 31 qubits, unless forced wide), f(uint64_t()) above
+template <typename F> int with_index_width(const qb_context* ctx, int n_bits, F&& f) {
+    return n_bits <= 31 && !ctx->force_idx64 ? f(uint32_t()) : f(uint64_t());
+}
+
+// ---- top states: validation, pass arguments, grids ----
+constexpr int64_t kTopMaxStates = int64_t(1) << 20;
+static_assert(sizeof(qb_top_select) == 88, "qb_top_select is mirrored by _native.TopSelect");
+
+int check_top_limits(int64_t max_states, double min_probability) {
+    if (max_states < 1 || max_states > kTopMaxStates) return fail(QB_ERR_INVALID, "max_states must be in 1..2^20, got " + std::to_string(max_states));
+    if (!std::isfinite(min_probability) || min_probability < 0.0) return fail(QB_ERR_INVALID, "min_probability must be finite and >= 0");
+    return QB_OK;
+}
+
+// a select state as qb_top_select_init / _pick leave it, and a bit map of distinct positions below 64 (null: the identity)
+int check_top_state(const qb_top_select* s, const int32_t* positions, bool want_done) {
+    if (!s) return fail(QB_ERR_INVALID, "null select state");
+    if (s->n_qubits < 1 || s->n_qubits > 63 || s->p_free < 0 || s->p_free > 64 || s->p_free % qb::kSelBits || s->idx_hi < 0 ||
+        s->idx_hi > s->n_qubits || (s->p_free && s->idx_hi != s->n_qubits))
+        return fail(QB_ERR_INVALID, "malformed select state");
+    if (bool(s->done) != want_done) return fail(QB_ERR_INVALID, want_done ? "the select is not done yet" : "the select is already done");
+    if (positions) {
+        uint64_t seen = 0;
+        for (int q = 0; q < s->n_qubits; ++q) {
+            const int p = positions[q];
+            if (p < 0 || p > 63 || ((seen >> p) & 1)) return fail(QB_ERR_INVALID, "bad bit map: positions must be distinct and below 64");
+            seen |= uint64_t(1) << p;
+        }
+    }
+    return QB_OK;
+}
+
+int top_position(const int32_t* positions, int q) { return positions ? positions[q] : q; }
+
+qb::TopSelectArgs top_select_args(const qb_top_select& s, const int32_t* positions, double min_probability, int entry) {
+    qb::TopSelectArgs t{};
+    qb::SelectArgs& a = t.sel;
+    a.e_prefix = s.p_prefix, a.e_free = s.p_free;
+    if (s.p_free > 0) {
+        a.digit_kind = 0, a.bits = qb::kSelBits;
+    } else {  // the probability key is fixed: logical index bits [lo, idx_hi), read at their physical positions
+        const int lo = std::max(0, s.idx_hi - qb::kSelBits);
+        a.digit_kind = 1, a.bits = s.idx_hi - lo;
+        for (int j = 0; j < a.bits; ++j) a.pos[j] = top_position(positions, lo + j);
+        for (int q = s.idx_hi; q < s.n_qubits; ++q) {
+            a.idx_mask |= uint64_t(1) << top_position(positions, q);
+            a.idx_value |= ((s.idx_prefix >> q) & 1) << top_position(positions, q);
+        }
+    }
+    t.min_probability = min_probability, t.entry = entry;
+    return t;
+}
+
+qb::TopCollectArgs top_collect_args(const qb_top_select& s, const int32_t* positions, double min_probability, int entry) {
+    qb::TopCollectArgs a{};
+    a.stop_key = s.stop_key, a.stop_index = s.stop_index, a.min_probability = min_probability, a.entry = entry;
+    if (positions) {
+        a.n_pos = s.n_qubits;
+        for (int q = 0; q < s.n_qubits; ++q) a.pos[q] = int8_t(positions[q]);
+    }
+    return a;
+}
+
+// select grid: one wave of resident CTAs, fewer for small states (fixed by the device and the state size)
+unsigned top_select_ctas(const qb_context* ctx, uint64_t size) {
+    return unsigned(std::min<uint64_t>(uint64_t(ctx->sm_count) * 8, std::max<uint64_t>(1, size / (32 * qb::kSelWarps * qb::kTopUnroll * 4))));
+}
+
+// collect grid: contiguous segments of whole kTopTile steps, about four waves
+unsigned top_collect_ctas(const qb_context* ctx, uint64_t size, uint64_t* seg) {
+    const uint64_t want = std::min<uint64_t>(uint64_t(ctx->sm_count) * 32, std::max<uint64_t>(1, size / qb::kTopTile));
+    *seg = ((size + want - 1) / want + qb::kTopTile - 1) / qb::kTopTile * qb::kTopTile;
+    return unsigned((size + *seg - 1) / *seg);
+}
+
+// one select pass over `m` states (rows `stride` amplitudes apart): d_counts[r][b] for args[r]; copied to host_counts
+template <typename T>
+int top_select_pass_t(qb_context* ctx, const void* states, uint64_t stride, uint64_t size, int n_bits, uint64_t index_offset,
+                      const qb::TopSelectArgs* host_args, int m, qb::TopSelectArgs* d_args, unsigned long long* d_counts, uint64_t* host_counts) {
+    using C = typename qb::Cx<T>::type;
+    const size_t count_bytes = sizeof(uint64_t) * qb::kSelBuckets * size_t(m);
+    QB_CUDA(cudaMemcpyAsync(d_args, host_args, sizeof(qb::TopSelectArgs) * size_t(m), cudaMemcpyHostToDevice, ctx->stream));
+    QB_CUDA(cudaMemsetAsync(d_counts, 0, count_bytes, ctx->stream));
+    const dim3 grid(top_select_ctas(ctx, size), unsigned(m));
+    QB_TRY(with_index_width(ctx, n_bits, [&](auto i) {
+        using Idx = decltype(i);
+        qb::top_select_kernel<T, Idx><<<grid, 32 * qb::kSelWarps, 0, ctx->stream>>>(static_cast<const C*>(states), stride, Idx(size), index_offset, d_args,
+                                                                                     d_counts);
+        return check_launch(ctx, "top_select_kernel");
+    }));
+    QB_TRY(ctx->pin_out.reserve(count_bytes));
+    QB_CUDA(cudaMemcpyAsync(ctx->pin_out.p, d_counts, count_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    QB_CUDA(cudaStreamSynchronize(ctx->stream));
+    std::memcpy(host_counts, ctx->pin_out.p, count_bytes);
+    return QB_OK;
+}
+
+// the collect of `n` states: count pass, check of the totals against `expect`, store pass into rows of `capacity`
+template <typename T>
+int top_collect_t(qb_context* ctx, const void* states, uint64_t stride, uint64_t size, int n_bits, uint64_t index_offset,
+                  const qb::TopCollectArgs* host_args, int n, qb::TopCollectArgs* d_args, uint32_t* d_cta, uint64_t capacity, int64_t* d_index,
+                  double* d_prob, std::vector<uint64_t>& totals) {
+    using C = typename qb::Cx<T>::type;
+    uint64_t seg = 0;
+    const unsigned n_cta = top_collect_ctas(ctx, size, &seg);
+    QB_CUDA(cudaMemcpyAsync(d_args, host_args, sizeof(qb::TopCollectArgs) * size_t(n), cudaMemcpyHostToDevice, ctx->stream));
+    const dim3 grid(n_cta, unsigned(n));
+    for (int store = 0; store < 2; ++store) {
+        QB_TRY(with_index_width(ctx, n_bits, [&](auto i) {
+            using Idx = decltype(i);
+            qb::top_collect_kernel<T, Idx><<<grid, qb::kTopCollectThreads, 0, ctx->stream>>>(static_cast<const C*>(states), stride, Idx(size), Idx(seg),
+                                                                                           index_offset, d_args, d_cta, store, capacity, d_index, d_prob);
+            return check_launch(ctx, "top_collect_kernel");
+        }));
+        if (store) break;
+        const size_t cta_bytes = sizeof(uint32_t) * n_cta * size_t(n);
+        QB_TRY(ctx->pin_out.reserve(cta_bytes));
+        QB_CUDA(cudaMemcpyAsync(ctx->pin_out.p, d_cta, cta_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+        QB_CUDA(cudaStreamSynchronize(ctx->stream));
+        const uint32_t* c = static_cast<const uint32_t*>(ctx->pin_out.p);
+        totals.assign(size_t(n), 0);
+        for (int r = 0; r < n; ++r)
+            for (unsigned i = 0; i < n_cta; ++i) totals[r] += c[size_t(r) * n_cta + i];
+        for (int r = 0; r < n; ++r)
+            if (totals[r] > capacity)
+                return fail(QB_ERR_INVALID, "the collect found " + std::to_string(totals[r]) + " entries, more than the capacity of " + std::to_string(capacity));
+    }
+    return QB_OK;
+}
+
+int check_top_shard(qb_context* ctx, int dtype, int n_local, const void* d_state, double min_probability, const qb_top_select* sel,
+                    const int32_t* positions, bool want_done) {
+    if (!ctx || !d_state) return fail(QB_ERR_INVALID, "null argument");
+    if (n_local < 8 || n_local > 36) return fail(QB_ERR_INVALID, "n_local out of range");
+    if (dtype != QB_C128 && dtype != QB_C64) return fail(QB_ERR_INVALID, "dtype must be QB_C128 or QB_C64");
+    QB_TRY(check_top_limits(1, min_probability));
+    return check_top_state(sel, positions, want_done);
+}
+
 }  // namespace
 
 // =====================================================================================================
@@ -1817,6 +1957,166 @@ int qb_evaluate_observables(qb_context* ctx, int batch, const int64_t* plan_ids,
     });
 }
 
+// ---- most probable basis states ------------------------------------------------------------------------
+int qb_top_select_init(qb_top_select* sel, int n_qubits, int64_t max_states) {
+    if (!sel) return fail(QB_ERR_INVALID, "null select state");
+    if (n_qubits < 1 || n_qubits > 63) return fail(QB_ERR_INVALID, "n_qubits must be in 1..63");
+    QB_TRY(check_top_limits(max_states, 0.0));
+    *sel = qb_top_select{};
+    sel->max_states = sel->need = uint64_t(max_states);
+    sel->n_qubits = n_qubits, sel->p_free = 64, sel->idx_hi = n_qubits;
+    return QB_OK;
+}
+
+// The decision rule of every route.  The buckets of this pass partition the entries of the current prefix range, in key order;
+// the first bucket at which the running count reaches `need` holds the cut.  Reached exactly: the bucket is taken whole and
+// the stop key is its last key.  Otherwise the bucket's digit is fixed and the next pass splits it.
+int qb_top_select_pick(qb_top_select* sel, const uint64_t counts[256]) {
+    if (!counts) return fail(QB_ERR_INVALID, "null counts");
+    QB_TRY(check_top_state(sel, nullptr, false));
+    qb_top_select& s = *sel;
+    uint64_t total = 0;
+    for (int b = 0; b < qb::kSelBuckets; ++b) total += counts[b];
+    const bool first = s.passes == 0;
+    s.passes++;
+    if (total <= s.need) {
+        if (!first) return fail(QB_ERR_INVALID, "the bucket counts of a later pass must exceed the entries still needed");
+        s.done = 1, s.selected = total;  // no more eligible entries than max_states: all of them
+        s.stop_key = s.stop_index = ~uint64_t(0);
+        return QB_OK;
+    }
+    int pick = 0;
+    uint64_t before = 0;
+    while (before + counts[pick] < s.need) before += counts[pick++];
+    const bool whole = before + counts[pick] == s.need;
+    if (s.p_free > 0) {
+        const int low = s.p_free - qb::kSelBits;
+        const uint64_t fixed = (s.p_free == 64 ? 0 : s.p_prefix << s.p_free) | (uint64_t(pick) << low);
+        if (whole) {
+            s.stop_key = fixed | ((uint64_t(1) << low) - 1), s.stop_index = ~uint64_t(0);
+        } else {
+            s.p_prefix = (s.p_free == 64 ? 0 : s.p_prefix << qb::kSelBits) | uint64_t(pick);
+            s.p_free = low;
+        }
+    } else {
+        const int lo = std::max(0, s.idx_hi - qb::kSelBits);
+        if (pick >> (s.idx_hi - lo)) return fail(QB_ERR_INVALID, "a count in a bucket beyond the digit's width");
+        const uint64_t fixed = s.idx_prefix | (uint64_t(pick) << lo);
+        if (whole) {
+            s.stop_key = s.p_prefix, s.stop_index = fixed | ((uint64_t(1) << lo) - 1);
+        } else {
+            if (lo == 0) return fail(QB_ERR_INVALID, "more than one entry counted for one complete key");
+            s.idx_prefix = fixed, s.idx_hi = lo;
+        }
+    }
+    if (whole) {
+        s.done = 1, s.selected = s.max_states;
+    } else {
+        s.taken += before, s.need -= before;
+    }
+    return QB_OK;
+}
+
+int qb_top_states(qb_context* ctx, int batch, const int64_t* plan_ids, const double* params, const int64_t* param_offsets, int64_t max_states,
+                  double min_probability, int64_t* out_counts, int64_t* out_indices, double* out_probs) {
+    if (!ctx || !plan_ids || !param_offsets || !out_counts || !out_indices || !out_probs) return fail(QB_ERR_INVALID, "null argument");
+    QB_TRY(check_top_limits(max_states, min_probability));
+    if (batch <= 0) return QB_OK;
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    QB_ON_DEVICE(ctx);
+    const Plan* first = find_plan(ctx, plan_ids[0]);
+    if (!first) return fail(QB_ERR_NOT_FOUND, "unknown plan id " + std::to_string(plan_ids[0]));
+    QB_TRY(check_plans(ctx, batch, plan_ids, first->n_qubits, "the first circuit acts", "top-states", &first));
+    const uint64_t size = uint64_t(1) << first->n_eff, M = uint64_t(max_states);
+    uint64_t seg = 0;
+    const unsigned col_ctas = top_collect_ctas(ctx, size, &seg);
+    // per state: the statevector, its output rows (16 B per slot), its bucket counts, per-CTA counts and pass arguments; once:
+    // the sort's second buffers and CUB's storage
+    size_t sort_bytes = 0;
+    {
+        cub::DoubleBuffer<double> keys(nullptr, nullptr);
+        cub::DoubleBuffer<int64_t> vals(nullptr, nullptr);
+        QB_CUDA(cub::DeviceRadixSort::SortPairsDescending(nullptr, sort_bytes, keys, vals, int(M), 0, 64, ctx->stream));
+    }
+    auto align = [](size_t v) { return (v + 255) & ~size_t(255); };
+    const size_t state_bytes = size_t(size) * amp_bytes(first->dtype);
+    const size_t row_bytes = align(16 * M) + align(sizeof(uint64_t) * qb::kSelBuckets) + align(sizeof(uint32_t) * col_ctas) +
+                             align(sizeof(qb::TopSelectArgs)) + align(sizeof(qb::TopCollectArgs));
+    const size_t once_bytes = align(16 * M) + align(sort_bytes);
+    const size_t limit = workspace_limit_of(ctx);
+    if (state_bytes + row_bytes + once_bytes > limit)
+        return fail(QB_ERR_MEMORY, "one statevector (" + std::to_string(state_bytes) + " bytes) and its top-states scratch (" +
+                                       std::to_string(row_bytes + once_bytes) + " bytes) do not fit the workspace of " + std::to_string(limit) + " bytes");
+    const int chunk = int(std::min<size_t>({size_t(batch), max_batch_for(ctx, first), (limit - once_bytes) / (state_bytes + row_bytes)}));
+    return run_oneshot(ctx, batch, plan_ids, params, param_offsets, nullptr, chunk, [&](DeviceBatch& b, int lo) {
+        const int n = b.batch;
+        const size_t nn = size_t(n);
+        size_t at = 0;
+        auto carve = [&](size_t bytes) {
+            const size_t here = at;
+            at += align(bytes);
+            return here;
+        };
+        const size_t o_counts = carve(sizeof(uint64_t) * qb::kSelBuckets * nn), o_cta = carve(sizeof(uint32_t) * col_ctas * nn);
+        const size_t o_idx = carve(sizeof(int64_t) * M * nn), o_prob = carve(sizeof(double) * M * nn);
+        const size_t o_alt_idx = carve(sizeof(int64_t) * M), o_alt_prob = carve(sizeof(double) * M);
+        const size_t o_sel = carve(sizeof(qb::TopSelectArgs) * nn), o_col = carve(sizeof(qb::TopCollectArgs) * nn), o_temp = carve(sort_bytes);
+        QB_TRY(ctx->scratch.reserve(at));
+        unsigned char* base = static_cast<unsigned char*>(ctx->scratch.p);
+        auto* d_counts = reinterpret_cast<unsigned long long*>(base + o_counts);
+        auto* d_cta = reinterpret_cast<uint32_t*>(base + o_cta);
+        auto* d_idx = reinterpret_cast<int64_t*>(base + o_idx);
+        auto* d_prob = reinterpret_cast<double*>(base + o_prob);
+        auto* d_sel = reinterpret_cast<qb::TopSelectArgs*>(base + o_sel);
+        auto* d_col = reinterpret_cast<qb::TopCollectArgs*>(base + o_col);
+        std::vector<qb_top_select> sel(nn);
+        for (auto& s : sel) QB_TRY(qb_top_select_init(&s, b.n_qubits, max_states));
+        // the select: every unfinished state of the chunk in each pass, one synchronisation per pass
+        std::vector<qb::TopSelectArgs> args;
+        std::vector<int> rows;
+        std::vector<uint64_t> counts;
+        for (;;) {
+            args.clear(), rows.clear();
+            for (int i = 0; i < n; ++i)
+                if (!sel[i].done) args.push_back(top_select_args(sel[i], nullptr, min_probability, i)), rows.push_back(i);
+            if (rows.empty()) break;
+            const int m = int(rows.size());
+            counts.resize(size_t(m) * qb::kSelBuckets);
+            QB_TRY(with_dtype(b.dtype, [&](auto t) {
+                return top_select_pass_t<decltype(t)>(ctx, b.states.p, size, size, b.n_eff, 0, args.data(), m, d_sel, d_counts, counts.data());
+            }));
+            for (int r = 0; r < m; ++r) QB_TRY(qb_top_select_pick(&sel[rows[r]], counts.data() + size_t(r) * qb::kSelBuckets));
+        }
+        std::vector<qb::TopCollectArgs> cargs(nn);
+        for (int i = 0; i < n; ++i) cargs[i] = top_collect_args(sel[i], nullptr, min_probability, i);
+        std::vector<uint64_t> totals;
+        QB_TRY(with_dtype(b.dtype, [&](auto t) {
+            return top_collect_t<decltype(t)>(ctx, b.states.p, size, size, b.n_eff, 0, cargs.data(), n, d_col, d_cta, M, d_idx, d_prob, totals);
+        }));
+        // per state: stable sort by descending p (the collect wrote index order), then its row straight into the caller's arrays
+        for (int pos = 0; pos < n; ++pos) {
+            if (totals[pos] != sel[pos].selected)
+                return fail(QB_ERR_CUDA, "the collect found " + std::to_string(totals[pos]) + " entries, the select " + std::to_string(sel[pos].selected));
+            const int cnt = int(totals[pos]);
+            cub::DoubleBuffer<double> keys(d_prob + size_t(pos) * M, reinterpret_cast<double*>(base + o_alt_prob));
+            cub::DoubleBuffer<int64_t> vals(d_idx + size_t(pos) * M, reinterpret_cast<int64_t*>(base + o_alt_idx));
+            if (cnt > 1) QB_CUDA(cub::DeviceRadixSort::SortPairsDescending(base + o_temp, sort_bytes, keys, vals, cnt, 0, 64, ctx->stream));
+            const size_t row = size_t(lo) + size_t(b.order[pos]);
+            int64_t* idx_row = out_indices + row * M;
+            double* prob_row = out_probs + row * M;
+            if (cnt) {
+                QB_CUDA(cudaMemcpyAsync(idx_row, vals.Current(), sizeof(int64_t) * cnt, cudaMemcpyDeviceToHost, ctx->stream));
+                QB_CUDA(cudaMemcpyAsync(prob_row, keys.Current(), sizeof(double) * cnt, cudaMemcpyDeviceToHost, ctx->stream));
+            }
+            QB_CUDA(cudaStreamSynchronize(ctx->stream));  // (the second buffers serve the next state)
+            std::fill(idx_row + cnt, idx_row + M, int64_t(-1));
+            std::fill(prob_row + cnt, prob_row + M, 0.0);
+            out_counts[row] = cnt;
+        }
+        return QB_OK;
+    });
+}
+
 int qb_statevector(qb_context* ctx, int64_t plan_id, const double* params, int n_params, double* out_re_im) {
     if (!ctx || !out_re_im) return fail(QB_ERR_INVALID, "null argument");
     std::lock_guard<std::mutex> lock(ctx->mu);
@@ -1966,6 +2266,53 @@ int qb_cvar_select_device(qb_context* ctx, int64_t ham_id, int dtype, int n_loca
     QB_CUDA(cudaStreamSynchronize(ctx->stream));
     std::memcpy(out_sums, ctx->pin_out.p, sums_bytes);
     std::memcpy(out_ints, static_cast<const unsigned char*>(ctx->pin_out.p) + sums_bytes, ints_bytes);
+    return QB_OK;
+}
+
+int qb_top_select_device(qb_context* ctx, int dtype, int n_local, const void* d_state, uint64_t index_offset, double min_probability,
+                         const qb_top_select* sel, const int32_t* positions, uint64_t* out_counts) {
+    if (!out_counts) return fail(QB_ERR_INVALID, "null argument");
+    QB_TRY(check_top_shard(ctx, dtype, n_local, d_state, min_probability, sel, positions, false));
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    QB_ON_DEVICE(ctx);
+    const qb::TopSelectArgs args = top_select_args(*sel, positions, min_probability, 0);
+    QB_TRY(ctx->scratch.reserve(sizeof(uint64_t) * qb::kSelBuckets + sizeof(qb::TopSelectArgs)));
+    auto* d_counts = ctx->scratch.as<unsigned long long>();
+    auto* d_args = reinterpret_cast<qb::TopSelectArgs*>(d_counts + qb::kSelBuckets);
+    const uint64_t size = uint64_t(1) << n_local;
+    return with_dtype(dtype, [&](auto t) {
+        return top_select_pass_t<decltype(t)>(ctx, d_state, size, size, n_local, index_offset, &args, 1, d_args, d_counts, out_counts);
+    });
+}
+
+int qb_top_collect_device(qb_context* ctx, int dtype, int n_local, const void* d_state, uint64_t index_offset, double min_probability,
+                          const qb_top_select* sel, const int32_t* positions, int64_t capacity, int64_t* out_count, int64_t* out_indices,
+                          double* out_probs) {
+    if (!out_count || !out_indices || !out_probs) return fail(QB_ERR_INVALID, "null argument");
+    if (capacity < 0) return fail(QB_ERR_INVALID, "negative capacity");
+    QB_TRY(check_top_shard(ctx, dtype, n_local, d_state, min_probability, sel, positions, true));
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    QB_ON_DEVICE(ctx);
+    const qb::TopCollectArgs args = top_collect_args(*sel, positions, min_probability, 0);
+    const uint64_t size = uint64_t(1) << n_local, cap = uint64_t(std::max<int64_t>(capacity, 1));
+    uint64_t seg = 0;
+    const unsigned n_cta = top_collect_ctas(ctx, size, &seg);
+    const size_t idx_bytes = sizeof(int64_t) * cap, cta_bytes = (sizeof(uint32_t) * n_cta + 15) & ~size_t(15);
+    QB_TRY(ctx->scratch.reserve(2 * idx_bytes + cta_bytes + sizeof(qb::TopCollectArgs)));
+    auto* d_idx = ctx->scratch.as<int64_t>();
+    auto* d_prob = reinterpret_cast<double*>(d_idx + cap);
+    auto* d_cta = reinterpret_cast<uint32_t*>(d_prob + cap);
+    auto* d_args = reinterpret_cast<qb::TopCollectArgs*>(reinterpret_cast<unsigned char*>(d_cta) + cta_bytes);
+    std::vector<uint64_t> totals;
+    QB_TRY(with_dtype(dtype, [&](auto t) {
+        return top_collect_t<decltype(t)>(ctx, d_state, size, size, n_local, index_offset, &args, 1, d_args, d_cta, uint64_t(capacity), d_idx, d_prob, totals);
+    }));
+    if (totals[0]) {
+        QB_CUDA(cudaMemcpyAsync(out_indices, d_idx, sizeof(int64_t) * totals[0], cudaMemcpyDeviceToHost, ctx->stream));
+        QB_CUDA(cudaMemcpyAsync(out_probs, d_prob, sizeof(double) * totals[0], cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    QB_CUDA(cudaStreamSynchronize(ctx->stream));
+    *out_count = int64_t(totals[0]);
     return QB_OK;
 }
 

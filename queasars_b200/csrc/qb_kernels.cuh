@@ -11,6 +11,7 @@
 //   chunk_prob_kernel / scan_chunks_kernel / sample_kernel   K5  prefix-sum CDF sampling
 //   cvar_chunk_kernel / scan_chunks_kernel / cvar_finish_kernel  K6  exact CVaR(alpha) of a diagonal Hamiltonian (sorted lower tail)
 //   cvar_select_kernel / cvar_select_reduce_kernel  K8  one radix-digit pass of the exact CVaR of a sharded state (weighted select)
+//   top_select_kernel / top_collect_kernel  K9  most probable basis states: counts-only radix select of (~bits(p), logical k), ordered collect
 //   swap_p2p_kernel            global <-> local qubit swap of a sharded state fused with its all-to-all (peer-memory stores)
 //
 // What the arithmetic follows ([upstream] = un-vendored qiskit 2.4.2, see oracle/qiskit_semantics.py):
@@ -1528,6 +1529,21 @@ __device__ __forceinline__ uint64_t energy_key(double e) {
     return (u >> 63) ? ~u : (u | 0x8000000000000000ull);
 }
 
+// Whether an entry with value key `key` (the energy key here, the probability key in top_select_kernel) and physical index kk
+// matches the prefix of `a`, and the digit d of its key (digit_kind 0) or of its logical index (digit_kind 1) for this pass
+__device__ __forceinline__ bool select_digit(const SelectArgs& a, uint64_t key, uint64_t kk, unsigned& d) {
+    const bool ok = (kk & a.idx_mask) == a.idx_value && (a.e_free >= 64 || (key >> a.e_free) == a.e_prefix);
+    d = 0;
+    if (a.digit_kind == 0) {
+        d = unsigned(key >> (a.e_free - a.bits)) & ((1u << a.bits) - 1u);
+    } else {
+#pragma unroll
+        for (int j = 0; j < kSelBits; ++j)  // (unrolled: constant indices keep a.pos in registers, off the stack)
+            if (j < a.bits) d |= unsigned((kk >> a.pos[j]) & 1) << j;
+    }
+    return ok;
+}
+
 // grid = n_cta (fixed by the device and the shard size), block = 32 * kSelWarps.  part_* = [bucket][cta];
 // ints = [count | emin | emax | kmin][bucket], initialised by the caller (0, ~0, 0, ~0)
 template <typename T>
@@ -1545,7 +1561,6 @@ cvar_select_kernel(const typename Cx<T>::type* __restrict__ state, double2* __re
         s_cnt[b] = 0, s_min[b] = ~0ull, s_max[b] = 0, s_kmin[b] = ~0ull;
     }
     __syncthreads();
-    const unsigned dmask = (1u << a.bits) - 1u;
     const uint64_t stride = uint64_t(gridDim.x) * kSelWarps * 32;
     // size is a multiple of 32: every lane of a warp runs the same iterations (the warp-synchronous steps below need it)
     for (uint64_t k = (uint64_t(blockIdx.x) * kSelWarps + warp) * 32 + lane; k < size; k += stride) {
@@ -1562,16 +1577,8 @@ cvar_select_kernel(const typename Cx<T>::type* __restrict__ state, double2* __re
             if (cache_mode == 1) cache[k] = make_double2(p, e);
         }
         const uint64_t kk = k | index_offset;
-        const uint64_t key = energy_key(e);
-        const bool ok = (kk & a.idx_mask) == a.idx_value && (a.e_free >= 64 || (key >> a.e_free) == a.e_prefix);
-        unsigned d = 0;
-        if (a.digit_kind == 0) {
-            d = unsigned(key >> (a.e_free - a.bits)) & dmask;
-        } else {
-#pragma unroll
-            for (int j = 0; j < kSelBits; ++j)  // (unrolled: constant indices keep a.pos in registers, off the stack)
-                if (j < a.bits) d |= unsigned((kk >> a.pos[j]) & 1) << j;
-        }
+        unsigned d;
+        const bool ok = select_digit(a, energy_key(e), kk, d);
         const unsigned peers = __match_any_sync(0xffffffffu, ok ? d : 0xffffffffu);
         st_p[warp][lane] = p, st_e[warp][lane] = e, st_k[warp][lane] = kk;
         __syncwarp();
@@ -1618,6 +1625,182 @@ cvar_select_reduce_kernel(const double* __restrict__ part, int n_cta, double* __
     for (int i = threadIdx.x; i < n_cta; i += blockDim.x) acc += p[i];
     const double total = block_sum(acc, s_red);
     if (threadIdx.x == 0) out[blockIdx.x] = total;
+}
+
+// ---------------------------------------------------------------------------------------------------
+// most probable basis states (K9): the max_states first entries of the composite key (prob_key(p_k), logical k) -- descending
+// p_k, ties in ascending logical index -- among the entries with p_k > 0 and p_k >= min_probability, without sorting the state.
+// top_select_kernel histograms one 8-bit digit of that key per pass (counts only, over the entries matching the prefix fixed so
+// far; SelectArgs / select_digit of the CVaR select with the probability key in place of the energy key); the host picks the
+// bucket (qb_top_select_pick) until the stop key is known, then top_collect_kernel writes every entry up to the stop key.
+// p_k = re^2 + im^2 in double, rounded without FMA contraction, so a NumPy re * re + im * im on the same amplitudes gives
+// every bit.  Counts are integers: the histograms and the compaction are the same on every run whatever the scheduling.
+// ---------------------------------------------------------------------------------------------------
+struct TopSelectArgs {
+    SelectArgs sel;  // prefix and digit of this pass (e_prefix / e_free: the probability key's)
+    double min_probability;
+    int32_t entry;   // row of `states`
+};
+
+struct TopCollectArgs {
+    uint64_t stop_key, stop_index;  // every eligible entry with (prob_key, logical k) <= (stop_key, stop_index) is written
+    double min_probability;
+    int32_t entry;                  // row of `states`
+    int32_t n_pos;                  // 0: logical index == physical index; else logical bit q sits at physical position pos[q]
+    int8_t pos[64];
+};
+
+template <typename C>
+__device__ __forceinline__ double top_prob(C a) {
+    const double x = double(a.x), y = double(a.y);
+    return __dadd_rn(__dmul_rn(x, x), __dmul_rn(y, y));
+}
+
+// ascending key = descending p: for p > 0 the bit pattern is ordered like the value
+__device__ __forceinline__ uint64_t prob_key(double p) { return ~uint64_t(__double_as_longlong(p)); }
+
+__device__ __forceinline__ bool top_eligible(double p, double min_probability) { return p > 0.0 && p >= min_probability; }
+
+constexpr int kTopUnroll = 4;  // amplitudes loaded per thread before any is processed
+
+// grid = (n_cta, entries of this pass), block = 32 * kSelWarps; counts = [entry][bucket], zeroed by the caller.  Idx: uint32_t
+// up to 2^31 amplitudes, uint64_t above (the sweep kernels' switch).
+template <typename T, typename Idx>
+__global__ void __launch_bounds__(32 * kSelWarps)
+top_select_kernel(const typename Cx<T>::type* __restrict__ states, uint64_t state_stride, Idx size, uint64_t index_offset,
+                  const TopSelectArgs* __restrict__ args, unsigned long long* __restrict__ counts) {
+    __shared__ uint32_t h[kSelWarps][kSelBuckets];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    for (int b = threadIdx.x; b < kSelWarps * kSelBuckets; b += blockDim.x) h[b / kSelBuckets][b % kSelBuckets] = 0;
+    __syncthreads();
+    const TopSelectArgs ta = args[blockIdx.y];
+    const auto* st = states + uint64_t(ta.entry) * state_stride;
+    const Idx stride = Idx(gridDim.x) * (kSelWarps * 32);
+    // size is a multiple of 32: every lane of a warp runs the same iterations (the warp-synchronous steps below need it)
+    for (Idx k0 = (Idx(blockIdx.x) * kSelWarps + warp) * 32 + lane; k0 < size; k0 += kTopUnroll * stride) {
+        typename Cx<T>::type v[kTopUnroll];
+#pragma unroll
+        for (int u = 0; u < kTopUnroll; ++u)
+            if (k0 + u * stride < size) v[u] = st[k0 + u * stride];
+#pragma unroll
+        for (int u = 0; u < kTopUnroll; ++u) {
+            const Idx k = k0 + u * stride;
+            if (k < size) {
+                const double p = top_prob(v[u]);
+                unsigned d = 0;
+                const bool ok = top_eligible(p, ta.min_probability) && select_digit(ta.sel, prob_key(p), uint64_t(k) | index_offset, d);
+                if (__ballot_sync(0xffffffffu, ok)) {  // one shared-memory add per distinct digit of the warp
+                    const unsigned peers = __match_any_sync(0xffffffffu, ok ? d : 0xffffffffu);
+                    if (ok && lane == __ffs(peers) - 1) atomicAdd(&h[warp][d], unsigned(__popc(peers)));
+                }
+            }
+        }
+    }
+    __syncthreads();
+    for (int b = threadIdx.x; b < kSelBuckets; b += blockDim.x) {
+        uint32_t c = 0;
+        for (int w = 0; w < kSelWarps; ++w) c += h[w][b];
+        if (c) atomicAdd(&counts[uint64_t(blockIdx.y) * kSelBuckets + b], (unsigned long long)c);
+    }
+}
+
+__device__ __forceinline__ bool top_taken(const TopCollectArgs& a, const TopCollectArgs* __restrict__ ga, double p, uint64_t kk) {
+    if (!top_eligible(p, a.min_probability)) return false;
+    const uint64_t key = prob_key(p);
+    if (key != a.stop_key) return key < a.stop_key;
+    if (a.stop_index == ~0ull) return true;
+    uint64_t logical = kk;
+    if (a.n_pos) {  // (entries tied with the stop key only)
+        logical = 0;
+        for (int q = 0; q < a.n_pos; ++q) logical |= ((kk >> ga->pos[q]) & 1ull) << q;
+    }
+    return logical <= a.stop_index;
+}
+
+constexpr int kTopCollectThreads = 256;
+constexpr int kTopTile = kTopCollectThreads * kTopUnroll;  // amplitudes per step: kTopUnroll consecutive ones per thread
+
+// grid = (n_cta, entries), block = kTopCollectThreads; CTA c owns the amplitudes [c * seg, (c + 1) * seg) of its entry.
+// store == 0: cta_counts[entry][c] = number of entries taken in the segment.  store == 1: each CTA starts at the sum of the
+// counts of the CTAs before it and writes its entries in index order (block scan per step): out_index[entry][i] = physical
+// index (index_offset | k), out_prob[entry][i] = p, i < capacity.
+template <typename T, typename Idx>
+__global__ void __launch_bounds__(kTopCollectThreads)
+top_collect_kernel(const typename Cx<T>::type* __restrict__ states, uint64_t state_stride, Idx size, Idx seg, uint64_t index_offset,
+                   const TopCollectArgs* __restrict__ args, uint32_t* __restrict__ cta_counts, int store, uint64_t capacity,
+                   int64_t* __restrict__ out_index, double* __restrict__ out_prob) {
+    __shared__ uint32_t s_warp[kTopCollectThreads / 32];
+    __shared__ uint64_t s_base;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const TopCollectArgs* ga = args + blockIdx.y;
+    const TopCollectArgs a = *ga;
+    const auto* st = states + uint64_t(a.entry) * state_stride;
+    uint32_t* row_counts = cta_counts + uint64_t(blockIdx.y) * gridDim.x;
+    const Idx begin = Idx(blockIdx.x) * seg, end = begin + seg < size ? begin + seg : size;
+    uint64_t base = 0;
+    if (store) {
+        uint64_t before = 0;
+        for (unsigned c = threadIdx.x; c < blockIdx.x; c += blockDim.x) before += row_counts[c];
+        for (int o = 16; o > 0; o >>= 1) before += __shfl_xor_sync(0xffffffffu, before, o);
+        if (threadIdx.x == 0) s_base = 0;
+        __syncthreads();
+        if (lane == 0 && before) atomicAdd(reinterpret_cast<unsigned long long*>(&s_base), (unsigned long long)before);
+        __syncthreads();
+        base = s_base;
+    }
+    uint32_t total = 0;
+    for (Idx t = begin; t < end; t += kTopTile) {
+        const Idx k0 = t + Idx(threadIdx.x) * kTopUnroll;
+        typename Cx<T>::type v[kTopUnroll];
+#pragma unroll
+        for (int u = 0; u < kTopUnroll; ++u)
+            if (k0 + u < end) v[u] = st[k0 + u];
+        unsigned flags = 0;
+#pragma unroll
+        for (int u = 0; u < kTopUnroll; ++u)
+            if (k0 + u < end && top_taken(a, ga, top_prob(v[u]), uint64_t(k0 + u) | index_offset)) flags |= 1u << u;
+        const uint32_t mine = __popc(flags);
+        if (!store) {
+            total += mine;
+            continue;
+        }
+        // exclusive prefix of `mine` over the block in thread order
+        uint32_t incl = mine;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const uint32_t nb = __shfl_up_sync(0xffffffffu, incl, o);
+            if (lane >= o) incl += nb;
+        }
+        if (lane == 31) s_warp[warp] = incl;
+        __syncthreads();
+        uint32_t warp_before = 0, step_total = 0;
+        for (int w = 0; w < kTopCollectThreads / 32; ++w) {
+            const uint32_t c = s_warp[w];
+            warp_before += w < warp ? c : 0;
+            step_total += c;
+        }
+        uint64_t at = base + warp_before + incl - mine;
+#pragma unroll
+        for (int u = 0; u < kTopUnroll; ++u) {
+            if ((flags >> u) & 1) {
+                if (at < capacity) {
+                    out_index[uint64_t(blockIdx.y) * capacity + at] = int64_t(uint64_t(k0 + u) | index_offset);
+                    out_prob[uint64_t(blockIdx.y) * capacity + at] = top_prob(v[u]);
+                }
+                ++at;
+            }
+        }
+        base += step_total;
+        __syncthreads();  // s_warp is rewritten by the next step
+    }
+    if (!store) {
+        for (int o = 16; o > 0; o >>= 1) total += __shfl_xor_sync(0xffffffffu, total, o);
+        if (threadIdx.x == 0) s_warp[0] = 0;
+        __syncthreads();
+        if (lane == 0 && total) atomicAdd(&s_warp[0], total);
+        __syncthreads();
+        if (threadIdx.x == 0) row_counts[blockIdx.x] = s_warp[0];
+    }
 }
 
 // ---------------------------------------------------------------------------------------------------

@@ -167,6 +167,34 @@ def observable_terms(operators):
     return int(width), np.concatenate(xs), np.concatenate(zs), np.concatenate(cs), np.asarray(offsets, dtype=np.int64)
 
 
+TOP_MAX_STATES = 1 << 20
+
+
+def check_top_limits(max_states, min_probability) -> tuple[int, float]:
+    """The limits of every top-states call: ``max_states`` in [1, 2^20], ``min_probability`` finite and >= 0 (ValueError otherwise)."""
+    if isinstance(max_states, bool) or not isinstance(max_states, (int, np.integer)) or not 1 <= int(max_states) <= TOP_MAX_STATES:
+        raise ValueError(f"max_states must be an integer in [1, 2^20], got {max_states!r}")
+    p = float(min_probability)
+    if not math.isfinite(p) or p < 0.0:
+        raise ValueError(f"min_probability must be finite and >= 0, got {min_probability!r}")
+    return int(max_states), p
+
+
+def top_select_new(n_qubits: int, max_states: int) -> _native.TopSelect:
+    """A fresh top-states select of ``max_states`` entries over a state of ``n_qubits`` logical qubits (``qb_top_select_init``)."""
+    sel = _native.TopSelect()
+    _native.check(_native.load().qb_top_select_init(byref(sel), int(n_qubits), int(max_states)))
+    return sel
+
+
+def top_select_pick(sel: _native.TopSelect, counts) -> None:
+    """Advance ``sel`` by the 256 bucket counts of its pass, summed over all shards (``qb_top_select_pick``, pure host code)."""
+    c = np.ascontiguousarray(counts, dtype=np.uint64).reshape(-1)
+    if c.size != 256:
+        raise ValueError("a select pass has 256 bucket counts")
+    _native.check(_native.load().qb_top_select_pick(byref(sel), _native.ptr(c)))
+
+
 @functools.lru_cache(maxsize=256)
 def pipeline_split_point(n: int, n_eff: int, tile_bits: int, sm_count: int) -> Optional[int]:
     """First-chunk size of the two-chunk pipelined submission of ``n`` evaluations of ``n_eff``-qubit states: the split (between
@@ -518,6 +546,21 @@ class Engine:
         _native.check(self._lib.qb_evaluate_cvar(self._ctx, len(plans), _native.ptr(ids), _native.ptr(flat), _native.ptr(offsets), ham.ham_id, float(alpha), _native.ptr(out)))
         return out
 
+    def top_states(self, plans: Sequence[PlanHandle], params: Sequence[Sequence[float]], max_states: int, min_probability: float = 0.0) -> list:
+        """The most probable basis states of every circuit's state, exactly, without shots or a copy of the state
+        (``qb_top_states``): per circuit (int64 logical indices, float64 probabilities), descending probability, ties in ascending
+        index, at most ``max_states`` entries with p > 0 and p >= ``min_probability``."""
+        max_states, min_probability = check_top_limits(max_states, min_probability)
+        if not plans:
+            return []
+        ids, flat, offsets = self._pack(plans, params)
+        counts = np.empty(len(plans), dtype=np.int64)
+        idx = np.empty((len(plans), max_states), dtype=np.int64)
+        probs = np.empty((len(plans), max_states), dtype=np.float64)
+        _native.check(self._lib.qb_top_states(self._ctx, len(plans), _native.ptr(ids), _native.ptr(flat), _native.ptr(offsets), max_states, min_probability,
+                                              _native.ptr(counts), _native.ptr(idx), _native.ptr(probs)))
+        return [(idx[i, : counts[i]].copy(), probs[i, : counts[i]].copy()) for i in range(len(plans))]
+
     def expectation_many(self, plans: Sequence[PlanHandle], params: Sequence[Sequence[float]], handle: ObservablesHandle) -> np.ndarray:
         """Re <psi_i|H_j|psi_i> of every circuit and every observable of ``handle``: float64 array [len(plans), n_obs], each
         distinct Pauli string reduced once per state (``qb_evaluate_observables``)."""
@@ -571,6 +614,30 @@ class Engine:
                                                       c_void_p(cache_ptr or None), int(cache_mode), int(e_prefix), int(e_free), int(digit_kind), int(bits),
                                                       _native.ptr(pos), int(idx_mask), int(idx_value), _native.ptr(sums), _native.ptr(ints)))
         return sums, ints
+
+    def top_select_device(self, dtype, n_local: int, state_ptr: int, index_offset: int, min_probability: float, sel: _native.TopSelect,
+                          positions: Optional[Sequence[int]] = None) -> np.ndarray:
+        """Bucket counts (uint64 [256]) of the select pass ``sel`` describes on a caller-owned shard (``qb_top_select_device``);
+        ``positions[q]`` = physical bit position of logical qubit q (None: the identity)."""
+        pos = None if positions is None else np.ascontiguousarray(positions, dtype=np.int32)
+        out = np.empty(256, dtype=np.uint64)
+        _native.check(self._lib.qb_top_select_device(self._ctx, _dtype_code(dtype), int(n_local), c_void_p(state_ptr), int(index_offset), float(min_probability),
+                                                     byref(sel), None if pos is None else _native.ptr(pos), _native.ptr(out)))
+        return out
+
+    def top_collect_device(self, dtype, n_local: int, state_ptr: int, index_offset: int, min_probability: float, sel: _native.TopSelect,
+                           positions: Optional[Sequence[int]], capacity: int):
+        """This shard's entries up to the stop key of the finished select ``sel`` (``qb_top_collect_device``), in physical index
+        order -> (int64 physical indices, float64 probabilities)."""
+        pos = None if positions is None else np.ascontiguousarray(positions, dtype=np.int32)
+        cap = max(1, int(capacity))
+        idx = np.empty(cap, dtype=np.int64)
+        probs = np.empty(cap, dtype=np.float64)
+        count = c_int64()
+        _native.check(self._lib.qb_top_collect_device(self._ctx, _dtype_code(dtype), int(n_local), c_void_p(state_ptr), int(index_offset), float(min_probability),
+                                                      byref(sel), None if pos is None else _native.ptr(pos), int(capacity), byref(count), _native.ptr(idx),
+                                                      _native.ptr(probs)))
+        return idx[: count.value].copy(), probs[: count.value].copy()
 
     def swap_global_p2p(self, dtype, n_local: int, state_ptr: int, peer_ptrs: Sequence[int], rank: int, local_positions: Sequence[int]):
         """Launch the fused swap + all-to-all kernel (asynchronous on the engine's stream; see include/queasars_b200.h)."""

@@ -61,12 +61,20 @@ if _ReferenceBase is not None:
     _ReferenceBase.register(BaseCircuitEvaluator)
 
 
-def measure_quasi_distributions(circuits: list, parameter_values: list[list[float]], sampler, shots: int) -> list[QuasiDistribution]:
+def measure_quasi_distributions(circuits: list, parameter_values: list[list[float]], sampler, shots: Optional[int], *,
+                                max_states: int = 1024) -> list[QuasiDistribution]:
     """Same contract as circuit_evaluation.py:29-59.  With a ``B200SamplerV2`` the ``measure_all`` copy and the
     per-pub primitive round trip are skipped (sampling the full register *is* measure_all); any other
-    SamplerV2 goes through the generic pub path exactly like the reference."""
+    SamplerV2 goes through the generic pub path exactly like the reference.
+
+    ``shots=None`` with a ``B200SamplerV2``: no sampling -- every distribution holds the exact probabilities of the
+    ``max_states`` most probable basis states of its circuit's state (``B200SamplerV2.top_states``; ties in ascending basis
+    index), with ``shots=None``.  The default of 1024 is the most entries a 1024-shot distribution can hold."""
     if isinstance(sampler, B200SamplerV2):
         pairs = [(c, p) for c, p in zip(circuits, parameter_values) if c is not None and p is not None]
+        if shots is None:
+            tops = sampler.top_states([c for c, _ in pairs], [p for _, p in pairs], max_states)
+            return [QuasiDistribution({int(k): float(v) for k, v in zip(idx, probs)}, shots=None) for idx, probs in tops]
         idx = sampler.sample_indices([c for c, _ in pairs], [p for _, p in pairs], shots)
         out = []
         for row in idx:

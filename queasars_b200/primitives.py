@@ -751,6 +751,25 @@ class B200SamplerV2(_B200Primitive):
             raise ValueError("all circuits of one sampler submission must act on the same number of qubits")
         return np.asarray(self._submit(("smp", int(shots), widths.pop()), (None, circuits, parameter_values)))
 
+    def top_states(self, circuits, parameter_values, max_states: int, min_probability: float = 0.0) -> list:
+        """The most probable basis states of every circuit's state, exactly and without shots: per circuit a pair (int64 logical
+        basis indices, float64 probabilities) of the entries with p > 0 and p >= ``min_probability``, in descending p, ties in
+        ascending index, at most ``max_states`` (1 .. 2^20) of them (``Engine.top_states``).  Circuits too wide for one GPU run
+        as one statevector sharded over the device set, one at a time, and give the same entries (``_ShardedLogic.top_states``);
+        that route needs no second device."""
+        from .engine import check_top_limits
+
+        max_states, min_probability = check_top_limits(max_states, min_probability)
+        circuits, parameter_values = list(circuits), list(parameter_values)
+        if len(circuits) != len(parameter_values):
+            raise ValueError(f"{len(circuits)} circuits but {len(parameter_values)} parameter vectors")
+        if not circuits:
+            return []
+        widths = {_width(c) for c in circuits}
+        if len(widths) != 1:
+            raise ValueError("all circuits of one sampler submission must act on the same number of qubits")
+        return list(self._submit(("top", widths.pop(), max_states, min_probability), (None, circuits, parameter_values)))
+
     def cvar_values(self, circuits, parameter_values, operator, alpha: float) -> np.ndarray:
         """Exact (shot-free) CVaR(alpha) of the diagonal ``operator`` on every circuit's full distribution |psi|^2:
         ``expectation.lower_tail_expectation_arrays(|psi|^2, E, alpha)`` over all 2^n basis states, computed on the device
@@ -811,6 +830,14 @@ class B200SamplerV2(_B200Primitive):
                 )
 
             return width, sample_on_state, sample_on_devices, np.stack
+        if key[0] == "top":
+            _, width, max_states, min_probability = key
+
+            def top_on_devices(circuits, values):
+                resolved = self._resolve_all(circuits, values, probabilities_only=True)
+                return self._run_per_device(resolved, lambda slot, plans, params: self.engines[slot].top_states(plans, params, max_states, min_probability))
+
+            return width, lambda sv: sv.top_states(max_states, min_probability), top_on_devices, list
         kind, _, fp, alpha, width = key
         operator = target
 

@@ -27,7 +27,7 @@ Two drivers share the schedule (``_ShardedLogic``):
                                ``cudaDeviceEnablePeerAccess`` instead of IPC, reductions on the host.
 
 The shard-local arithmetic is delegated to a *backend* object (``apply``, ``diagonal_expectation``, ``pauli_expectation``,
-``sample``, ``cvar_select``, ``swap_p2p``); the product default drives the CUDA engine.  Tests inject a NumPy backend to exercise the
+``sample``, ``cvar_select``, ``top_select``, ``top_collect``, ``swap_p2p``); the product default drives the CUDA engine.  Tests inject a NumPy backend to exercise the
 multi-rank host logic on CPU with the gloo backend.
 """
 from __future__ import annotations
@@ -125,6 +125,16 @@ class CudaShardBackend:
         return self.engine.cvar_select_device(self._select_ham[1], "complex128", n_local, _state_ptr(state), index_offset,
                                               0 if cache is None else _state_ptr(cache), cache_mode, *spec)
 
+    def top_select(self, state, n_local: int, index_offset: int, min_probability: float, sel, positions) -> np.ndarray:
+        """One select pass of ``_ShardedLogic.top_states`` on this shard (``qb_top_select_device``): uint64 bucket counts [256]."""
+        self._join_torch_stream(state)
+        return self.engine.top_select_device("complex128", n_local, _state_ptr(state), index_offset, min_probability, sel, positions)
+
+    def top_collect(self, state, n_local: int, index_offset: int, min_probability: float, sel, positions, capacity: int):
+        """This shard's entries up to the stop key of ``sel`` (``qb_top_collect_device``) -> (physical indices, probabilities)."""
+        self._join_torch_stream(state)
+        return self.engine.top_collect_device("complex128", n_local, _state_ptr(state), index_offset, min_probability, sel, positions, capacity)
+
     def swap_p2p(self, state, peer_ptrs: Sequence[int], n_local: int, rank: int, local_positions: Sequence[int]) -> None:
         """Fused swap + all-to-all into the peers' buffers; returns when this rank's stores have been issued and completed."""
         self._join_torch_stream(state)
@@ -140,6 +150,8 @@ class _ShardedLogic:
       _sum_over_shards(fn)                        sum over all shards of fn(rank, state) -> float  (every caller gets the total)
       _shard_masses()                             |shard|^2 of all shards, ndarray [world]
       _select_pass(z, c, cache_mode, spec)        every shard's bucket arrays of one cvar select pass, in rank order
+      _top_pass(sel, positions, min_p)            every shard's bucket counts of one top-states select pass, in rank order
+      _top_collect(sel, positions, min_p)         every shard's (physical indices, probabilities) up to the stop key, in rank order
       _sample_shards(owner, local_u)              physical indices of the shots (owner[s] = shard of shot s), int64 [shots]"""
 
     def _init_logic(self, n_qubits: int, world: int, min_local: int):
@@ -351,6 +363,40 @@ class _ShardedLogic:
             hi = lo
             if hi == 0:
                 raise RuntimeError("cvar select: the full logical index matched more than one entry")
+
+    def top_states(self, max_states: int, min_probability: float = 0.0) -> tuple[np.ndarray, np.ndarray]:
+        """The most probable basis states of the state, exactly and without shots: (int64 logical indices, float64 p) of the
+        entries with p > 0 and p >= ``min_probability``, descending p, ties in ascending logical index, at most ``max_states`` of
+        them -- ``Engine.top_states`` of the unsharded state, bit for bit.
+
+        A counts-only select fixes the composite key (~bits(p), logical k) 8 bits per pass: every shard histograms the next
+        digit over its entries that match the prefix fixed so far (``qb_top_select_device``; logical index bits are read at
+        their physical positions), the shards' counts are added in rank order and ``qb_top_select_pick`` -- the decision rule of
+        the one-GPU route too -- keeps the bucket in which the cut falls.  Then every shard writes its entries up to the stop key
+        (``qb_top_collect_device``); their physical indices are mapped to logical ones and the few entries are merged by the key
+        here.  No data moves and no swap happens; every caller gets the same result."""
+        from .engine import check_top_limits, top_select_new, top_select_pick
+
+        max_states, min_probability = check_top_limits(max_states, min_probability)
+        sel = top_select_new(self.n_qubits, max_states)
+        positions = [int(p) for p in self.position]
+        self.top_passes = 0
+        while not sel.done:
+            total = np.zeros(256, dtype=np.uint64)
+            for counts in self._top_pass(sel, positions, min_probability):  # rank order
+                total = total + np.asarray(counts, dtype=np.uint64)
+            top_select_pick(sel, total)
+            self.top_passes += 1
+        parts = self._top_collect(sel, positions, min_probability)
+        physical = np.concatenate([np.asarray(i, dtype=np.int64) for i, _ in parts])
+        probs = np.concatenate([np.asarray(p, dtype=np.float64) for _, p in parts])
+        if physical.size != sel.selected:
+            raise RuntimeError(f"top states: the shards collected {physical.size} entries, the select {sel.selected}")
+        logical = np.zeros_like(physical)
+        for q in range(self.n_qubits):
+            logical |= ((physical >> self.position[q]) & 1) << q
+        order = np.lexsort((logical, -probs))
+        return logical[order], probs[order]
 
     def sample(self, shots: int, seed=None, uniforms: Optional[np.ndarray] = None) -> np.ndarray:
         """``shots`` basis-state indices (logical qubit order) drawn from |psi|^2; every caller gets all of them.
@@ -575,6 +621,23 @@ class ShardedStatevector(_ShardedLogic):
             out.append((a[:512].view(np.float64).reshape(2, 256), a[512:].view(np.uint64).reshape(4, 256)))
         return out
 
+    def _top_pass(self, sel, positions, min_probability) -> list:
+        counts = np.asarray(self.backend.top_select(self.state, self.n_local, self.index_offset, min_probability, sel, positions), dtype=np.uint64)
+        if self.world == 1:
+            return [counts]
+        t = self._torch.from_numpy(counts.view(np.int64).copy()).to(self.device)
+        parts = [self._torch.empty_like(t) for _ in range(self.world)]
+        self._dist.all_gather(parts, t, group=self.group)
+        return [part.cpu().numpy().view(np.uint64) for part in parts]
+
+    def _top_collect(self, sel, positions, min_probability) -> list:
+        mine = self.backend.top_collect(self.state, self.n_local, self.index_offset, min_probability, sel, positions, int(sel.selected))
+        if self.world == 1:
+            return [mine]
+        parts = [None] * self.world
+        self._dist.all_gather_object(parts, (np.asarray(mine[0]), np.asarray(mine[1])), group=self.group)
+        return parts
+
     def _sample_shards(self, owner: np.ndarray, local_u: np.ndarray) -> np.ndarray:
         physical = np.zeros(owner.size, dtype=np.int64)
         mine = np.nonzero(owner == self.rank)[0]
@@ -683,6 +746,13 @@ class LocalShardedStatevector(_ShardedLogic):
         spare = self._bufs[1 - self._cur]
         return self._each(lambda r: self.backends[r].cvar_select(self._state(r), spare[r].ptr, cache_mode, z_masks, coeffs, self.n_qubits, self.n_local,
                                                                  r << self.n_local, spec))
+
+    def _top_pass(self, sel, positions, min_probability) -> list:
+        return self._each(lambda r: self.backends[r].top_select(self._state(r), self.n_local, r << self.n_local, min_probability, sel, positions))
+
+    def _top_collect(self, sel, positions, min_probability) -> list:
+        return self._each(lambda r: self.backends[r].top_collect(self._state(r), self.n_local, r << self.n_local, min_probability, sel, positions,
+                                                                 int(sel.selected)))
 
     def _sample_shards(self, owner: np.ndarray, local_u: np.ndarray) -> np.ndarray:
         physical = np.zeros(owner.size, dtype=np.int64)
