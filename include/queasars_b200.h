@@ -341,6 +341,17 @@ int qb_top_collect_device(qb_context* ctx, int dtype, int n_local, const void* d
  * rank touches its destination buffer. */
 int qb_swap_global_p2p(qb_context* ctx, int dtype, int n_local, const void* d_state, void* const* peer_dst, int world, int rank,
                        int n_global, const int32_t* local_positions);
+/* The same exchange in place, with ONE shard buffer per rank: shard_states[d] is rank d's state buffer mapped into this process
+ * (shard_states[rank] = the caller's own).  The exchange is an involution: amplitude i of rank r whose local bits
+ * local_positions[j] read d != r trades places with amplitude i' (the same index with those bits replaced by the bits of r) of
+ * rank d.  Each pair is swapped by one of its two ranks (the one whose highest non-exchanged local bit of i equals (rank > d)), by
+ * a load and a store on each side.  Needs n_local >= n_global + 1; validated like qb_swap_global_p2p, nothing launches on invalid
+ * input.  Asynchronous on the context's stream.  The kernel reads and writes the peers' live states, so the caller owns two
+ * preconditions:
+ *   - every rank's earlier work on its shard has completed before ANY rank launches this kernel;
+ *   - every rank's kernel has completed before any rank uses its shard again. */
+int qb_swap_global_inplace_p2p(qb_context* ctx, int dtype, int n_local, void* const* shard_states, int world, int rank, int n_global,
+                               const int32_t* local_positions);
 
 /* --- device memory and peer mapping for sharded states ----------------------------------------------------
  * The shard buffers of a state sharded over several GPUs are plain cudaMalloc allocations owned by the engine of their device.

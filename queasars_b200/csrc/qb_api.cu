@@ -2347,6 +2347,46 @@ int qb_swap_global_p2p(qb_context* ctx, int dtype, int n_local, const void* d_st
     });
 }
 
+int qb_swap_global_inplace_p2p(qb_context* ctx, int dtype, int n_local, void* const* shard_states, int world, int rank, int n_global,
+                               const int32_t* local_positions) {
+    if (!ctx || !shard_states || !local_positions) return fail(QB_ERR_INVALID, "null argument");
+    if (dtype != QB_C128 && dtype != QB_C64) return fail(QB_ERR_INVALID, "dtype must be QB_C128 or QB_C64");
+    if (n_global < 1 || n_global > 4 || world != (1 << n_global) || rank < 0 || rank >= world) return fail(QB_ERR_INVALID, "bad rank layout");
+    if (n_local < n_global + 1 || n_local > 36) return fail(QB_ERR_INVALID, "n_local out of range (the in-place exchange needs n_local >= n_global + 1)");
+    qb::SwapInplaceArgs args{};
+    uint64_t seen = 0;
+    for (int j = 0; j < n_global; ++j) {
+        const int p = local_positions[j];
+        if (p < 0 || p >= n_local || ((seen >> p) & 1) || (j && p <= local_positions[j - 1])) return fail(QB_ERR_INVALID, "local positions must be distinct, ascending and below n_local");
+        seen |= 1ull << p;
+        args.lpmask |= 1ull << p;
+        args.rbits |= uint64_t((rank >> j) & 1) << p;
+    }
+    for (int r = 0; r < world; ++r) {
+        if (!shard_states[r]) return fail(QB_ERR_INVALID, "null shard buffer");
+        args.state[r] = shard_states[r];
+    }
+    // the owner bit: the highest local position not exchanged (exists because n_local > n_global).  Any such bit partitions the
+    // pairs; a high one keeps neighbouring pair numbers on neighbouring amplitudes (bit 0 would halve every sector's use).
+    int p0 = n_local - 1;
+    while ((seen >> p0) & 1) --p0;
+    int s = 0;  // merge p0 into the ascending lp
+    for (; s < n_global && local_positions[s] < p0; ++s) args.ins_pos[s] = local_positions[s], args.ins_src[s] = s;
+    args.ins_pos[s] = p0, args.ins_src[s] = n_global;
+    for (int j = s; j < n_global; ++j) args.ins_pos[j + 1] = local_positions[j], args.ins_src[j + 1] = j;
+    args.g = n_global, args.rank = rank;
+    args.run_bits = std::min(qb::kSwapRunBits, n_local - n_global - 1);
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    QB_ON_DEVICE(ctx);
+    const uint64_t items = uint64_t(world - 1) << (n_local - n_global - 1);
+    const int blocks = int(std::min<uint64_t>(uint64_t(ctx->sm_count) * 8, std::max<uint64_t>(1, items / (256 * qb::kInplaceUnroll))));
+    return with_dtype(dtype, [&](auto t) {
+        using C = typename qb::Cx<decltype(t)>::type;
+        qb::swap_inplace_p2p_kernel<C><<<blocks, 256, 0, ctx->stream>>>(args, items);
+        return check_launch(ctx, "swap_inplace_p2p_kernel");
+    });
+}
+
 int qb_evaluate_expectation_submit(qb_context* ctx, int batch, const int64_t* plan_ids, const double* params, const int64_t* param_offsets,
                                    int64_t ham_id) {
     if (!ctx || !plan_ids || !param_offsets) return fail(QB_ERR_INVALID, "null argument");

@@ -13,6 +13,7 @@
 //   cvar_select_kernel / cvar_select_reduce_kernel  K8  one radix-digit pass of the exact CVaR of a sharded state (weighted select)
 //   top_select_kernel / top_collect_kernel  K9  most probable basis states: counts-only radix select of (~bits(p), logical k), ordered collect
 //   swap_p2p_kernel            global <-> local qubit swap of a sharded state fused with its all-to-all (peer-memory stores)
+//   swap_inplace_p2p_kernel    the same exchange in place, one buffer per rank (pairs swapped by peer loads + stores)
 //
 // What the arithmetic follows ([upstream] = un-vendored qiskit 2.4.2, see oracle/qiskit_semantics.py):
 //   gate matrices   UGate / CU3Gate as emitted by evqe/quantum_circuit/quantum_gate.py:96-102, 157-165
@@ -1861,6 +1862,75 @@ swap_p2p_kernel(const C* __restrict__ src, SwapArgs args, uint64_t size) {
         for (int u = 0; u < kUnroll; ++u) {
             const uint64_t t = t0 + u * stride;
             if (t < size) static_cast<C*>(args.peer[dst[u]])[(at[u] & ~lpmask) | rbits] = v[u];
+        }
+    }
+}
+
+// ---------------------------------------------------------------------------------------------------
+// The same exchange in place, one buffer per rank.  Swapping the g rank bits with the local bits lp is an involution: element i
+// of rank r whose lp bits read d != r trades places with element i' = (i & ~lpmask) | rbits(r) of rank d; elements with d == r
+// stay.  One thread swaps a pair (loads both, stores both crosswise); no other thread on any GPU touches those two addresses.
+// Pair ownership: p0 = the highest local bit not in lp is the same in i and i'; rank r handles the pair iff that bit is (r > d),
+// so exactly one of the two ranks does (a high owner bit keeps the accesses of neighbouring items contiguous).  Each rank moves half of its cross elements toward every peer: half of the bytes cross
+// NVLink as remote loads, half as remote stores, the same bytes per GPU and direction as swap_p2p_kernel.
+// ---------------------------------------------------------------------------------------------------
+struct SwapInplaceArgs {
+    void* state[kMaxSwapRanks];  // every rank's state buffer, peer-mapped (state[rank] = own)
+    uint64_t lpmask, rbits;      // exchanged local bits; this rank's bits dropped in at them
+    int32_t ins_pos[5];          // the g + 1 inserted bit positions (lp and p0), ascending
+    int32_t ins_src[5];          // bit of (d | owner << g) that goes to ins_pos[s]: j < g = bit j of d, g = the owner bit
+    int32_t g, rank;
+    int32_t run_bits;            // log2 of the run length, <= n_local - g - 1
+};
+
+// Remote loads have to cover the NVLink round trip with bytes in flight: twice the pairs per thread of swap_p2p_kernel's elements.
+constexpr int kInplaceUnroll = 8;
+
+// Work order (as in swap_p2p_kernel): items t < (W-1) 2^(n_local-g-1), run u = t >> run_bits goes to peer d = rank ^ (1 + u % (W-1)),
+// so at any item number the ranks target pairwise different peers and each rank rotates over all of its peers.  Within a peer
+// the pair number is ((u / (W-1)) << run_bits) | (t & run_mask), expanded to i by dropping in d's bits at lp and the owner bit at p0.
+template <typename C>
+__global__ void __launch_bounds__(256)
+swap_inplace_p2p_kernel(SwapInplaceArgs args, uint64_t items) {
+    const int g = args.g, rank = args.rank, rb = args.run_bits;
+    const uint32_t peers = (1u << g) - 1u;
+    const uint64_t run_mask = (1ull << rb) - 1ull;
+    C* __restrict__ own = static_cast<C*>(args.state[rank]);
+    auto locate = [&](uint64_t t, int& d) -> uint64_t {
+        const uint32_t u = uint32_t(t >> rb);  // < (W-1) 2^(n_local-g-1-run_bits) < 2^32 for n_local <= 36
+        const uint32_t k = 1u + u % peers;
+        d = rank ^ int(k);
+        const uint32_t bits = uint32_t(d) | (uint32_t(rank > d) << g);
+        uint64_t i = (uint64_t(u / peers) << rb) | (t & run_mask);
+        for (int s = 0; s <= g; ++s) {  // ascending: open a gap at each inserted position and drop its bit in
+            const int p = args.ins_pos[s];
+            i = ((i >> p) << (p + 1)) | (i & ((1ull << p) - 1ull)) | (uint64_t((bits >> args.ins_src[s]) & 1u) << p);
+        }
+        return i;
+    };
+    const uint64_t stride = uint64_t(gridDim.x) * blockDim.x;
+    for (uint64_t t0 = blockIdx.x * uint64_t(blockDim.x) + threadIdx.x; t0 < items; t0 += stride * kInplaceUnroll) {
+        C a[kInplaceUnroll], b[kInplaceUnroll];
+        C* there[kInplaceUnroll];
+        uint64_t at[kInplaceUnroll];
+#pragma unroll
+        for (int u = 0; u < kInplaceUnroll; ++u) {
+            const uint64_t t = t0 + u * stride;
+            if (t < items) {
+                int d;
+                at[u] = locate(t, d);
+                there[u] = static_cast<C*>(args.state[d]) + ((at[u] & ~args.lpmask) | args.rbits);
+                a[u] = __ldcg(own + at[u]);
+                b[u] = __ldcg(there[u]);
+            }
+        }
+#pragma unroll
+        for (int u = 0; u < kInplaceUnroll; ++u) {
+            const uint64_t t = t0 + u * stride;
+            if (t < items) {
+                own[at[u]] = b[u];
+                *there[u] = a[u];
+            }
         }
     }
 }

@@ -646,6 +646,15 @@ class Engine:
         lp = np.asarray(list(local_positions), dtype=np.int32)
         _native.check(self._lib.qb_swap_global_p2p(self._ctx, _dtype_code(dtype), int(n_local), c_void_p(state_ptr), _native.ptr(ptrs), world, int(rank), len(lp), _native.ptr(lp)))
 
+    def swap_global_inplace_p2p(self, dtype, n_local: int, shard_ptrs: Sequence[int], rank: int, local_positions: Sequence[int]):
+        """Launch the in-place exchange kernel on every rank's state buffer ``shard_ptrs`` (one buffer per rank; asynchronous on the
+        engine's stream; the caller owns the before / after barriers of include/queasars_b200.h)."""
+        world = len(shard_ptrs)
+        ptrs = np.asarray([int(p) for p in shard_ptrs], dtype=np.uint64)
+        lp = np.asarray(list(local_positions), dtype=np.int32)
+        _native.check(self._lib.qb_swap_global_inplace_p2p(self._ctx, _dtype_code(dtype), int(n_local), _native.ptr(ptrs), world, int(rank), len(lp),
+                                                           _native.ptr(lp)))
+
     # ------------------------------------------------------------------ device memory / peer mapping (sharded states)
     def device_alloc(self, nbytes: int) -> int:
         out = c_void_p()

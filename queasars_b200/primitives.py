@@ -392,7 +392,8 @@ class _B200Primitive:
 
     def _sharded_state(self, n_qubits: int):
         """One state of ``n_qubits`` sharded over the largest power-of-two prefix of the device set (kept between calls: two
-        shard-sized buffers per GPU).  BASELINE config C5: 35 qubits over 8 GPUs."""
+        shard-sized buffers per GPU where they fit, one otherwise -- the in-place exchange).  BASELINE config C5: 35 qubits over
+        8 GPUs; one buffer per GPU reaches 34 qubits on 2 GPUs and 36 on 8."""
         from .sharded import LocalShardedStatevector
 
         if self.dtype != "complex128":
@@ -412,7 +413,14 @@ class _B200Primitive:
             for old in self._sharded_obj.values():  # one resident sharded state at a time: they are sized for most of the memory
                 old.close()
             self._sharded_obj.clear()
-        sv = LocalShardedStatevector(n_qubits, engines[:count], min_local=min(12, n_qubits - int(np.log2(count))))
+        try:
+            sv = LocalShardedStatevector(n_qubits, engines[:count], min_local=min(12, n_qubits - int(np.log2(count))), buffers=None)
+        except _native.QbError as exc:
+            if exc.code != _native.QB_ERR_MEMORY:
+                raise
+            shard = 16 << (n_qubits - int(np.log2(count)))
+            raise ValueError(f"a {n_qubits}-qubit statevector sharded over {count} GPUs needs at least one {shard} byte buffer "
+                             f"({shard / 2**30:.0f} GiB) per GPU, which does not fit: {exc}") from exc
         with self._lock:
             self._sharded_obj[n_qubits] = sv
         return sv

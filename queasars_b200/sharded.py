@@ -10,10 +10,15 @@ bit position p < n-g is local, p >= n-g is a rank bit.  Logical qubits are track
     (``qb_apply_plan_device`` with ``index_offset = rank << n_local``: a control or diagonal target on a rank bit is
     a per-shard predicate, no communication);
   * before a gate that *targets* a rank bit, all g rank bits are exchanged with g local positions whose qubits are
-    needed latest.  On GPUs the exchange is ONE kernel per shard (``qb_swap_global_p2p``): it streams the shard once and
-    stores every amplitude straight into the GPU that owns it afterwards, at its final index, through peer-mapped
-    buffers over NVLink 5 / NVSwitch -- the all-to-all is fused into the permutation, there is no pack pass, no staging
-    copy and no unpack pass.  Two buffers of shard size are used in ping-pong.
+    needed latest.  On GPUs the exchange is ONE kernel per shard, fused with its all-to-all through peer-mapped buffers
+    over NVLink 5 / NVSwitch -- there is no pack pass, no staging copy and no unpack pass.  Two modes, chosen when the
+    state is built (``buffers``):
+      - two shard-sized buffers per GPU in ping-pong (``qb_swap_global_p2p``): the kernel streams the shard once and
+        stores every amplitude straight into the GPU that owns it afterwards, at its final index, in that GPU's idle spare;
+      - ONE buffer per GPU (``qb_swap_global_inplace_p2p``): the exchange is an involution, so every pair of amplitudes
+        that trade places is swapped in place by one of its two GPUs (a peer load and a peer store).  Same NVLink bytes,
+        half the memory: the widest state a device set holds grows by one qubit (34 on 2 GPUs, 36 on 8).
+    ``buffers=None`` takes two buffers where they fit and one otherwise.
 
 Two drivers share the schedule (``_ShardedLogic``):
 
@@ -27,7 +32,7 @@ Two drivers share the schedule (``_ShardedLogic``):
                                ``cudaDeviceEnablePeerAccess`` instead of IPC, reductions on the host.
 
 The shard-local arithmetic is delegated to a *backend* object (``apply``, ``diagonal_expectation``, ``pauli_expectation``,
-``sample``, ``cvar_select``, ``top_select``, ``top_collect``, ``swap_p2p``); the product default drives the CUDA engine.  Tests inject a NumPy backend to exercise the
+``sample``, ``cvar_select``, ``top_select``, ``top_collect``, ``swap_p2p``, ``swap_inplace_p2p``); the product default drives the CUDA engine.  Tests inject a NumPy backend to exercise the
 multi-rank host logic on CPU with the gloo backend.
 """
 from __future__ import annotations
@@ -38,6 +43,7 @@ from typing import Optional, Sequence
 
 import numpy as np
 
+from . import _native
 from .gate_list import DENSE, GateList, KernelOp
 
 
@@ -141,6 +147,13 @@ class CudaShardBackend:
         self.engine.swap_global_p2p("complex128", n_local, _state_ptr(state), peer_ptrs, rank, local_positions)
         self.engine.synchronize()
 
+    def swap_inplace_p2p(self, state, shard_ptrs: Sequence[int], n_local: int, rank: int, local_positions: Sequence[int]) -> None:
+        """The same exchange in place on every rank's ONE state buffer (``shard_ptrs``, peer-mapped); returns when this rank's
+        loads and stores have completed.  The caller runs the cross-rank barriers before and after (include/queasars_b200.h)."""
+        self._join_torch_stream(state)
+        self.engine.swap_global_inplace_p2p("complex128", n_local, shard_ptrs, rank, local_positions)
+        self.engine.synchronize()
+
 
 class _ShardedLogic:
     """Placement-independent part: qubit permutation, segmenting of a gate list into shard-local runs separated by global
@@ -167,6 +180,7 @@ class _ShardedLogic:
         self.bytes_sent = 0
         self._fresh = True
         self.swap_fallback_reason: Optional[str] = None
+        self.buffers = 2  # shard-sized buffers per shard: 2 = ping-pong exchange, 1 = in-place exchange
 
     def reset(self) -> None:
         """Forget the current state: the next ``run`` starts from |0...0> with the identity qubit placement."""
@@ -302,11 +316,12 @@ class _ShardedLogic:
         as it holds one entry.  Logical index bits are read from their physical positions: no data moves.  The first pass
         stores (p, E) of every entry in the idle spare buffer, the later ones read it from there.  Every rank makes the same
         decisions from the same all-gathered numbers, so every caller gets the same result.  ``cache=False`` recomputes p and E
-        from the state on every pass instead (same values)."""
+        from the state on every pass instead (same values); so does a state with one buffer per shard, which has no spare."""
         from . import expectation as ex
         from .engine import merge_duplicate_terms
 
         ex.check_alpha(alpha)
+        cache = cache and self.buffers == 2
         _, zs, cs = merge_duplicate_terms(np.zeros(len(z_masks), dtype=np.uint64), np.asarray(z_masks, dtype=np.uint64), np.asarray(coeffs, dtype=np.float64))
         phys = np.asarray([self._physical_mask(z) for z in zs], dtype=np.uint64)
         cf = np.ascontiguousarray(np.real(cs), dtype=np.float64)
@@ -423,13 +438,52 @@ class _ShardedLogic:
 
     def describe(self) -> dict:
         return {"n_qubits": self.n_qubits, "shards": self.world, "n_local": self.n_local, "swaps_done": self.swaps_done, "swap_path": self.swap_path,
-                "swap_fallback_reason": self.swap_fallback_reason}
+                "swap_fallback_reason": self.swap_fallback_reason, "buffers": self.buffers}
 
     def _logical_from_physical(self, full: np.ndarray) -> np.ndarray:
         n = self.n_qubits
         # physical axis a <-> physical bit n-1-a ; logical bit q lives at physical position[q]
         perm = [n - 1 - self.position[q] for q in range(n - 1, -1, -1)]
         return np.ascontiguousarray(full.reshape((2,) * n).transpose(perm)).reshape(-1)
+
+
+def _check_buffers(buffers) -> None:
+    if buffers not in (None, 1, 2):
+        raise ValueError(f"buffers must be None (two where they fit, else one), 1 or 2, not {buffers!r}")
+
+
+def _out_of_memory(exc: BaseException) -> bool:
+    return isinstance(exc, _native.QbError) and exc.code == _native.QB_ERR_MEMORY
+
+
+def _allocate_set(engines: Sequence, size: int) -> list:
+    """One shard buffer of ``size`` amplitudes per engine; what was allocated is freed again when one allocation fails."""
+    bufs = []
+    try:
+        for e in engines:
+            bufs.append(_DeviceBuffer(e, size))
+    except BaseException:
+        for b in bufs:
+            b.free()
+        raise
+    return bufs
+
+
+def _allocate_sets(engines: Sequence, size: int, buffers) -> list:
+    """[first set] or [first set, second set] of shard buffers: ``buffers`` = 1 / 2 forces the count; None takes the second set
+    when it fits (an allocation failing with QB_ERR_MEMORY frees the partial set and keeps one; any other error is raised)."""
+    sets = [_allocate_set(engines, size)]
+    if buffers == 1:
+        return sets
+    try:
+        sets.append(_allocate_set(engines, size))
+    except Exception as exc:  # noqa: BLE001
+        if buffers is None and _out_of_memory(exc):
+            return sets
+        for b in sets[0]:
+            b.free()
+        raise
+    return sets
 
 
 class _DeviceBuffer:
@@ -455,10 +509,15 @@ class _DeviceBuffer:
 class ShardedStatevector(_ShardedLogic):
     """One process per GPU / rank; collectives over ``torch.distributed`` (NCCL on GPUs, gloo in the CPU tests)."""
 
-    def __init__(self, n_qubits: int, backend=None, group=None, device=None, min_local: int = 12):
+    def __init__(self, n_qubits: int, backend=None, group=None, device=None, min_local: int = 12, buffers: Optional[int] = None):
+        """``buffers``: shard-sized buffers per rank where the ranks map each other's memory -- 2 (ping-pong exchange), 1 (in-place
+        exchange: one qubit wider for the same memory) or None (two where every rank can allocate them, else one; the ranks agree).
+        The pack + all-to-all route (``QB_SWAP=nccl``, no CUDA IPC, CPU tensors) stages through a spare: it always has two, and
+        ``buffers=1`` there raises ValueError on every rank."""
         import torch
         import torch.distributed as dist
 
+        _check_buffers(buffers)
         self._torch, self._dist = torch, dist
         self.group = group
         world = dist.get_world_size(group) if dist.is_initialized() else 1
@@ -480,30 +539,48 @@ class ShardedStatevector(_ShardedLogic):
         if want_p2p and os.environ.get("QB_SWAP", "p2p") == "nccl":
             want_p2p, self.swap_fallback_reason = False, "QB_SWAP=nccl"
         if want_p2p:
-            self._setup_ipc_buffers(size)
+            self._setup_ipc_buffers(size, buffers)
         if self._peer_ptrs is None:
+            if buffers == 1 and self.world > 1:  # the same decision on every rank: nothing has been allocated
+                reason = self.swap_fallback_reason or f"shards on {self.device.type} with {type(backend).__name__}"
+                raise ValueError("one buffer per shard needs the in-place exchange over peer-mapped memory; this state has none "
+                                 f"({reason}): the pack + all-to-all route stages through a second buffer")
             self.state = torch.zeros(size, dtype=torch.complex128, device=self.device)
-            self.spare = torch.empty(size, dtype=torch.complex128, device=self.device)
+            self.spare = None if buffers == 1 else torch.empty(size, dtype=torch.complex128, device=self.device)
+            self.buffers = 1 if buffers == 1 else 2
 
-    def _setup_ipc_buffers(self, size: int) -> None:
-        """Shard buffers = cudaMalloc allocations of this rank's engine; every rank maps every other rank's buffers through
-        CUDA IPC handles (all-gathered).  All ranks must agree on the outcome, so failures are all-reduced."""
-        torch, dist = self._torch, self._dist
+    def _map_ipc_buffers(self, size: int, buffers: Optional[int]):
+        """Allocate this rank's shard buffers (``_allocate_sets``), agree on their count over all ranks (the least count any rank
+        got: every rank runs the same exchange), and map every other rank's buffers through CUDA IPC handles (all-gathered).
+        -> (own buffers, peer[i][r] = address of rank r's buffer i in this process), or None when any rank failed (the reason is
+        kept in ``swap_fallback_reason``; everything is released again).  All ranks take the same outcome."""
+        dist = self._dist
         engine = self.backend.engine
         error, bufs, handles = None, [], []
         try:
-            bufs = [_DeviceBuffer(engine, size) for _ in range(2)]
-            handles = [engine.ipc_export(b.ptr) for b in bufs]
+            bufs = [s[0] for s in _allocate_sets([engine], size, buffers)]
         except Exception as exc:  # noqa: BLE001
             error = repr(exc)
+        counts = [None] * self.world
+        dist.all_gather_object(counts, (error, len(bufs)), group=self.group)
+        failed = [e for e, _ in counts if e]
+        count = min(n for _, n in counts)
+        for b in bufs[count:]:  # another rank could not allocate its second buffer
+            b.free()
+        bufs = bufs[:count]
+        if not failed:
+            try:
+                handles = [engine.ipc_export(b.ptr) for b in bufs]
+            except Exception as exc:  # noqa: BLE001
+                error = repr(exc)
         gathered = [None] * self.world
         dist.all_gather_object(gathered, (error, handles), group=self.group)
-        failed = [e for e, _ in gathered if e]
-        peer = [[0] * self.world for _ in range(2)]
+        failed = failed or [e for e, _ in gathered if e]
+        peer = [[0] * self.world for _ in range(count)]
         if not failed:
             try:
                 for r, (_, hs) in enumerate(gathered):
-                    for i in range(2):
+                    for i in range(count):
                         if r == self.rank:
                             peer[i][r] = bufs[i].ptr
                         else:
@@ -524,11 +601,21 @@ class ShardedStatevector(_ShardedLogic):
             self._mapped = []
             for b in bufs:
                 b.free()
+            return None
+        return bufs, peer
+
+    def _setup_ipc_buffers(self, size: int, buffers: Optional[int]) -> None:
+        """Shard buffers = cudaMalloc allocations of this rank's engine, mapped into every other rank (``_map_ipc_buffers``)."""
+        torch, dist = self._torch, self._dist
+        mapped = self._map_ipc_buffers(size, buffers)
+        if mapped is None:
             return
+        bufs, peer = mapped
         self._owned = bufs
         tensors = [torch.as_tensor(b, device=self.device) for b in bufs]
         self._peer_ptrs = {t.data_ptr(): peer[i] for i, t in enumerate(tensors)}
-        self.state, self.spare = tensors
+        self.state, self.spare = tensors[0], (tensors[1] if len(tensors) == 2 else None)
+        self.buffers = len(tensors)
         self.state.zero_()
         torch.cuda.synchronize(self.device)
         dist.barrier(group=self.group)
@@ -551,7 +638,9 @@ class ShardedStatevector(_ShardedLogic):
     def swap_path(self) -> str:
         if self.world == 1:
             return "none (one shard)"
-        return "swap_p2p_kernel over CUDA-IPC-mapped peer buffers" if self._peer_ptrs is not None else "pack + all_to_all_single + unpack"
+        if self._peer_ptrs is None:
+            return "pack + all_to_all_single + unpack"
+        return ("swap_p2p_kernel" if self.buffers == 2 else "swap_inplace_p2p_kernel") + " over CUDA-IPC-mapped peer buffers"
 
     @property
     def index_offset(self) -> int:
@@ -563,6 +652,13 @@ class ShardedStatevector(_ShardedLogic):
     def _swap(self, lp: list) -> None:
         g, nl = self.n_global, self.n_local
         torch, dist = self._torch, self._dist
+        if self._peer_ptrs is not None and self.buffers == 1:
+            # the in-place kernel reads and writes the peers' live states: every rank's earlier work has to be complete first
+            torch.cuda.synchronize(self.device)
+            dist.barrier(group=self.group)
+            self.backend.swap_inplace_p2p(self.state, self._peer_ptrs[self.state.data_ptr()], nl, self.rank, lp)
+            dist.barrier(group=self.group)  # every rank's pairs have been swapped before anyone reads its shard
+            return
         if self._peer_ptrs is not None:
             # one kernel: every amplitude goes straight to the rank that owns it afterwards, at its final index
             self.backend.swap_p2p(self.state, self._peer_ptrs[self.spare.data_ptr()], nl, self.rank, lp)
@@ -665,14 +761,18 @@ class ShardedStatevector(_ShardedLogic):
 
 class LocalShardedStatevector(_ShardedLogic):
     """ONE process, all shards: ``engines[r]`` (one per shard; the same engine may appear several times -- several shards on one
-    GPU, used by the single-GPU tests) owns shard r's two buffers.  Shard-local work of all devices runs concurrently on one
-    worker thread per shard (the native calls release the GIL); the swap kernel of every device stores into the other devices'
+    GPU, used by the single-GPU tests) owns shard r's buffers.  Shard-local work of all devices runs concurrently on one
+    worker thread per shard (the native calls release the GIL); the swap kernel of every device reaches the other devices'
     buffers through peer access (``cudaDeviceEnablePeerAccess``); reductions happen on the host.  This is what the evaluators
-    use for circuits too wide for one GPU."""
+    use for circuits too wide for one GPU.
 
-    def __init__(self, n_qubits: int, engines: Sequence, min_local: int = 12):
+    ``buffers``: shard-sized buffers per shard -- 2 (ping-pong exchange), 1 (in-place exchange) or None (two where they can be
+    allocated, else one)."""
+
+    def __init__(self, n_qubits: int, engines: Sequence, min_local: int = 12, buffers: Optional[int] = None):
         from concurrent.futures import ThreadPoolExecutor
 
+        _check_buffers(buffers)
         engines = list(engines)
         self._init_logic(n_qubits, len(engines), min_local)
         self.engines = engines
@@ -682,13 +782,16 @@ class LocalShardedStatevector(_ShardedLogic):
             for d in set(devices):
                 e.enable_peer_access(d)  # raises (with the reason) when the GPUs cannot map each other's memory
         size = 1 << self.n_local
-        self._bufs = [[_DeviceBuffer(e, size) for e in engines] for _ in range(2)]  # [which][shard]
+        self._bufs = _allocate_sets(engines, size, buffers)  # [which][shard]
+        self.buffers = len(self._bufs)
         self._cur = 0
         self._pool = ThreadPoolExecutor(max_workers=len(engines), thread_name_prefix="qb-shard") if len(engines) > 1 else None
 
     @property
     def swap_path(self) -> str:
-        return "none (one shard)" if self.world == 1 else "swap_p2p_kernel over peer access (one process)"
+        if self.world == 1:
+            return "none (one shard)"
+        return ("swap_p2p_kernel" if self.buffers == 2 else "swap_inplace_p2p_kernel") + " over peer access (one process)"
 
     def close(self):
         for e in set(self.engines):
@@ -729,6 +832,14 @@ class LocalShardedStatevector(_ShardedLogic):
         self._each(lambda r: self.backends[r].apply(self._state(r), segment, params, self.n_local, n_params, r << self.n_local, fresh))
 
     def _swap(self, lp: list) -> None:
+        if self.buffers == 1:
+            states = [self._state(r) for r in range(self.world)]
+            # the in-place kernel reads and writes the peers' live states: every shard's earlier work is complete before any
+            # shard launches (the join of the synchronisations), and every shard's pairs are swapped before anyone reads its
+            # shard again (swap_inplace_p2p returns once its kernel completed, _each joins all of them)
+            self._each(lambda r: self.engines[r].synchronize())
+            self._each(lambda r: self.backends[r].swap_inplace_p2p(states[r], states, self.n_local, r, lp))
+            return
         dst = [self._bufs[1 - self._cur][r].ptr for r in range(self.world)]
         # every shard's kernel stores into all destination buffers; swap_p2p returns once its own stores completed, and _each
         # joins all of them: the barrier of the multi-process driver
@@ -743,8 +854,8 @@ class LocalShardedStatevector(_ShardedLogic):
         return np.asarray(self._each(lambda r: self.backends[r].diagonal_expectation(self._state(r), z, c, self.n_qubits, self.n_local, r << self.n_local)))
 
     def _select_pass(self, z_masks, coeffs, cache_mode: int, spec) -> list:
-        spare = self._bufs[1 - self._cur]
-        return self._each(lambda r: self.backends[r].cvar_select(self._state(r), spare[r].ptr, cache_mode, z_masks, coeffs, self.n_qubits, self.n_local,
+        spare = [b.ptr for b in self._bufs[1 - self._cur]] if self.buffers == 2 else [None] * self.world  # one buffer: no cache
+        return self._each(lambda r: self.backends[r].cvar_select(self._state(r), spare[r], cache_mode, z_masks, coeffs, self.n_qubits, self.n_local,
                                                                  r << self.n_local, spec))
 
     def _top_pass(self, sel, positions, min_probability) -> list:
