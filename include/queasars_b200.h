@@ -137,7 +137,8 @@ int qb_plan_destroy(qb_context* ctx, int64_t plan_id);
  * ONE circuit whose leading layers are bound numerically and only one layer's parameters change): `plan_id` (compiled
  * for application to an existing state, no parameters in the prefix) starts from the state produced by the
  * parameter-free plan `prefix_plan_id` instead of |0...0>.  The prefix state is computed once, on first use, and kept on
- * the device (16 B * 2^n) until the plan is destroyed. */
+ * the device (16 B * 2^n) until the plan is destroyed.  Every later evaluation of `plan_id` starts from the new prefix,
+ * including the single-circuit calls of an earlier cached graph and the resident batches that contain it. */
 int qb_plan_set_prefix(qb_context* ctx, int64_t plan_id, int64_t prefix_plan_id);
 
 /* --- Hamiltonians ---------------------------------------------------------------------------------------
@@ -272,7 +273,9 @@ int qb_evaluate_expectation_collect(qb_context* ctx, int total, double* out_valu
 
 /* --- resident batches (benchmarks, optimizer inner loops) ---------------------------------------------
  * Same work as qb_evaluate_expectation split into its host<->device and device-only parts so the
- * device-resident throughput can be timed separately from the end-to-end call. */
+ * device-resident throughput can be timed separately from the end-to-end call.  After one of its plans or its Hamiltonian is
+ * destroyed, set_params / run / run_timed / read of a batch return QB_ERR_NOT_FOUND and launch nothing; after one of its
+ * plans is given a prefix (qb_plan_set_prefix) they use the new start, and parameters uploaded before stay valid. */
 int qb_batch_create(qb_context* ctx, int batch, const int64_t* plan_ids, int64_t ham_id, int64_t* batch_id);
 int qb_batch_set_params(qb_context* ctx, int64_t batch_id, const double* params, const int64_t* param_offsets);
 int qb_batch_run(qb_context* ctx, int64_t batch_id);   /* asynchronous on the context's stream */

@@ -161,6 +161,7 @@ struct DeviceBatch {
     std::vector<int64_t> param_begin;  // per caller index, offset into the params buffer
     int64_t total_params = 0, total_ops = 0;
     const Ham* ham = nullptr;
+    int64_t ham_id = 0;  // resident batches: the Hamiltonian is looked up again by id whenever the batch is re-assembled
     // what the buffers were last assembled for: an identical request (same plans, Hamiltonian, start) re-uses them as they are
     std::vector<int64_t> built_ids;
     uint64_t built_epoch = 0, built_offset = 0;
@@ -1452,6 +1453,9 @@ int qb_plan_set_prefix(qb_context* ctx, int64_t plan_id, int64_t prefix_plan_id)
     if (pl->has_init) return fail(QB_ERR_INVALID, "a prefixed plan must be compiled for application to an existing state");
     if (pre->n_params != 0 || pre->prefix_id || pre->n_eff != pl->n_eff || pre->dtype != pl->dtype || pre->n_qubits != pl->n_qubits)
         return fail(QB_ERR_INVALID, "prefix plan must be parameter-free, un-prefixed and of the same shape");
+    QB_ON_DEVICE(ctx);
+    cudaStreamSynchronize(ctx->stream);
+    drop_single_graphs(ctx, plan_id, 0);  // a cached graph of this plan starts it from |0...0>, not from the prefix state
     pl->prefix_id = prefix_plan_id;
     pl->prefix_ready = false;
     ctx->epoch++;  // assembled batches may hold this plan's old start
@@ -1711,6 +1715,7 @@ int qb_batch_create(qb_context* ctx, int batch, const int64_t* plan_ids, int64_t
         if (!ham) return fail(QB_ERR_NOT_FOUND, "unknown Hamiltonian id");
     }
     auto b = std::make_unique<DeviceBatch>();
+    b->ham_id = ham_id;
     QB_TRY(build_batch(ctx, *b, batch, plan_ids, ham, nullptr, 1, 0));
     *batch_id = ctx->next_id++;
     ctx->batches[*batch_id] = std::move(b);
@@ -1722,12 +1727,34 @@ static DeviceBatch* find_batch(qb_context* ctx, int64_t id) {
     return it == ctx->batches.end() ? nullptr : it->second.get();
 }
 
+// The resident batch `id`, re-assembled first when a plan or Hamiltonian was destroyed or a plan given a prefix since it was
+// built (its entries may point into freed device memory or miss the new start): QB_ERR_NOT_FOUND, before anything is launched,
+// when one of its plans or its Hamiltonian is gone.  The parameter layout depends on the plans alone, so uploaded parameters
+// stay valid across a re-assembly.
+static int current_batch(qb_context* ctx, int64_t id, DeviceBatch** out) {
+    DeviceBatch* b = find_batch(ctx, id);
+    if (!b) return fail(QB_ERR_NOT_FOUND, "unknown batch id");
+    if (b->built_epoch != ctx->epoch) {
+        const Ham* ham = nullptr;
+        if (b->ham_id && !(ham = find_ham(ctx, b->ham_id)))
+            return fail(QB_ERR_NOT_FOUND, "Hamiltonian " + std::to_string(b->ham_id) + " of the batch no longer exists");
+        const std::vector<int64_t> ids = b->built_ids;  // (build_batch clears built_ids before it reads the list)
+        const int rc = build_batch(ctx, *b, int(ids.size()), ids.data(), ham, nullptr, 1, 0);
+        if (rc != QB_OK) {
+            b->built_ids = ids;  // still stale (built_epoch is unchanged): the next call tries again and fails the same way
+            return rc;
+        }
+    }
+    *out = b;
+    return QB_OK;
+}
+
 int qb_batch_set_params(qb_context* ctx, int64_t batch_id, const double* params, const int64_t* param_offsets) {
     if (!ctx || !param_offsets) return fail(QB_ERR_INVALID, "null argument");
     std::lock_guard<std::mutex> lock(ctx->mu);
     QB_ON_DEVICE(ctx);
-    DeviceBatch* b = find_batch(ctx, batch_id);
-    if (!b) return fail(QB_ERR_NOT_FOUND, "unknown batch id");
+    DeviceBatch* b = nullptr;
+    QB_TRY(current_batch(ctx, batch_id, &b));
     return batch_upload_params(ctx, *b, params, param_offsets);
 }
 
@@ -1735,8 +1762,8 @@ int qb_batch_run(qb_context* ctx, int64_t batch_id) {
     if (!ctx) return fail(QB_ERR_INVALID, "null context");
     std::lock_guard<std::mutex> lock(ctx->mu);
     QB_ON_DEVICE(ctx);
-    DeviceBatch* b = find_batch(ctx, batch_id);
-    if (!b) return fail(QB_ERR_NOT_FOUND, "unknown batch id");
+    DeviceBatch* b = nullptr;
+    QB_TRY(current_batch(ctx, batch_id, &b));
     const int64_t before = ctx->launches;
     QB_TRY(launch_circuits(ctx, *b, nullptr));
     if (b->ham) QB_TRY(launch_expectation(ctx, *b));
@@ -1748,8 +1775,8 @@ int qb_batch_run_timed(qb_context* ctx, int64_t batch_id, int max_launches, floa
     if (!ctx || !sweep_ms || !sweep_states || !n_launches) return fail(QB_ERR_INVALID, "null argument");
     std::lock_guard<std::mutex> lock(ctx->mu);
     QB_ON_DEVICE(ctx);
-    DeviceBatch* b = find_batch(ctx, batch_id);
-    if (!b) return fail(QB_ERR_NOT_FOUND, "unknown batch id");
+    DeviceBatch* b = nullptr;
+    QB_TRY(current_batch(ctx, batch_id, &b));
     if (max_launches < b->max_sweeps) return fail(QB_ERR_INVALID, "output arrays too small");
     std::vector<cudaEvent_t> events(2 * size_t(b->max_sweeps));
     for (auto& e : events) QB_CUDA(cudaEventCreate(&e));
@@ -1773,8 +1800,8 @@ int qb_batch_read(qb_context* ctx, int64_t batch_id, double* out_values) {
     if (!ctx || !out_values) return fail(QB_ERR_INVALID, "null argument");
     std::lock_guard<std::mutex> lock(ctx->mu);
     QB_ON_DEVICE(ctx);
-    DeviceBatch* b = find_batch(ctx, batch_id);
-    if (!b) return fail(QB_ERR_NOT_FOUND, "unknown batch id");
+    DeviceBatch* b = nullptr;
+    QB_TRY(current_batch(ctx, batch_id, &b));
     return batch_read(ctx, *b, out_values);
 }
 

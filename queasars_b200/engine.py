@@ -288,9 +288,11 @@ class Engine:
         if split < min_prefix_ops or split == len(gates.ops) or gates.n_params == 0:
             return self.compile(gates, dtype, defer=False)
         with self._lock:
-            if self._prefix_bytes + state_bytes > self._prefix_budget:
-                return self.compile(gates, dtype, defer=False)
-            self._prefix_bytes += state_bytes
+            fits = self._prefix_bytes + state_bytes <= self._prefix_budget
+            if fits:
+                self._prefix_bytes += state_bytes
+        if not fits:  # (compile takes the lock itself: not inside the block above)
+            return self.compile(gates, dtype, defer=False)
         try:
             prefix = self.compile(GateList(gates.n_qubits, list(gates.ops[:split]), 0, ()), dtype, from_zero_state=True, defer=False)
             suffix = self.compile(GateList(gates.n_qubits, list(gates.ops[split:]), gates.n_params, gates.param_names), dtype, from_zero_state=False, cache=False, defer=False)
