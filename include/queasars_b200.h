@@ -231,6 +231,15 @@ int qb_top_select_pick(qb_top_select* sel, const uint64_t counts[256]);
 int qb_top_states(qb_context* ctx, int batch, const int64_t* plan_ids, const double* params, const int64_t* param_offsets,
                   int64_t max_states, double min_probability, int64_t* out_counts, int64_t* out_indices, double* out_probs);
 
+/* Exact marginal probabilities without shots ([upstream] Statevector.probabilities(qargs)): out[i * 2^n_measured + b] = sum of
+ * |psi_i(k)|^2 over every basis index k whose bit qubits[j] equals bit j of b, for j < n_measured.  `qubits` are distinct qubits of
+ * the circuits, in any order, 1 <= n_measured <= 26.  The sums run in an order fixed by the qubits and the state width alone,
+ * without atomics: two calls on the same state give the same bits.  Plans must share the first one's width and dtype.
+ * QB_ERR_INVALID for a bad qubit list; QB_ERR_MEMORY when one statevector and its 2^n_measured doubles of output (and partial
+ * rows) do not fit the workspace. */
+int qb_marginal_probabilities(qb_context* ctx, int batch, const int64_t* plan_ids, const double* params, const int64_t* param_offsets,
+                              int n_measured, const int* qubits, double* out);
+
 /* --- observable sets ------------------------------------------------------------------------------------
  * Several observables H_j = sum_t c_{j,t} P_t evaluated on one simulated state (EstimatorV2 pubs with an array of observables).
  * Observable j owns the terms term_offsets[j] .. term_offsets[j+1]-1 of the mask / coefficient arrays (term_offsets[0] == 0).
@@ -334,6 +343,12 @@ int qb_top_select_device(qb_context* ctx, int dtype, int n_local, const void* d_
 int qb_top_collect_device(qb_context* ctx, int dtype, int n_local, const void* d_state, uint64_t index_offset, double min_probability,
                           const qb_top_select* sel, const int32_t* positions, int64_t capacity, int64_t* out_count, int64_t* out_indices,
                           double* out_probs);
+/* qb_marginal_probabilities on a caller-owned shard of 2^n_local amplitudes whose physical indices are `index_offset | k`:
+ * qubits[j] is the physical bit position (0..63, distinct) that becomes bit j of the output index.  Positions >= n_local are rank
+ * bits: their value comes from index_offset, so the shard's mass lands in the bins of its rank bits and the marginal of the
+ * whole state is the sum of the shards' outputs.  out: 2^n_measured doubles.  Synchronous. */
+int qb_marginal_device(qb_context* ctx, int dtype, int n_local, const void* d_state, uint64_t index_offset, int n_measured, const int* qubits,
+                       double* out);
 
 /* Global <-> local qubit swap of a state sharded over `world` = 2^n_global GPUs of one node (BASELINE config C5), fused with its
  * all-to-all: the calling rank streams its shard `d_state` once and stores every amplitude directly into the rank that owns it

@@ -10,7 +10,7 @@ Importing the package never touches CUDA; the first evaluation loads the native 
 it has not been built or no B200 is present (there is no CPU fallback).
 """
 from .bitstring_evaluation import BitstringEvaluator, BitstringEvaluatorException, DiagonalEnergyBitstringEvaluator  # noqa: F401
-from .circuit import CU3Gate, Parameter, QuantumCircuit, circuit_to_gate  # noqa: F401
+from .circuit import ClassicalRegister, Clbit, CU3Gate, Parameter, QuantumCircuit, circuit_to_gate  # noqa: F401
 from .operators import SparsePauliOp  # noqa: F401
 
 __all__ = [
@@ -18,6 +18,8 @@ __all__ = [
     "BitstringEvaluatorException",
     "DiagonalEnergyBitstringEvaluator",
     "QuantumCircuit",
+    "ClassicalRegister",
+    "Clbit",
     "Parameter",
     "CU3Gate",
     "circuit_to_gate",

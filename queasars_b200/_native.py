@@ -92,6 +92,8 @@ def _declare(lib):
         "qb_top_select_device": [c_void_p, c_int, c_int, c_void_p, c_uint64, c_double, P(TopSelect), c_void_p, c_void_p],
         "qb_top_collect_device": [c_void_p, c_int, c_int, c_void_p, c_uint64, c_double, P(TopSelect), c_void_p, c_int64, P(c_int64), c_void_p,
                                   c_void_p],
+        "qb_marginal_probabilities": [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p],
+        "qb_marginal_device": [c_void_p, c_int, c_int, c_void_p, c_uint64, c_int, c_void_p, c_void_p],
     }
     for name, argtypes in sigs.items():
         fn = getattr(lib, name)
@@ -117,7 +119,8 @@ EXPORTED_SYMBOLS = (
     "qb_batch_create qb_batch_set_params qb_batch_run qb_batch_run_timed qb_batch_read qb_batch_destroy qb_batch_stats "
     "qb_apply_plan_device qb_expectation_device qb_sample_device qb_cvar_select_device qb_swap_global_p2p qb_swap_global_inplace_p2p qb_record_sizes "
     "qb_device_alloc qb_device_free qb_device_read qb_enable_peer_access qb_ipc_export qb_ipc_open qb_ipc_close "
-    "qb_top_select_init qb_top_select_pick qb_top_states qb_top_select_device qb_top_collect_device"
+    "qb_top_select_init qb_top_select_pick qb_top_states qb_top_select_device qb_top_collect_device "
+    "qb_marginal_probabilities qb_marginal_device"
 ).split()
 
 

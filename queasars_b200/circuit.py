@@ -141,12 +141,52 @@ class Qubit:
         return f"Qubit({self._index})"
 
 
+class Clbit:
+    """A classical bit; the bits of a ``ClassicalRegister`` know their register and position in it."""
+
+    __slots__ = ("_register", "_index")
+
+    def __init__(self, register: "Optional[ClassicalRegister]" = None, index: Optional[int] = None):
+        self._register, self._index = register, index
+
+    def __repr__(self):
+        return f"Clbit({self._register.name if self._register is not None else None}, {self._index})"
+
+
+class ClassicalRegister:
+    """``qiskit.circuit.ClassicalRegister(size, name)``: ``size`` fresh clbits, indexable and iterable."""
+
+    _count = 0
+
+    def __init__(self, size: int, name: Optional[str] = None):
+        size = int(size)
+        if size < 0:
+            raise ValueError("a register's size must be non-negative")
+        if name is None:
+            name = f"c{ClassicalRegister._count}"
+            ClassicalRegister._count += 1
+        self.name, self.size = str(name), size
+        self._bits = [Clbit(self, i) for i in range(size)]
+
+    def __len__(self):
+        return self.size
+
+    def __getitem__(self, key):
+        return self._bits[key]
+
+    def __iter__(self):
+        return iter(self._bits)
+
+    def __repr__(self):
+        return f"ClassicalRegister({self.size}, '{self.name}')"
+
+
 class _BitLocation:
     __slots__ = ("index", "registers")
 
-    def __init__(self, index):
+    def __init__(self, index, registers=None):
         self.index = index
-        self.registers = []
+        self.registers = registers or []
 
 
 class Instruction:
@@ -198,18 +238,53 @@ _STANDARD_ARITY = {
 
 
 class QuantumCircuit:
-    def __init__(self, num_qubits: int, name: Optional[str] = None):
+    """``QuantumCircuit(num_qubits)``, ``QuantumCircuit(num_qubits, num_clbits)`` (clbits in one register "c") or
+    ``QuantumCircuit(num_qubits, *cregs)`` (``ClassicalRegister``s); a circuit without clbits has no classical registers."""
+
+    def __init__(self, num_qubits: int, *cregs, name: Optional[str] = None):
+        if len(cregs) == 1 and isinstance(cregs[0], str):  # QuantumCircuit(n, name): the earlier positional form
+            name, cregs = cregs[0], ()
         self.num_qubits = int(num_qubits)
         self.name = name or "circuit"
         self.qubits = [Qubit(i) for i in range(self.num_qubits)]
         self.data: list[CircuitInstruction] = []
         self.global_phase = 0.0
-        self.num_clbits = 0
+        self.cregs: list[ClassicalRegister] = []
+        self.clbits: list[Clbit] = []
+        self._clbit_index: dict = {}  # Clbit -> index in self.clbits
         self._b200_version = 0  # bumped by every in-place change that keeps len(data) (plan-cache fingerprint, primitives.py)
+        if len(cregs) == 1 and isinstance(cregs[0], numbers.Integral):
+            if int(cregs[0]) > 0:
+                self.add_register(ClassicalRegister(int(cregs[0]), "c"))
+        else:
+            for reg in cregs:
+                self.add_register(reg)
 
     # ------------------------------------------------------------------ inspection
-    def find_bit(self, bit: Qubit) -> _BitLocation:
+    @property
+    def num_clbits(self) -> int:
+        return len(self.clbits)
+
+    def find_bit(self, bit) -> _BitLocation:
+        """Index of a qubit, or index and (register, position) pairs of a clbit, like ``QuantumCircuit.find_bit``."""
+        if isinstance(bit, Clbit):
+            try:
+                index = self._clbit_index[bit]
+            except KeyError:
+                raise ValueError(f"{bit!r} is not in the circuit") from None
+            return _BitLocation(index, [(bit._register, bit._index)] if bit._register is not None else [])
         return _BitLocation(bit._index)
+
+    def add_register(self, register: ClassicalRegister) -> None:
+        if not isinstance(register, ClassicalRegister):
+            raise TypeError(f"expected a ClassicalRegister, got {type(register).__name__}")
+        if any(reg.name == register.name for reg in self.cregs):
+            raise ValueError(f'register name "{register.name}" already exists')
+        self.cregs.append(register)
+        for bit in register:
+            if bit not in self._clbit_index:
+                self._clbit_index[bit] = len(self.clbits)
+                self.clbits.append(bit)
 
     @property
     def parameters(self) -> list:
@@ -260,7 +335,34 @@ class QuantumCircuit:
             )
         if len({q._index for q in qubits}) != len(qubits):
             raise ValueError("duplicate qubit arguments")
-        self.data.append(CircuitInstruction(instruction, qubits, tuple(cargs)))
+        self.data.append(CircuitInstruction(instruction, qubits, tuple(self._clbit(c) for c in cargs)))
+        return self
+
+    def _clbit(self, c) -> Clbit:
+        if isinstance(c, Clbit):
+            if c not in self._clbit_index:
+                raise ValueError(f"{c!r} is not in the circuit")
+            return c
+        return self.clbits[int(c)]
+
+    def _bit_list(self, arg, resolve) -> list:
+        """One bit or a sequence of them (register, range, list), as ``measure`` accepts them."""
+        if isinstance(arg, (ClassicalRegister, range, list, tuple)):
+            return [resolve(a) for a in arg]
+        return [resolve(arg)]
+
+    def measure(self, qubit, cbit):
+        """Measure ``qubit`` into ``cbit``; each may be one bit or a sequence (a register, a range, a list).  One qubit and several
+        clbits measures it into each of them; otherwise the two sequences pair up and must have the same length (Qiskit's
+        broadcasting)."""
+        qubits = self._bit_list(qubit, self._qubit)
+        clbits = self._bit_list(cbit, self._clbit)
+        if len(qubits) == 1 and len(clbits) > 1:
+            qubits = qubits * len(clbits)
+        if len(qubits) != len(clbits):
+            raise ValueError(f"the amount of qubit({len(qubits)})/clbit({len(clbits)}) arguments does not match the gate expectation")
+        for q, c in zip(qubits, clbits):
+            self.data.append(CircuitInstruction(Instruction("measure", 1), [q], (c,)))
         return self
 
     def _std(self, name, qubits, params=()):
@@ -349,10 +451,16 @@ class QuantumCircuit:
         return self
 
     # ------------------------------------------------------------------ transformations
-    def copy(self, name: Optional[str] = None) -> "QuantumCircuit":
-        out = QuantumCircuit(self.num_qubits, name or self.name)
+    def _empty_like(self, name: Optional[str] = None) -> "QuantumCircuit":
+        """Same width, name, phase and classical registers (the same register and clbit objects, as Qiskit's ``copy``); no data."""
+        out = QuantumCircuit(self.num_qubits, name=name or self.name)
         out.global_phase = self.global_phase
-        out.num_clbits = self.num_clbits
+        for reg in self.cregs:
+            out.add_register(reg)
+        return out
+
+    def copy(self, name: Optional[str] = None) -> "QuantumCircuit":
+        out = self._empty_like(name)
         for inst in self.data:
             op = inst.operation
             new_op = type(op).__new__(type(op))
@@ -361,29 +469,45 @@ class QuantumCircuit:
         return out
 
     def measure_all(self, inplace: bool = True, add_bits: bool = True):
+        """Barrier, then every qubit i measured into clbit i of a new register "meas" (``add_bits``) or of the circuit's own clbits."""
         circ = self if inplace else self.copy()
+        if add_bits:
+            name = "meas"
+            if any(r.name == name for r in circ.cregs):  # (upstream: a fresh name with the same prefix)
+                name = f"meas{ClassicalRegister._count}"
+                ClassicalRegister._count += 1
+            reg = ClassicalRegister(circ.num_qubits, name)
+            circ.add_register(reg)
+            clbits = list(reg)
+        else:
+            if circ.num_clbits < circ.num_qubits:
+                raise ValueError("The number of classical bits must be equal or greater than the number of qubits.")
+            clbits = circ.clbits[: circ.num_qubits]
         circ.barrier()
-        for i, q in enumerate(circ.qubits):
-            circ.data.append(CircuitInstruction(Instruction("measure", 1), [q], (i,)))
-        circ.num_clbits = circ.num_qubits
+        circ.measure(list(range(circ.num_qubits)), clbits)
         return None if inplace else circ
 
-    def compose(self, other: "QuantumCircuit", qubits: Optional[Sequence[int]] = None, inplace: bool = False):
+    def compose(self, other: "QuantumCircuit", qubits: Optional[Sequence[int]] = None, clbits: Optional[Sequence[int]] = None,
+                inplace: bool = False):
+        """``other``'s instructions appended on ``qubits`` (default: the first ones) and its clbits mapped onto ``clbits`` (default: the
+        first ones) of this circuit, whose registers are kept."""
         if other.num_qubits > self.num_qubits:
             raise ValueError("Trying to compose with another QuantumCircuit which has more 'in' edges.")
+        if other.num_clbits > self.num_clbits:
+            raise ValueError("Trying to compose with another QuantumCircuit which has more 'out' edges.")
         dest = self if inplace else self.copy()
         mapping = list(range(other.num_qubits)) if qubits is None else [int(q) for q in qubits]
+        cmap = list(range(other.num_clbits)) if clbits is None else [dest.find_bit(dest._clbit(c)).index for c in clbits]
         for inst in other.copy().data:
             dest.data.append(
-                CircuitInstruction(inst.operation, [dest.qubits[mapping[q._index]] for q in inst.qubits], inst.clbits)
+                CircuitInstruction(inst.operation, [dest.qubits[mapping[q._index]] for q in inst.qubits],
+                                   tuple(dest.clbits[cmap[other.find_bit(c).index]] for c in inst.clbits))
             )
         dest.global_phase += other.global_phase
         return None if inplace else dest
 
     def decompose(self) -> "QuantumCircuit":
-        out = QuantumCircuit(self.num_qubits, self.name)
-        out.global_phase = self.global_phase
-        out.num_clbits = self.num_clbits
+        out = self._empty_like()
         for inst in self.copy().data:
             definition = inst.operation.definition
             if definition is None:

@@ -94,10 +94,22 @@ class PubResult:
 
 class SamplerPubResult(PubResult):
     def join_data(self, names=None):
+        """The registers ``names`` (default: all, in the data's order) joined into one, as upstream's
+        ``BitArray.concatenate_bits``: the first register's bits are the least significant."""
         keys = list(self.data.keys()) if names is None else list(names)
-        if len(keys) != 1:
-            raise NotImplementedError("join_data over several registers")
-        return self.data[keys[0]]
+        if not keys:
+            raise ValueError("join_data needs at least one register name")
+        regs = [self.data[k] for k in keys]
+        if len(regs) == 1:
+            return regs[0]
+        width = sum(r.num_bits for r in regs)
+        if width > 63:
+            raise NotImplementedError(f"joined registers of more than 63 bits are not supported (got {width})")
+        joined, shift = np.zeros(regs[0].indices.shape, dtype=np.int64), 0
+        for r in regs:
+            joined |= r.indices << shift
+            shift += r.num_bits
+        return ShotRegister(joined, width, regs[0].shape)
 
 
 class PrimitiveResult:

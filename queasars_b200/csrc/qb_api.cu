@@ -1213,6 +1213,67 @@ int check_top_shard(qb_context* ctx, int dtype, int n_local, const void* d_state
     return check_top_state(sel, positions, want_done);
 }
 
+// ---- exact marginal probabilities ----
+// The kernel arguments for measured bit positions pos[0..m) (distinct, below `limit`) of a state of 2^n_bits amplitudes whose
+// indices are index_offset | k: positions >= n_bits are rank bits and read their value from index_offset.  The slice count
+// (2^slice_bits items per measured-bit value) brings the items to about 2^kMargItemBits.
+int marginal_args(int n_bits, uint64_t index_offset, int m, const int* pos, int limit, qb::MarginalArgs* out) {
+    if (!pos) return fail(QB_ERR_INVALID, "null qubit list");
+    if (m < 1 || m > qb::kMargMaxBits) return fail(QB_ERR_INVALID, "n_measured must be in 1.." + std::to_string(qb::kMargMaxBits) + ", got " + std::to_string(m));
+    qb::MarginalArgs a{};
+    int out_of[64];
+    std::fill(out_of, out_of + 64, -1);
+    for (int j = 0; j < m; ++j) {
+        if (pos[j] < 0 || pos[j] >= limit || out_of[pos[j]] >= 0)
+            return fail(QB_ERR_INVALID, "measured qubits must be distinct and in 0.." + std::to_string(limit - 1));
+        out_of[pos[j]] = j;
+    }
+    for (int p = 0; p < 64; ++p) {
+        const int j = out_of[p];
+        if (p < 5) {
+            if (j >= 0) a.lane_bin[p] = 1u << j;
+            else if (p < n_bits) a.lane_sum |= 1u << p;
+        } else if (p < n_bits) {
+            if (j >= 0) a.h_pos[a.h_bits] = int8_t(p - 5), a.h_out[a.h_bits] = int8_t(j), ++a.h_bits;
+            else a.v_pos[a.v_bits] = int8_t(p - 5), a.v_mask |= 1u << (p - 5), ++a.v_bits;
+        } else if (j >= 0) {
+            a.bin_fixed |= uint32_t((index_offset >> p) & 1) << j;
+            a.fixed_mask |= 1u << j;
+        }
+    }
+    a.m = m;
+    a.slice_bits = std::min(a.v_bits, std::max(0, qb::kMargItemBits - a.h_bits));
+    *out = a;
+    return QB_OK;
+}
+
+// bytes of device scratch per state: the marginal, and the [bin][slice] partial rows when there are several slices
+size_t marginal_scratch_bytes(const qb::MarginalArgs& a) {
+    return (sizeof(double) << a.m) + (a.slice_bits ? sizeof(double) << (a.m + a.slice_bits) : 0);
+}
+
+// the marginals of `n` states (rows `stride` amplitudes apart) into d_out[n][2^m]; d_part: n rows of partials when sliced
+template <typename T>
+int marginal_t(qb_context* ctx, const void* states, uint64_t stride, int n, int n_bits, const qb::MarginalArgs& a, double* d_part, double* d_out) {
+    using C = typename qb::Cx<T>::type;
+    const uint64_t items = uint64_t(1) << (a.h_bits + a.slice_bits);
+    const dim3 grid(unsigned(std::min<uint64_t>(uint64_t(ctx->sm_count) * 8, (items + qb::kMargWarps - 1) / qb::kMargWarps)), unsigned(n));
+    double* dst = a.slice_bits ? d_part : d_out;
+    // a shard's items only reach the bins of its own rank-bit pattern: the others are zero
+    if (!a.slice_bits && a.fixed_mask) QB_CUDA(cudaMemsetAsync(d_out, 0, (sizeof(double) << a.m) * size_t(n), ctx->stream));
+    QB_TRY(with_index_width(ctx, n_bits, [&](auto i) {
+        using Idx = decltype(i);
+        qb::marginal_kernel<T, Idx><<<grid, 32 * qb::kMargWarps, 0, ctx->stream>>>(static_cast<const C*>(states), stride, a, dst);
+        return check_launch(ctx, "marginal_kernel");
+    }));
+    if (!a.slice_bits) return QB_OK;
+    const int group_bits = std::min(8, std::max(5, a.slice_bits - 6));  // 32..256 threads per bin, 64 slices per thread below 256
+    const int bins_per_block = 256 >> group_bits;
+    const dim3 rgrid(unsigned(((uint64_t(1) << a.m) + bins_per_block - 1) / bins_per_block), unsigned(n));
+    qb::marginal_reduce_kernel<<<rgrid, 256, 0, ctx->stream>>>(d_part, a.m, a.slice_bits, group_bits, a.fixed_mask, a.bin_fixed, d_out);
+    return check_launch(ctx, "marginal_reduce_kernel");
+}
+
 }  // namespace
 
 // =====================================================================================================
@@ -2142,6 +2203,62 @@ int qb_top_states(qb_context* ctx, int batch, const int64_t* plan_ids, const dou
         }
         return QB_OK;
     });
+}
+
+// ---- exact marginal probabilities ------------------------------------------------------------------------
+int qb_marginal_probabilities(qb_context* ctx, int batch, const int64_t* plan_ids, const double* params, const int64_t* param_offsets, int n_measured,
+                              const int* qubits, double* out) {
+    if (!ctx || !plan_ids || !param_offsets || !qubits || !out) return fail(QB_ERR_INVALID, "null argument");
+    if (n_measured < 1 || n_measured > qb::kMargMaxBits)
+        return fail(QB_ERR_INVALID, "n_measured must be in 1.." + std::to_string(qb::kMargMaxBits) + ", got " + std::to_string(n_measured));
+    if (batch <= 0) return QB_OK;
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    QB_ON_DEVICE(ctx);
+    const Plan* first = find_plan(ctx, plan_ids[0]);
+    if (!first) return fail(QB_ERR_NOT_FOUND, "unknown plan id " + std::to_string(plan_ids[0]));
+    QB_TRY(check_plans(ctx, batch, plan_ids, first->n_qubits, "the first circuit acts", "marginal", &first));
+    qb::MarginalArgs a;
+    QB_TRY(marginal_args(first->n_eff, 0, n_measured, qubits, first->n_qubits, &a));
+    const uint64_t size = uint64_t(1) << first->n_eff;
+    const size_t state_bytes = size_t(size) * amp_bytes(first->dtype), row_bytes = marginal_scratch_bytes(a);
+    const size_t limit = workspace_limit_of(ctx);
+    if (state_bytes + row_bytes > limit)
+        return fail(QB_ERR_MEMORY, "one statevector (" + std::to_string(state_bytes) + " bytes) and its marginal scratch (" + std::to_string(row_bytes) +
+                                       " bytes) do not fit the workspace of " + std::to_string(limit) + " bytes");
+    const int chunk = int(std::min<size_t>({size_t(batch), max_batch_for(ctx, first), limit / (state_bytes + row_bytes)}));
+    const size_t out_row = size_t(1) << n_measured;
+    return run_oneshot(ctx, batch, plan_ids, params, param_offsets, nullptr, chunk, [&](DeviceBatch& b, int lo) {
+        const size_t nn = size_t(b.batch);
+        QB_TRY(ctx->scratch.reserve(nn * row_bytes));
+        double* d_out = ctx->scratch.as<double>();
+        double* d_part = d_out + nn * out_row;
+        QB_TRY(with_dtype(b.dtype, [&](auto t) { return marginal_t<decltype(t)>(ctx, b.states.p, size, b.batch, b.n_eff, a, d_part, d_out); }));
+        for (size_t pos = 0; pos < nn; ++pos)
+            QB_CUDA(cudaMemcpyAsync(out + (size_t(lo) + size_t(b.order[pos])) * out_row, d_out + pos * out_row, sizeof(double) * out_row,
+                                    cudaMemcpyDeviceToHost, ctx->stream));
+        QB_CUDA(cudaStreamSynchronize(ctx->stream));
+        return QB_OK;
+    });
+}
+
+int qb_marginal_device(qb_context* ctx, int dtype, int n_local, const void* d_state, uint64_t index_offset, int n_measured, const int* qubits,
+                       double* out) {
+    if (!ctx || !d_state || !qubits || !out) return fail(QB_ERR_INVALID, "null argument");
+    if (n_local < 8 || n_local > 36) return fail(QB_ERR_INVALID, "n_local out of range");
+    if (dtype != QB_C128 && dtype != QB_C64) return fail(QB_ERR_INVALID, "dtype must be QB_C128 or QB_C64");
+    if (index_offset & ((uint64_t(1) << n_local) - 1)) return fail(QB_ERR_INVALID, "index_offset has bits below n_local");
+    qb::MarginalArgs a;
+    QB_TRY(marginal_args(n_local, index_offset, n_measured, qubits, 64, &a));
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    QB_ON_DEVICE(ctx);
+    QB_TRY(ctx->scratch.reserve(marginal_scratch_bytes(a)));
+    double* d_out = ctx->scratch.as<double>();
+    double* d_part = d_out + (size_t(1) << n_measured);
+    const uint64_t size = uint64_t(1) << n_local;
+    QB_TRY(with_dtype(dtype, [&](auto t) { return marginal_t<decltype(t)>(ctx, d_state, size, 1, n_local, a, d_part, d_out); }));
+    QB_CUDA(cudaMemcpyAsync(out, d_out, sizeof(double) << n_measured, cudaMemcpyDeviceToHost, ctx->stream));
+    QB_CUDA(cudaStreamSynchronize(ctx->stream));
+    return QB_OK;
 }
 
 int qb_statevector(qb_context* ctx, int64_t plan_id, const double* params, int n_params, double* out_re_im) {

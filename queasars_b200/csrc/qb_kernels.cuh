@@ -1805,6 +1805,116 @@ top_collect_kernel(const typename Cx<T>::type* __restrict__ states, uint64_t sta
 }
 
 // ---------------------------------------------------------------------------------------------------
+// exact marginal probabilities (K11): out[b] = sum of |psi_k|^2 over every k whose measured bits read b, where bit j of b is
+// amplitude bit pos[j] (any subset of the index bits, in any order).  One read of the state, no atomics:
+//   * a warp reads 32 consecutive amplitudes at a time, so amplitude bits 0..4 are the lane and bits >= 5 the "chunk";
+//   * a warp item is (t, s): t fixes the measured chunk bits, s is a slice of the values of the unmeasured chunk bits.  Each lane
+//     sums its amplitudes over the slice in ascending order in a register, then an xor-shuffle butterfly over the unmeasured
+//     lane bits (ascending) adds up the lanes of one bin; one lane per bin writes part[b][s];
+//   * with several slices per t, marginal_reduce_kernel sums part[b][0..S) per bin: threads in slice order, then a fixed tree.
+// Every sum's order depends on the bit positions and the state width alone, so two calls give the same bits.  Items are
+// independent: the grid only spreads them.  p_k is top_prob's (no FMA contraction), so with every qubit measured out[k] is
+// NumPy's re * re + im * im bit for bit.
+// ---------------------------------------------------------------------------------------------------
+constexpr int kMargMaxBits = 26;    // measured qubits of one call: 2^26 doubles (512 MiB) of output per state
+constexpr int kMargWarps = 8;
+constexpr int kMargItemBits = 16;   // split a state into about 2^16 warp items: several waves on the device, small partial rows
+constexpr int kMargUnroll = 4;      // chunk loads in flight per lane
+
+struct MarginalArgs {
+    uint32_t lane_sum;     // amplitude bits 0..4 that are not measured (summed across lanes)
+    uint32_t lane_bin[5];  // output bit (1 << j) of amplitude bit b < 5, 0 where not measured
+    uint32_t bin_fixed;    // output bits of measured qubits above the state (rank bits of a shard, from index_offset)
+    uint32_t fixed_mask;   // the output bits of those qubits: bins with another pattern get no amplitude of this state
+    uint32_t v_mask;       // unmeasured chunk bits (amplitude bits >= 5, shifted down by 5)
+    int32_t h_bits, v_bits, slice_bits, m;
+    int8_t h_pos[32], h_out[32];  // measured chunk bits, ascending, and their output bits
+    int8_t v_pos[32];             // unmeasured chunk bits, ascending
+};
+
+// grid = (CTAs, states), block = 32 * kMargWarps.  Rows `state_stride` amplitudes apart; out row = 2^(m + slice_bits) doubles,
+// [bin][slice] (with slice_bits == 0 the marginal itself).
+template <typename T, typename Idx>
+__global__ void __launch_bounds__(32 * kMargWarps)
+marginal_kernel(const typename Cx<T>::type* __restrict__ states, uint64_t state_stride, MarginalArgs a, double* __restrict__ out) {
+    // byte-wise deposit tables of t (measured chunk bits, their output bits) and of the slice start (unmeasured chunk bits)
+    __shared__ uint32_t s_hc[4][256], s_hb[4][256], s_vc[4][256];
+    for (int e = threadIdx.x; e < 4 * 256; e += blockDim.x) {
+        const int byte = e >> 8, x = e & 255;
+        uint32_t hc = 0, hb = 0, vc = 0;
+        for (int b = 0; b < 8; ++b) {
+            const int i = 8 * byte + b;
+            if (!((x >> b) & 1)) continue;
+            if (i < a.h_bits) hc |= 1u << a.h_pos[i], hb |= 1u << a.h_out[i];
+            if (i < a.v_bits) vc |= 1u << a.v_pos[i];
+        }
+        s_hc[byte][x] = hc, s_hb[byte][x] = hb, s_vc[byte][x] = vc;
+    }
+    __syncthreads();
+    auto deposit = [](const uint32_t (*tab)[256], uint32_t x) { return tab[0][x & 255] | tab[1][(x >> 8) & 255] | tab[2][(x >> 16) & 255] | tab[3][x >> 24]; };
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    uint32_t lane_bin = a.bin_fixed;
+#pragma unroll
+    for (int b = 0; b < 5; ++b) lane_bin |= ((lane >> b) & 1) ? a.lane_bin[b] : 0u;
+    const auto* st = states + uint64_t(blockIdx.y) * state_stride;
+    double* row = out + (uint64_t(blockIdx.y) << (a.m + a.slice_bits));
+    const int len_bits = a.v_bits - a.slice_bits;
+    const uint64_t len = uint64_t(1) << len_bits, items = uint64_t(1) << (a.h_bits + a.slice_bits);
+    const uint32_t slice_mask = (1u << a.slice_bits) - 1u;
+    for (uint64_t item = uint64_t(blockIdx.x) * kMargWarps + warp; item < items; item += uint64_t(gridDim.x) * kMargWarps) {  // warp-uniform
+        const uint32_t t = uint32_t(item >> a.slice_bits), s = uint32_t(item) & slice_mask;
+        const uint32_t hc = deposit(s_hc, t), bin = lane_bin | deposit(s_hb, t);
+        uint32_t v = deposit(s_vc, uint32_t(uint64_t(s) << len_bits));
+        double acc = 0.0;
+        for (uint64_t j = 0; j < len; j += kMargUnroll) {
+            typename Cx<T>::type x[kMargUnroll];
+#pragma unroll
+            for (int u = 0; u < kMargUnroll; ++u) {
+                if (j + u < len) {
+                    x[u] = st[(Idx(hc | v) << 5) | Idx(lane)];
+                    v = ((v | ~a.v_mask) + 1u) & a.v_mask;  // next value of the unmeasured chunk bits
+                }
+            }
+#pragma unroll
+            for (int u = 0; u < kMargUnroll; ++u)
+                if (j + u < len) acc += top_prob(x[u]);
+        }
+#pragma unroll
+        for (int b = 0; b < 5; ++b)
+            if ((a.lane_sum >> b) & 1) acc += __shfl_xor_sync(0xffffffffu, acc, 1 << b);  // a + b == b + a: every lane of a bin agrees
+        if ((uint32_t(lane) & a.lane_sum) == 0) row[(uint64_t(bin) << a.slice_bits) | s] = acc;
+    }
+}
+
+// out[row][b] = sum over s of part[row][b][s]: a group of 2^group_bits threads (32..256, from the slice count) per bin, thread i
+// adding s = i, i + G, ... in order, then a fixed xor tree per warp and the group's warps in order.  Bins whose rank-bit pattern
+// (fixed_mask) is not this shard's (fixed_value) have no partials and get 0.  grid = (ceil(2^m / bins per block), states), block = 256.
+__global__ void __launch_bounds__(256)
+marginal_reduce_kernel(const double* __restrict__ part, int m, int slice_bits, int group_bits, uint32_t fixed_mask, uint32_t fixed_value,
+                       double* __restrict__ out) {
+    __shared__ double s_w[8];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int g = threadIdx.x >> group_bits, i = threadIdx.x & ((1 << group_bits) - 1);
+    const uint64_t bin = (uint64_t(blockIdx.x) << (8 - group_bits)) + g;
+    const bool live = bin < (uint64_t(1) << m) && (uint32_t(bin) & fixed_mask) == fixed_value;
+    double acc = 0.0;
+    if (live) {
+        const double* p = part + (uint64_t(blockIdx.y) << (m + slice_bits)) + (bin << slice_bits);
+        for (uint64_t s = i; s < (uint64_t(1) << slice_bits); s += (1u << group_bits)) acc += p[s];
+    }
+    for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+    if (group_bits > 5) {
+        if (lane == 0) s_w[warp] = acc;
+        __syncthreads();
+        if (i == 0) {
+            acc = 0.0;
+            for (int w = 0; w < (1 << (group_bits - 5)); ++w) acc += s_w[(g << (group_bits - 5)) + w];
+        }
+    }
+    if (i == 0 && bin < (uint64_t(1) << m)) out[(uint64_t(blockIdx.y) << m) + bin] = acc;
+}
+
+// ---------------------------------------------------------------------------------------------------
 // global <-> local qubit swap of a sharded state, fused with its all-to-all: every rank streams its shard ONCE and stores
 // each amplitude straight into the peer that owns it afterwards (peer-mapped buffers, NVLink 5 / NVSwitch), already at its
 // final position -- no pack pass, no staging buffer, no unpack pass.

@@ -180,6 +180,23 @@ def check_top_limits(max_states, min_probability) -> tuple[int, float]:
     return int(max_states), p
 
 
+MARGINAL_MAX_QUBITS = 26
+
+
+def check_marginal_qubits(qubits, n_qubits: int) -> list:
+    """The measured qubits of a marginal: distinct qubit indices of an ``n_qubits``-qubit state, 1 to 26 of them (the output holds
+    2^m doubles per state: 512 MiB at the cap).  ValueError otherwise."""
+    try:
+        qs = [int(q) for q in qubits]
+    except TypeError:
+        raise ValueError(f"qubits must be a sequence of qubit indices, got {qubits!r}") from None
+    if not 1 <= len(qs) <= MARGINAL_MAX_QUBITS:
+        raise ValueError(f"a marginal measures 1 to {MARGINAL_MAX_QUBITS} qubits (2^m doubles per state), got {len(qs)}")
+    if len(set(qs)) != len(qs) or not all(0 <= q < n_qubits for q in qs):
+        raise ValueError(f"qubits must be distinct indices in [0, {n_qubits}), got {qs}")
+    return qs
+
+
 def top_select_new(n_qubits: int, max_states: int) -> _native.TopSelect:
     """A fresh top-states select of ``max_states`` entries over a state of ``n_qubits`` logical qubits (``qb_top_select_init``)."""
     sel = _native.TopSelect()
@@ -563,6 +580,19 @@ class Engine:
                                               _native.ptr(counts), _native.ptr(idx), _native.ptr(probs)))
         return [(idx[i, : counts[i]].copy(), probs[i, : counts[i]].copy()) for i in range(len(plans))]
 
+    def marginal_probabilities(self, plans: Sequence[PlanHandle], params: Sequence[Sequence[float]], qubits: Sequence[int]) -> np.ndarray:
+        """Exact marginal probabilities of every circuit's state on ``qubits``, without shots or a copy of the state
+        (``qb_marginal_probabilities``): float64 [len(plans), 2^m], bit j of the column index = qubit ``qubits[j]`` (the convention of
+        ``Statevector.probabilities(qargs)``).  Deterministic: the same state gives the same bits."""
+        if not plans:
+            return np.zeros((0, 1 << len(qubits)))
+        qs = np.asarray(check_marginal_qubits(qubits, plans[0].n_qubits), dtype=np.int32)
+        ids, flat, offsets = self._pack(plans, params)
+        out = np.empty((len(plans), 1 << qs.size), dtype=np.float64)
+        _native.check(self._lib.qb_marginal_probabilities(self._ctx, len(plans), _native.ptr(ids), _native.ptr(flat), _native.ptr(offsets), int(qs.size),
+                                                          _native.ptr(qs), _native.ptr(out)))
+        return out
+
     def expectation_many(self, plans: Sequence[PlanHandle], params: Sequence[Sequence[float]], handle: ObservablesHandle) -> np.ndarray:
         """Re <psi_i|H_j|psi_i> of every circuit and every observable of ``handle``: float64 array [len(plans), n_obs], each
         distinct Pauli string reduced once per state (``qb_evaluate_observables``)."""
@@ -640,6 +670,15 @@ class Engine:
                                                       byref(sel), None if pos is None else _native.ptr(pos), int(capacity), byref(count), _native.ptr(idx),
                                                       _native.ptr(probs)))
         return idx[: count.value].copy(), probs[: count.value].copy()
+
+    def marginal_device(self, dtype, n_local: int, state_ptr: int, index_offset: int, positions: Sequence[int]) -> np.ndarray:
+        """This shard's part of a marginal (``qb_marginal_device``): float64 [2^m], bit j of the index = physical bit ``positions[j]``;
+        rank bits (positions >= n_local) read their value from ``index_offset``."""
+        pos = np.ascontiguousarray(positions, dtype=np.int32)
+        out = np.empty(1 << pos.size, dtype=np.float64)
+        _native.check(self._lib.qb_marginal_device(self._ctx, _dtype_code(dtype), int(n_local), c_void_p(state_ptr), int(index_offset), int(pos.size),
+                                                   _native.ptr(pos), _native.ptr(out)))
+        return out
 
     def swap_global_p2p(self, dtype, n_local: int, state_ptr: int, peer_ptrs: Sequence[int], rank: int, local_positions: Sequence[int]):
         """Launch the fused swap + all-to-all kernel (asynchronous on the engine's stream; see include/queasars_b200.h)."""

@@ -351,6 +351,58 @@ def from_circuit_or_none(circuit) -> Optional[GateList]:
         return None
 
 
+_CONTROL_FLOW = ("if_else", "while_loop", "for_loop", "switch_case")
+
+
+def _classically_controlled(inst) -> bool:
+    op = inst.operation
+    if op.name in _CONTROL_FLOW or inst.clbits:
+        return True
+    for attr in ("_condition", "condition"):  # (``c_if``; Qiskit 1.x keeps it in ``_condition``, 2.x has neither)
+        try:
+            if getattr(op, attr, None) is not None:
+                return True
+        except Exception:  # a deprecated property that refuses to be read
+            pass
+    return False
+
+
+def final_measurements(circuit) -> list[tuple[str, int, list[Optional[int]]]]:
+    """The final measurements of a (Qiskit-API) circuit: per classical register of ``circuit.cregs``, in that order,
+    (name, size, [measured qubit or None per position]).  Qiskit semantics: the last measurement written to a clbit wins, one
+    qubit may be written to several clbits, and a clbit nobody writes reads 0 (None here).  Clbits are located through
+    ``circuit.find_bit(clbit).registers``, so real Qiskit circuits and the stand-in go through the same code.
+
+    ``NotImplementedError`` for what a sampler that draws from the final state cannot reproduce: a gate on a qubit after it was
+    measured (mid-circuit measurement), ``reset``, and classical control (``c_if``, ``if_else`` and the other control-flow
+    operations, or any other operation with clbits)."""
+    cregs = list(getattr(circuit, "cregs", None) or [])
+    by_reg = {reg.name: [None] * len(reg) for reg in cregs}
+    measured: set = set()
+    for inst in circuit.data:
+        name = inst.operation.name
+        if name == "measure":
+            q = circuit.find_bit(inst.qubits[0]).index
+            for clbit in inst.clbits:
+                for reg, pos in circuit.find_bit(clbit).registers:
+                    if reg.name in by_reg:
+                        by_reg[reg.name][pos] = q
+            measured.add(q)
+            continue
+        if name == "reset":
+            raise NotImplementedError("reset is not supported by the B200 sampler: it draws from the final state of a unitary circuit")
+        if _classically_controlled(inst):
+            raise NotImplementedError(f"classically controlled operation '{name}' is not supported by the B200 sampler")
+        if name == "barrier":
+            continue
+        hit = measured.intersection(circuit.find_bit(qb).index for qb in inst.qubits)
+        if hit:
+            raise NotImplementedError(
+                f"mid-circuit measurement is not supported by the B200 sampler: '{name}' acts on qubit {min(hit)} after it was measured"
+            )
+    return [(reg.name, len(reg), by_reg[reg.name]) for reg in cregs]
+
+
 # -------------------------------------------------------------------------------------------------
 # direct genome -> gate list path (SURVEY.md section 8f-3): bypasses QuantumCircuit construction
 # -------------------------------------------------------------------------------------------------

@@ -35,7 +35,7 @@ from . import containers as ct
 from . import expectation as ex
 from .batching import CoalescingQueue
 from .engine import Engine, HamiltonianHandle, ObservablesHandle, PlanHandle
-from .gate_list import from_circuit_or_none, from_circuit
+from .gate_list import final_measurements, from_circuit_or_none, from_circuit
 
 _engines: dict = {}
 _engines_lock = threading.Lock()
@@ -724,15 +724,25 @@ def _single_observable(observables):
     return obs
 
 
-def _check_measure_all(circuit) -> None:
-    """The sampler returns ONE full-width register named "meas" -- what ``measure_all`` produces and the only shape QUEASARS
-    consumes (circuit_evaluation.py:50-55).  Circuits with other classical registers would get a silently different result
-    from upstream's per-register BitArrays, so they are rejected."""
-    cregs = getattr(circuit, "cregs", None)
-    if not cregs:
-        return
-    if len(cregs) != 1 or getattr(cregs[0], "name", "meas") != "meas" or len(cregs[0]) != int(circuit.num_qubits):
-        raise NotImplementedError("B200SamplerV2 supports circuits measured with measure_all() only (one register 'meas' over all qubits)")
+def _registers(circuit) -> list:
+    """(name, size, measured qubit or None per position) of every classical register of a pub's circuit (``final_measurements``).
+    A circuit without classical registers (or an EVQE genome) reads out as one register "meas" over all qubits, as before
+    registers were supported."""
+    n = _width(circuit)
+    return ([] if _is_genome(circuit) else final_measurements(circuit)) or [("meas", n, list(range(n)))]
+
+
+def register_values(indices: np.ndarray, qubits: Sequence[Optional[int]]) -> np.ndarray:
+    """Value of one classical register for every drawn basis index: sum over positions j of ((k >> qubits[j]) & 1) << j; a position
+    measured by no qubit (None) reads 0."""
+    k = np.asarray(indices, dtype=np.int64)
+    if len(qubits) > 63:
+        raise NotImplementedError(f"classical registers of more than 63 bits are not supported (got {len(qubits)})")
+    out = np.zeros(k.shape, dtype=np.int64)
+    for j, q in enumerate(qubits):
+        if q is not None:
+            out |= ((k >> q) & 1) << j
+    return out
 
 
 class B200SamplerV2(_B200Primitive):
@@ -777,6 +787,24 @@ class B200SamplerV2(_B200Primitive):
         if len(widths) != 1:
             raise ValueError("all circuits of one sampler submission must act on the same number of qubits")
         return list(self._submit(("top", widths.pop(), max_states, min_probability), (None, circuits, parameter_values)))
+
+    def marginal_probabilities(self, circuits, parameter_values, qubits) -> np.ndarray:
+        """Exact marginal probabilities of every circuit's state on ``qubits`` (distinct qubit indices, 1 to 26 of them), without
+        shots: float64 [len(circuits), 2^m], bit j of the column index = qubit ``qubits[j]`` -- ``Statevector.probabilities(qargs)``
+        with ``qargs = qubits``.  Reduced on the device (``Engine.marginal_probabilities``); circuits too wide for one GPU run as one
+        statevector sharded over the device set, one at a time, and give the same marginal (``_ShardedLogic.marginal``)."""
+        from .engine import check_marginal_qubits
+
+        circuits, parameter_values = list(circuits), list(parameter_values)
+        if len(circuits) != len(parameter_values):
+            raise ValueError(f"{len(circuits)} circuits but {len(parameter_values)} parameter vectors")
+        widths = {_width(c) for c in circuits}
+        if len(widths) > 1:
+            raise ValueError("all circuits of one sampler submission must act on the same number of qubits")
+        qubits = tuple(check_marginal_qubits(qubits, widths.pop() if widths else 64))
+        if not circuits:
+            return np.zeros((0, 1 << len(qubits)))
+        return np.asarray(self._submit(("marg", _width(circuits[0]), qubits), (None, circuits, parameter_values)), dtype=np.float64)
 
     def cvar_values(self, circuits, parameter_values, operator, alpha: float) -> np.ndarray:
         """Exact (shot-free) CVaR(alpha) of the diagonal ``operator`` on every circuit's full distribution |psi|^2:
@@ -846,6 +874,14 @@ class B200SamplerV2(_B200Primitive):
                 return self._run_per_device(resolved, lambda slot, plans, params: self.engines[slot].top_states(plans, params, max_states, min_probability))
 
             return width, lambda sv: sv.top_states(max_states, min_probability), top_on_devices, list
+        if key[0] == "marg":
+            _, width, qubits = key
+
+            def marginal_on_devices(circuits, values):
+                resolved = self._resolve_all(circuits, values, probabilities_only=True)
+                return self._run_per_device(resolved, lambda slot, plans, params: list(self.engines[slot].marginal_probabilities(plans, params, qubits)))
+
+            return width, lambda sv: sv.marginal(qubits), marginal_on_devices, lambda rows: np.asarray(rows, dtype=np.float64).reshape(len(rows), 1 << len(qubits))
         kind, _, fp, alpha, width = key
         operator = target
 
@@ -873,13 +909,14 @@ class B200SamplerV2(_B200Primitive):
             for pub in coerced:
                 n_shots = int(pub.shots if pub.shots is not None else self.default_shots)
                 rows, shape = _param_rows(pub.parameter_values)
-                _check_measure_all(pub.circuit)
+                registers = _registers(pub.circuit)  # (raises NotImplementedError for measurements the sampler cannot read out)
                 if shape == ():
                     idx = self.sample_indices([pub.circuit], [rows[0]], n_shots)[0]
                 else:  # a parameter array: one submission over all rows, one register position per row
                     idx = self.sample_indices([pub.circuit] * len(rows), list(rows), n_shots).reshape(shape + (n_shots,))
-                reg = ct.ShotRegister(idx, int(pub.circuit.num_qubits), shape)
-                results.append(ct.SamplerPubResult(ct.DataBin(meas=reg, shape=shape), metadata={"shots": n_shots, "circuit_metadata": {}}))
+                # the full basis index of every shot is a draw from |psi|^2, so its measured bits are a draw from their marginal
+                data = {name: ct.ShotRegister(register_values(idx, qubits), size, shape) for name, size, qubits in registers}
+                results.append(ct.SamplerPubResult(ct.DataBin(shape=shape, **data), metadata={"shots": n_shots, "circuit_metadata": {}}))
             return ct.FinishedJob(ct.PrimitiveResult(results, metadata={"version": 2, "backend": "queasars_b200"}))
         except Exception as exc:
             return ct.FinishedJob(error=exc)

@@ -141,6 +141,11 @@ class CudaShardBackend:
         self._join_torch_stream(state)
         return self.engine.top_collect_device("complex128", n_local, _state_ptr(state), index_offset, min_probability, sel, positions, capacity)
 
+    def marginal(self, state, n_local: int, index_offset: int, positions) -> np.ndarray:
+        """This shard's part of ``_ShardedLogic.marginal`` (``qb_marginal_device``): float64 [2^len(positions)]."""
+        self._join_torch_stream(state)
+        return self.engine.marginal_device("complex128", n_local, _state_ptr(state), index_offset, positions)
+
     def swap_p2p(self, state, peer_ptrs: Sequence[int], n_local: int, rank: int, local_positions: Sequence[int]) -> None:
         """Fused swap + all-to-all into the peers' buffers; returns when this rank's stores have been issued and completed."""
         self._join_torch_stream(state)
@@ -165,6 +170,7 @@ class _ShardedLogic:
       _select_pass(z, c, cache_mode, spec)        every shard's bucket arrays of one cvar select pass, in rank order
       _top_pass(sel, positions, min_p)            every shard's bucket counts of one top-states select pass, in rank order
       _top_collect(sel, positions, min_p)         every shard's (physical indices, probabilities) up to the stop key, in rank order
+      _marginal_parts(positions)                  every shard's marginal on the physical bits ``positions``, in rank order
       _sample_shards(owner, local_u)              physical indices of the shots (owner[s] = shard of shot s), int64 [shots]"""
 
     def _init_logic(self, n_qubits: int, world: int, min_local: int):
@@ -412,6 +418,20 @@ class _ShardedLogic:
             logical |= ((physical >> self.position[q]) & 1) << q
         order = np.lexsort((logical, -probs))
         return logical[order], probs[order]
+
+    def marginal(self, qubits: Sequence[int]) -> np.ndarray:
+        """Exact marginal probabilities on the logical ``qubits``: float64 [2^m], bit j of the index = qubit ``qubits[j]`` -- what
+        ``Engine.marginal_probabilities`` gives for the unsharded state.  Every shard reduces its own amplitudes with the logical
+        qubits read at their physical positions (rank bits enter through the shard's index offset), so no data moves and no swap
+        happens; the shards' marginals are added in rank order and every caller gets the same result."""
+        from .engine import check_marginal_qubits
+
+        positions = [int(self.position[q]) for q in check_marginal_qubits(qubits, self.n_qubits)]
+        parts = self._marginal_parts(positions)
+        total = np.array(parts[0], dtype=np.float64)
+        for part in parts[1:]:
+            total += part
+        return total
 
     def sample(self, shots: int, seed=None, uniforms: Optional[np.ndarray] = None) -> np.ndarray:
         """``shots`` basis-state indices (logical qubit order) drawn from |psi|^2; every caller gets all of them.
@@ -734,6 +754,15 @@ class ShardedStatevector(_ShardedLogic):
         self._dist.all_gather_object(parts, (np.asarray(mine[0]), np.asarray(mine[1])), group=self.group)
         return parts
 
+    def _marginal_parts(self, positions) -> list:
+        mine = np.asarray(self.backend.marginal(self.state, self.n_local, self.index_offset, positions), dtype=np.float64)
+        if self.world == 1:
+            return [mine]
+        t = self._torch.from_numpy(mine).to(self.device)
+        parts = [self._torch.empty_like(t) for _ in range(self.world)]
+        self._dist.all_gather(parts, t, group=self.group)
+        return [part.cpu().numpy() for part in parts]
+
     def _sample_shards(self, owner: np.ndarray, local_u: np.ndarray) -> np.ndarray:
         physical = np.zeros(owner.size, dtype=np.int64)
         mine = np.nonzero(owner == self.rank)[0]
@@ -864,6 +893,9 @@ class LocalShardedStatevector(_ShardedLogic):
     def _top_collect(self, sel, positions, min_probability) -> list:
         return self._each(lambda r: self.backends[r].top_collect(self._state(r), self.n_local, r << self.n_local, min_probability, sel, positions,
                                                                  int(sel.selected)))
+
+    def _marginal_parts(self, positions) -> list:
+        return self._each(lambda r: self.backends[r].marginal(self._state(r), self.n_local, r << self.n_local, positions))
 
     def _sample_shards(self, owner: np.ndarray, local_u: np.ndarray) -> np.ndarray:
         physical = np.zeros(owner.size, dtype=np.int64)
