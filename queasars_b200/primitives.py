@@ -393,11 +393,10 @@ class _B200Primitive:
     def _sharded_state(self, n_qubits: int):
         """One state of ``n_qubits`` sharded over the largest power-of-two prefix of the device set (kept between calls: two
         shard-sized buffers per GPU where they fit, one otherwise -- the in-place exchange).  BASELINE config C5: 35 qubits over
-        8 GPUs; one buffer per GPU reaches 34 qubits on 2 GPUs and 36 on 8."""
-        from .sharded import LocalShardedStatevector
+        8 GPUs; one buffer per GPU reaches 34 qubits on 2 GPUs and 36 on 8, one more in complex64 (the state takes the dtype of
+        the device set's engines, which is the primitive's)."""
+        from .sharded import AMPLITUDE_BYTES, LocalShardedStatevector
 
-        if self.dtype != "complex128":
-            raise NotImplementedError("sharded statevectors are complex128")
         with self._lock:
             sv = self._sharded_obj.get(n_qubits)
         if sv is not None:
@@ -418,7 +417,7 @@ class _B200Primitive:
         except _native.QbError as exc:
             if exc.code != _native.QB_ERR_MEMORY:
                 raise
-            shard = 16 << (n_qubits - int(np.log2(count)))
+            shard = AMPLITUDE_BYTES[self.dtype] << (n_qubits - int(np.log2(count)))
             raise ValueError(f"a {n_qubits}-qubit statevector sharded over {count} GPUs needs at least one {shard} byte buffer "
                              f"({shard / 2**30:.0f} GiB) per GPU, which does not fit: {exc}") from exc
         with self._lock:

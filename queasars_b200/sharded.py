@@ -20,6 +20,10 @@ bit position p < n-g is local, p >= n-g is a rank bit.  Logical qubits are track
         half the memory: the widest state a device set holds grows by one qubit (34 on 2 GPUs, 36 on 8).
     ``buffers=None`` takes two buffers where they fit and one otherwise.
 
+A state is complex128 or complex64 (``dtype``: the dtype of its engines).  complex64 takes 8 instead of 16 bytes per amplitude, so
+every device set holds one qubit more (35 on 2 GPUs, 37 on 8 with one buffer each); the kernels, routes and read-outs are the
+same, except that the exact CVaR select has no (p, E) cache in complex64 (``_ShardedLogic.cvar``).
+
 Two drivers share the schedule (``_ShardedLogic``):
 
   ``ShardedStatevector``       one process per GPU (``torchrun``): collectives over ``torch.distributed``; the shard buffers are
@@ -79,6 +83,7 @@ class CudaShardBackend:
 
     def __init__(self, engine):
         self.engine = engine
+        self.dtype = _engine_dtype(engine)  # every native call reads and writes the shard as this dtype
         self._select_ham = None
 
     @staticmethod
@@ -103,7 +108,7 @@ class CudaShardBackend:
         op = SparsePauliOp._raw(n_total, [0] * len(z_masks), [int(z) for z in z_masks], [float(c) for c in coeffs])
         ham = self.engine.hamiltonian(op, build_table=False)
         self._join_torch_stream(state)
-        return self.engine.expectation_device(ham, "complex128", n_local, _state_ptr(state), index_offset)
+        return self.engine.expectation_device(ham, self.dtype, n_local, _state_ptr(state), index_offset)
 
     def pauli_expectation(self, state, x_masks, z_masks, coeffs, n_total: int, n_local: int, index_offset: int) -> float:
         """Shard-local part of Re <psi| sum_t c_t P_t |psi> for terms whose X part only flips local qubits (z may reach
@@ -113,11 +118,11 @@ class CudaShardBackend:
         op = SparsePauliOp._raw(n_total, [int(x) for x in x_masks], [int(z) for z in z_masks], [complex(c) for c in coeffs])
         ham = self.engine.hamiltonian(op, build_table=False)
         self._join_torch_stream(state)
-        return self.engine.expectation_device(ham, "complex128", n_local, _state_ptr(state), index_offset)
+        return self.engine.expectation_device(ham, self.dtype, n_local, _state_ptr(state), index_offset)
 
     def sample(self, state, uniforms: np.ndarray, n_local: int) -> np.ndarray:
         self._join_torch_stream(state)
-        return self.engine.sample_device("complex128", n_local, _state_ptr(state), uniforms)
+        return self.engine.sample_device(self.dtype, n_local, _state_ptr(state), uniforms)
 
     def cvar_select(self, state, cache, cache_mode: int, z_masks, coeffs, n_total: int, n_local: int, index_offset: int, spec):
         """One select pass of ``_ShardedLogic.cvar`` on this shard (``qb_cvar_select_device``); ``cache`` is the idle spare buffer."""
@@ -128,35 +133,35 @@ class CudaShardBackend:
             op = SparsePauliOp._raw(n_total, [0] * len(key[1]), list(key[1]), list(key[2]))
             self._select_ham = (key, self.engine.hamiltonian(op, build_table=False))
         self._join_torch_stream(state)
-        return self.engine.cvar_select_device(self._select_ham[1], "complex128", n_local, _state_ptr(state), index_offset,
+        return self.engine.cvar_select_device(self._select_ham[1], self.dtype, n_local, _state_ptr(state), index_offset,
                                               0 if cache is None else _state_ptr(cache), cache_mode, *spec)
 
     def top_select(self, state, n_local: int, index_offset: int, min_probability: float, sel, positions) -> np.ndarray:
         """One select pass of ``_ShardedLogic.top_states`` on this shard (``qb_top_select_device``): uint64 bucket counts [256]."""
         self._join_torch_stream(state)
-        return self.engine.top_select_device("complex128", n_local, _state_ptr(state), index_offset, min_probability, sel, positions)
+        return self.engine.top_select_device(self.dtype, n_local, _state_ptr(state), index_offset, min_probability, sel, positions)
 
     def top_collect(self, state, n_local: int, index_offset: int, min_probability: float, sel, positions, capacity: int):
         """This shard's entries up to the stop key of ``sel`` (``qb_top_collect_device``) -> (physical indices, probabilities)."""
         self._join_torch_stream(state)
-        return self.engine.top_collect_device("complex128", n_local, _state_ptr(state), index_offset, min_probability, sel, positions, capacity)
+        return self.engine.top_collect_device(self.dtype, n_local, _state_ptr(state), index_offset, min_probability, sel, positions, capacity)
 
     def marginal(self, state, n_local: int, index_offset: int, positions) -> np.ndarray:
         """This shard's part of ``_ShardedLogic.marginal`` (``qb_marginal_device``): float64 [2^len(positions)]."""
         self._join_torch_stream(state)
-        return self.engine.marginal_device("complex128", n_local, _state_ptr(state), index_offset, positions)
+        return self.engine.marginal_device(self.dtype, n_local, _state_ptr(state), index_offset, positions)
 
     def swap_p2p(self, state, peer_ptrs: Sequence[int], n_local: int, rank: int, local_positions: Sequence[int]) -> None:
         """Fused swap + all-to-all into the peers' buffers; returns when this rank's stores have been issued and completed."""
         self._join_torch_stream(state)
-        self.engine.swap_global_p2p("complex128", n_local, _state_ptr(state), peer_ptrs, rank, local_positions)
+        self.engine.swap_global_p2p(self.dtype, n_local, _state_ptr(state), peer_ptrs, rank, local_positions)
         self.engine.synchronize()
 
     def swap_inplace_p2p(self, state, shard_ptrs: Sequence[int], n_local: int, rank: int, local_positions: Sequence[int]) -> None:
         """The same exchange in place on every rank's ONE state buffer (``shard_ptrs``, peer-mapped); returns when this rank's
         loads and stores have completed.  The caller runs the cross-rank barriers before and after (include/queasars_b200.h)."""
         self._join_torch_stream(state)
-        self.engine.swap_global_inplace_p2p("complex128", n_local, shard_ptrs, rank, local_positions)
+        self.engine.swap_global_inplace_p2p(self.dtype, n_local, shard_ptrs, rank, local_positions)
         self.engine.synchronize()
 
 
@@ -173,10 +178,12 @@ class _ShardedLogic:
       _marginal_parts(positions)                  every shard's marginal on the physical bits ``positions``, in rank order
       _sample_shards(owner, local_u)              physical indices of the shots (owner[s] = shard of shot s), int64 [shots]"""
 
-    def _init_logic(self, n_qubits: int, world: int, min_local: int):
+    def _init_logic(self, n_qubits: int, world: int, min_local: int, dtype: str = "complex128"):
         g = int(round(math.log2(world)))
         if 1 << g != world:
             raise ValueError("the number of shards must be a power of two")
+        self.dtype = _check_dtype(dtype)
+        self.amp_bytes = AMPLITUDE_BYTES[self.dtype]
         self.world = world
         self.n_qubits, self.n_global, self.n_local = n_qubits, g, n_qubits - g
         if self.n_local < max(min_local, 2 * g):
@@ -210,7 +217,7 @@ class _ShardedLogic:
             elif p in lp:
                 self.position[q] = nl + lp.index(p)
         self.swaps_done += 1
-        self.bytes_sent += (self.world - 1) * ((1 << nl) // self.world) * 16
+        self.bytes_sent += (self.world - 1) * ((1 << nl) // self.world) * self.amp_bytes
 
     # ------------------------------------------------------------------ circuit execution
     def run(self, gates: GateList, params: Sequence[float]) -> None:
@@ -322,12 +329,13 @@ class _ShardedLogic:
         as it holds one entry.  Logical index bits are read from their physical positions: no data moves.  The first pass
         stores (p, E) of every entry in the idle spare buffer, the later ones read it from there.  Every rank makes the same
         decisions from the same all-gathered numbers, so every caller gets the same result.  ``cache=False`` recomputes p and E
-        from the state on every pass instead (same values); so does a state with one buffer per shard, which has no spare."""
+        from the state on every pass instead (same values); so does a state with one buffer per shard, which has no spare, and a
+        complex64 state, whose spare holds 8 of the 16 bytes a (p, E) entry takes."""
         from . import expectation as ex
         from .engine import merge_duplicate_terms
 
         ex.check_alpha(alpha)
-        cache = cache and self.buffers == 2
+        cache = cache and self.buffers == 2 and self.amp_bytes == 16
         _, zs, cs = merge_duplicate_terms(np.zeros(len(z_masks), dtype=np.uint64), np.asarray(z_masks, dtype=np.uint64), np.asarray(coeffs, dtype=np.float64))
         phys = np.asarray([self._physical_mask(z) for z in zs], dtype=np.uint64)
         cf = np.ascontiguousarray(np.real(cs), dtype=np.float64)
@@ -458,13 +466,28 @@ class _ShardedLogic:
 
     def describe(self) -> dict:
         return {"n_qubits": self.n_qubits, "shards": self.world, "n_local": self.n_local, "swaps_done": self.swaps_done, "swap_path": self.swap_path,
-                "swap_fallback_reason": self.swap_fallback_reason, "buffers": self.buffers}
+                "swap_fallback_reason": self.swap_fallback_reason, "buffers": self.buffers, "dtype": self.dtype}
 
     def _logical_from_physical(self, full: np.ndarray) -> np.ndarray:
         n = self.n_qubits
         # physical axis a <-> physical bit n-1-a ; logical bit q lives at physical position[q]
         perm = [n - 1 - self.position[q] for q in range(n - 1, -1, -1)]
         return np.ascontiguousarray(full.reshape((2,) * n).transpose(perm)).reshape(-1)
+
+
+AMPLITUDE_BYTES = {"complex128": 16, "complex64": 8}
+
+
+def _check_dtype(dtype) -> str:
+    """The dtype's name (``complex128`` or ``complex64``: the dtypes of the engine)."""
+    name = np.dtype(dtype).name
+    if name not in AMPLITUDE_BYTES:
+        raise ValueError(f"a sharded statevector is complex128 or complex64, not {dtype!r}")
+    return name
+
+
+def _engine_dtype(engine) -> str:
+    return _check_dtype(getattr(engine, "dtype", "complex128"))  # (complex128: the engine's default)
 
 
 def _check_buffers(buffers) -> None:
@@ -476,12 +499,12 @@ def _out_of_memory(exc: BaseException) -> bool:
     return isinstance(exc, _native.QbError) and exc.code == _native.QB_ERR_MEMORY
 
 
-def _allocate_set(engines: Sequence, size: int) -> list:
+def _allocate_set(engines: Sequence, size: int, dtype: str) -> list:
     """One shard buffer of ``size`` amplitudes per engine; what was allocated is freed again when one allocation fails."""
     bufs = []
     try:
         for e in engines:
-            bufs.append(_DeviceBuffer(e, size))
+            bufs.append(_DeviceBuffer(e, size, dtype))
     except BaseException:
         for b in bufs:
             b.free()
@@ -489,14 +512,14 @@ def _allocate_set(engines: Sequence, size: int) -> list:
     return bufs
 
 
-def _allocate_sets(engines: Sequence, size: int, buffers) -> list:
+def _allocate_sets(engines: Sequence, size: int, buffers, dtype: str) -> list:
     """[first set] or [first set, second set] of shard buffers: ``buffers`` = 1 / 2 forces the count; None takes the second set
     when it fits (an allocation failing with QB_ERR_MEMORY frees the partial set and keeps one; any other error is raised)."""
-    sets = [_allocate_set(engines, size)]
+    sets = [_allocate_set(engines, size, dtype)]
     if buffers == 1:
         return sets
     try:
-        sets.append(_allocate_set(engines, size))
+        sets.append(_allocate_set(engines, size, dtype))
     except Exception as exc:  # noqa: BLE001
         if buffers is None and _out_of_memory(exc):
             return sets
@@ -509,10 +532,11 @@ def _allocate_sets(engines: Sequence, size: int, buffers) -> list:
 class _DeviceBuffer:
     """cudaMalloc allocation owned by an engine, usable as a torch tensor through ``__cuda_array_interface__``."""
 
-    def __init__(self, engine, n_amplitudes: int):
+    def __init__(self, engine, n_amplitudes: int, dtype: str):
         self.engine, self.size = engine, int(n_amplitudes)
-        self.ptr = engine.device_alloc(16 * self.size)
-        self.__cuda_array_interface__ = {"shape": (self.size,), "typestr": "<c16", "data": (self.ptr, False), "version": 3, "strides": None}
+        amp = AMPLITUDE_BYTES[dtype]
+        self.ptr = engine.device_alloc(amp * self.size)
+        self.__cuda_array_interface__ = {"shape": (self.size,), "typestr": f"<c{amp}", "data": (self.ptr, False), "version": 3, "strides": None}
 
     def free(self):
         if self.ptr:
@@ -529,11 +553,13 @@ class _DeviceBuffer:
 class ShardedStatevector(_ShardedLogic):
     """One process per GPU / rank; collectives over ``torch.distributed`` (NCCL on GPUs, gloo in the CPU tests)."""
 
-    def __init__(self, n_qubits: int, backend=None, group=None, device=None, min_local: int = 12, buffers: Optional[int] = None):
+    def __init__(self, n_qubits: int, backend=None, group=None, device=None, min_local: int = 12, buffers: Optional[int] = None,
+                 dtype: str = "complex128"):
         """``buffers``: shard-sized buffers per rank where the ranks map each other's memory -- 2 (ping-pong exchange), 1 (in-place
         exchange: one qubit wider for the same memory) or None (two where every rank can allocate them, else one; the ranks agree).
         The pack + all-to-all route (``QB_SWAP=nccl``, no CUDA IPC, CPU tensors) stages through a spare: it always has two, and
-        ``buffers=1`` there raises ValueError on every rank."""
+        ``buffers=1`` there raises ValueError on every rank.  ``dtype`` (complex128 or complex64) is the dtype of the shard buffers
+        and of the engine this rank creates; a given backend's engine must have it."""
         import torch
         import torch.distributed as dist
 
@@ -542,13 +568,15 @@ class ShardedStatevector(_ShardedLogic):
         self.group = group
         world = dist.get_world_size(group) if dist.is_initialized() else 1
         self.rank = dist.get_rank(group) if dist.is_initialized() else 0
-        self._init_logic(n_qubits, world, min_local)
+        self._init_logic(n_qubits, world, min_local, dtype)
         if backend is None:
             from .primitives import get_engine
 
             dev_index = torch.cuda.current_device() if device is None else torch.device(device).index
-            backend = CudaShardBackend(get_engine(dev_index, "complex128"))
+            backend = CudaShardBackend(get_engine(dev_index, self.dtype))
             device = torch.device("cuda", dev_index)
+        elif hasattr(backend, "engine") and _engine_dtype(backend.engine) != self.dtype:
+            raise ValueError(f"a {self.dtype} sharded statevector cannot run on a {_engine_dtype(backend.engine)} engine")
         self.backend = backend
         self.device = torch.device("cpu") if device is None else torch.device(device)
         size = 1 << self.n_local
@@ -565,8 +593,9 @@ class ShardedStatevector(_ShardedLogic):
                 reason = self.swap_fallback_reason or f"shards on {self.device.type} with {type(backend).__name__}"
                 raise ValueError("one buffer per shard needs the in-place exchange over peer-mapped memory; this state has none "
                                  f"({reason}): the pack + all-to-all route stages through a second buffer")
-            self.state = torch.zeros(size, dtype=torch.complex128, device=self.device)
-            self.spare = None if buffers == 1 else torch.empty(size, dtype=torch.complex128, device=self.device)
+            dt = getattr(torch, self.dtype)
+            self.state = torch.zeros(size, dtype=dt, device=self.device)
+            self.spare = None if buffers == 1 else torch.empty(size, dtype=dt, device=self.device)
             self.buffers = 1 if buffers == 1 else 2
 
     def _map_ipc_buffers(self, size: int, buffers: Optional[int]):
@@ -578,7 +607,7 @@ class ShardedStatevector(_ShardedLogic):
         engine = self.backend.engine
         error, bufs, handles = None, [], []
         try:
-            bufs = [s[0] for s in _allocate_sets([engine], size, buffers)]
+            bufs = [s[0] for s in _allocate_sets([engine], size, buffers, self.dtype)]
         except Exception as exc:  # noqa: BLE001
             error = repr(exc)
         counts = [None] * self.world
@@ -796,14 +825,18 @@ class LocalShardedStatevector(_ShardedLogic):
     use for circuits too wide for one GPU.
 
     ``buffers``: shard-sized buffers per shard -- 2 (ping-pong exchange), 1 (in-place exchange) or None (two where they can be
-    allocated, else one)."""
+    allocated, else one).  The state has the dtype of its engines (complex128 or complex64; engines of different dtypes raise
+    ValueError)."""
 
     def __init__(self, n_qubits: int, engines: Sequence, min_local: int = 12, buffers: Optional[int] = None):
         from concurrent.futures import ThreadPoolExecutor
 
         _check_buffers(buffers)
         engines = list(engines)
-        self._init_logic(n_qubits, len(engines), min_local)
+        dtypes = sorted({_engine_dtype(e) for e in engines})
+        if len(dtypes) != 1:
+            raise ValueError(f"the engines of one sharded statevector must have one dtype, not {dtypes}")
+        self._init_logic(n_qubits, len(engines), min_local, dtypes[0])
         self.engines = engines
         self.backends = [CudaShardBackend(e) for e in engines]
         devices = [e.device for e in engines]
@@ -811,7 +844,7 @@ class LocalShardedStatevector(_ShardedLogic):
             for d in set(devices):
                 e.enable_peer_access(d)  # raises (with the reason) when the GPUs cannot map each other's memory
         size = 1 << self.n_local
-        self._bufs = _allocate_sets(engines, size, buffers)  # [which][shard]
+        self._bufs = _allocate_sets(engines, size, buffers, self.dtype)  # [which][shard]
         self.buffers = len(self._bufs)
         self._cur = 0
         self._pool = ThreadPoolExecutor(max_workers=len(engines), thread_name_prefix="qb-shard") if len(engines) > 1 else None
@@ -910,7 +943,7 @@ class LocalShardedStatevector(_ShardedLogic):
 
     def gather_physical(self) -> np.ndarray:
         size = 1 << self.n_local
-        full = np.empty(self.world * size, dtype=np.complex128)
+        full = np.empty(self.world * size, dtype=self.dtype)
         for r in range(self.world):
             self.engines[r].device_read(self._state(r), 0, full[r * size : (r + 1) * size])
         return full
